@@ -1,10 +1,15 @@
 """Benchmark of the hot path: CV grid fits/sec (alpha x fold), device-timed.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference]
-                    [--workload c3|c2|c1|c4|c5]
+                    [--workload c3|c2|c1|c4|c5] [--dump-outputs DIR]
 
 One "step" = one full cross-validated grid search of the workload (every
 (alpha, fold) problem solved to the duality-gap tolerance and scored).
+
+--dump-outputs DIR writes what the last timed step of the device-resident arm returned as DIR/<name>.npy
+(float64): the test-score table, the solver info per (alpha, fold) and every alpha's warm-start solution.
+The inputs are generated from fixed seeds, so two builds run with the same arguments can be compared
+output for output.  bench_outputs/ is the directory git ignores for this.
 
 * value     : fits/sec with X, y already resident in HBM when the timed region starts
               (Gram build + Lipschitz + batched solve + CV scoring, CUDA events, max over ranks)
@@ -537,6 +542,8 @@ def run_engine(args):
     tim = engine.timing_read()
     exec_flops, dense_flops = engine.apply_stats()
     engine.timing_enable(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, len(alphas))
     ms = float(np.mean(times))
     if world > 1:
         import torch.distributed as dist
@@ -580,6 +587,28 @@ def run_engine(args):
         e2e = run_e2e(args, torch, wl, shard, barrier, world, dev)
     finish(args, wl, res, engine, tim, exec_flops, dense_flops, ms, value, e2e, launches, clocks, peak, world, rank,
            weak, parity, tall)
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, res, n_cand):
+    """Write what batched_cv returned to its caller as out_dir/<name>.npy (float64): the test-score table
+    [alpha, fold], the solver info tables [alpha, fold] (info_*), the iteration and unconverged counts, and
+    each alpha's warm-start solution [alpha, feature] (its solution on the first training fold that solved it,
+    in the solver's feature order: the start point of the refit; NaN rows were solved by another rank)."""
+    arrays = {"test_scores": res["test_scores"], "iters_run": res["iters_run"], "n_unconverged": res["n_unconverged"]}
+    arrays.update({f"info_{k}": v for k, v in res["info"].items()})
+    warm = [res["warm"].get(ci) for ci in range(n_cand)]
+    pe = next(w.numel() for w in warm if w is not None)
+    arrays["warm_start_coef"] = np.stack([np.full(pe, np.nan) if w is None else w.cpu().numpy() for w in warm])
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_MAX_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def run_tall(args, torch, engine, shard, barrier, world, rank, dev, peak):
@@ -840,7 +869,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--no-weak", action="store_true", help="skip the weak-scaling companion run (N > 1)")
     ap.add_argument("--no-tall", action="store_true", help="skip the tall-design (C5) companion object")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (engine only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs needs --impl engine")
     args.warmup = max(args.warmup, 3) if args.impl == "engine" else args.warmup
     if args.impl == "reference":
         run_reference(args)
