@@ -47,6 +47,7 @@ struct Family {
 };
 
 constexpr int kMaxScount = 4096;
+constexpr int kMaxDevices = 64;  // function attributes are per device: launchers keep their one-time set-up per device
 
 struct slm_ctx {
     int device = 0;
@@ -55,6 +56,7 @@ struct slm_ctx {
     int64_t launches = 0;
     int64_t tma_launches = 0;
     bool timing = false;
+    bool newton_smem_set = false;  // the Newton kernels' dynamic shared-memory limits are raised on this device
     Family fam[FAM_COUNT];
     int* d_counter = nullptr;
     int* h_counter = nullptr;
@@ -196,7 +198,10 @@ template <int WM, int WN, int MI, int NI, bool AM, bool SYM, int MINB, bool KSP 
 static cudaError_t launch_gemm_t(slm_ctx* ctx, GemmBatch& b, cudaStream_t s) {
     using Cfg = GemmCfg<WM, WN, MI, NI, BK, STAGES, AM>;
     auto kern = gemm_f64_kernel<WM, WN, MI, NI, BK, STAGES, AM, SYM, MINB, KSP>;
-    static int occupancy = 0;  // resident CTAs per SM (the spin-wait fix-up needs co-residency)
+    // resident CTAs per SM (the spin-wait fix-up needs co-residency); the shared-memory limit is raised per device
+    static int occupancy_of[kMaxDevices] = {};
+    if (ctx->device >= kMaxDevices) return cudaErrorInvalidDevice;
+    int& occupancy = occupancy_of[ctx->device];
     if (occupancy == 0) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              (int)Cfg::SMEM);
@@ -263,7 +268,9 @@ template <int WM, int WN, int MI, int NI, bool SYM, int MINB, bool KSP, int BK, 
 static cudaError_t launch_gemm_tma_w(slm_ctx* ctx, GemmBatch& b, cudaStream_t s) {
     using Cfg = TmaCfg<WM, WN, MI, NI, BK, STAGES, WIDE>;
     auto kern = gemm_f64_tma_kernel<WM, WN, MI, NI, BK, STAGES, SYM, MINB, KSP, WIDE>;
-    static int occupancy = 0;
+    static int occupancy_of[kMaxDevices] = {};  // per device, like the shared-memory limit it is measured with
+    if (ctx->device >= kMaxDevices) return cudaErrorInvalidDevice;
+    int& occupancy = occupancy_of[ctx->device];
     if (occupancy == 0) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
         if (e != cudaSuccess) return e;
@@ -1995,12 +2002,12 @@ int slm_newton_step(slm_ctx* ctx, const double* G, int64_t g_stride, int64_t pa,
     CUDA_OK(cudaMemsetAsync(info, 0, sizeof(int) * (size_t)k, s));
     CUDA_OK(cudaMemsetAsync(Z, 0, sizeof(double) * (size_t)n_folds * p * ldz, s));
 
-    static bool attr_done = false;
-    if (!attr_done) {
+    if (!ctx->newton_smem_set) {  // per device (a function attribute is set on the current device only)
         CUDA_OK(cudaFuncSetAttribute(chol_diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NW_TILE_SMEM));
         CUDA_OK(cudaFuncSetAttribute(chol_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NW_TILE_SMEM));
         CUDA_OK(cudaFuncSetAttribute(newton_linesearch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 98304));
-        attr_done = true;
+        CUDA_OK(cudaFuncSetAttribute(chol_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 98304));
+        ctx->newton_smem_set = true;
     }
     const dim3 vgrid((unsigned)((p + NW_T - 1) / NW_T), (unsigned)k);
     newton_prepare_kernel<<<k, NW_T, 0, s>>>((int)p, n_groups, gptr, X, ldv, W2, D2, NRM, U, KK, DP, ACT, MS);
@@ -2079,11 +2086,6 @@ int slm_newton_step(slm_ctx* ctx, const double* G, int64_t g_stride, int64_t pa,
     const size_t solve_smem = sizeof(double) * ((size_t)ldh + NW_NB + (NW_TS / 32) * NW_NB);
     if (solve_smem > 98304 || 2 * sizeof(double) * (size_t)n_groups > 98304)
         return fail(ctx, 1, "slm_newton_step: design too large for the solve / line-search kernels");
-    static bool attr2 = false;
-    if (!attr2) {
-        CUDA_OK(cudaFuncSetAttribute(chol_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 98304));
-        attr2 = true;
-    }
     chol_solve_kernel<<<k, NW_TS, solve_smem, s>>>(H, ldh, (int)p, ACT, MS, INV, npan, GRAD, DIR, ldv);
     newton_linesearch_kernel<<<k, NW_T, 2 * sizeof(double) * (size_t)n_groups, s>>>(
         (int)p, n_groups, gptr, X, DIR, GS, GRAD, U, KK, DP, ldv, W2, NRM, info, out);

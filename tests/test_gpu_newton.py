@@ -122,3 +122,52 @@ def test_newton_step_kernels_match_torch_model(engine):
     assert (out - ref).abs().max().item() <= 1e-7 * ref.abs().max().item()
     # inactive groups stay exactly zero
     assert torch.equal(out == 0, ref == 0)
+
+
+def test_newton_kernels_and_torch_model_give_the_same_cv_search(monkeypatch):
+    """One overlap CV batch at p_ext ~ 520, so that the Newton systems span several 64-wide panels, through the
+    engine's kernels (SLM_NEWTON_TORCH=0) and through the torch / library-Cholesky model of the same iteration
+    (=1): same status and score table, and the same amount of second-order work.  The duality-gap certificate
+    would accept the points of a descending but wrong Newton direction; the work it takes to get there is
+    where such a direction shows end to end."""
+    from types import SimpleNamespace
+
+    import torch
+    from sklearn.model_selection import KFold
+
+    from sparselm_b200.engine import get_engine
+    from sparselm_b200.model_selection import batched_cv
+
+    X, y, group_list = _overlap_problem(seed=3, n=600, p=400, G=40)
+    amax = np.abs(X.T @ y).max() / len(y)
+    est = AdaptiveOverlapGroupLasso(group_list=group_list, solver_options={"tol": 1e-10, "max_iter": 100000,
+                                                                          "newton": True})
+    p = X.shape[1]
+    ests, specs = [], []
+    for a in amax * np.array([0.03, 3e-3, 1e-3, 3e-4]):
+        est.set_params(alpha=a)
+        specs.append(est._problem_spec(p))
+        ests.append(SimpleNamespace(fit_intercept=False))
+    engine = get_engine(0)
+    folds = [te for _, te in KFold(5).split(X)]
+    Xd = torch.from_numpy(X).to(engine.device)
+    res = {}
+    for torch_model in ("0", "1"):
+        monkeypatch.setenv("SLM_NEWTON_TORCH", torch_model)
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            res[torch_model] = batched_cv(engine, Xd, y, folds, ests, specs, dict(est._engine_options()),
+                                          "neg_root_mean_squared_error")
+    a, b = res["0"], res["1"]
+    assert len(specs[0].ext_idx) > 6 * 64
+    assert max(int((a["warm"][ci] != 0).sum()) for ci in range(len(specs))) > 2 * 64  # multi-panel systems
+    np.testing.assert_array_equal(a["info"]["status"], b["info"]["status"])
+    assert (a["info"]["status"] == 0).all()
+    np.testing.assert_allclose(a["test_scores"], b["test_scores"], rtol=1e-6)
+    na, nb = a["newton"], b["newton"]
+    counts = (na, nb, a["iters_run"], b["iters_run"])
+    assert na["factorizations"] > 0 and abs(na["phases"] - nb["phases"]) <= 1, counts
+    assert abs(na["factorizations"] - nb["factorizations"]) <= 0.05 * nb["factorizations"] + 2, counts
+    assert abs(a["iters_run"] - b["iters_run"]) <= 0.05 * b["iters_run"] + 20, counts
+    ia, ib = a["info"]["n_iter"].sum(), b["info"]["n_iter"].sum()
+    assert abs(ia - ib) <= 0.05 * ib + 20, (ia, ib)

@@ -96,3 +96,58 @@ def test_newton_phase_columns_on_different_grams():
                             torch.ones(3), 1e-10, chol_batched=False)
     for k in range(3):
         assert np.abs(Xn[k].numpy() - refs[k]).max() <= 1e-8 * np.abs(refs[k]).max()
+
+
+def _step_problem(seed, p=150, F=2, K=9):
+    """Groups of 1..12 features (a run of singletons included), two Grams, per-column n, ridge on some
+    columns, start points with a few active groups per column (a far, heavily weighted one among them)."""
+    rng = np.random.default_rng(seed)
+    sizes = list(rng.integers(2, 13, 14)) + [1] * 20
+    sizes.append(p - sum(sizes))
+    gptr = np.concatenate([[0], np.cumsum(sizes)])
+    Gn = len(sizes)
+    Gs = np.zeros((F, p + 2, p + 2))
+    for f in range(F):
+        n = 3 * p
+        X = rng.standard_normal((n, p))
+        y = X @ (rng.standard_normal(p) * (rng.random(p) < 0.2)) + 0.3 * rng.standard_normal(n)
+        Xa = np.hstack([X, y[:, None], np.ones((n, 1))])
+        Gs[f] = Xa.T @ Xa
+    fold = rng.integers(0, F, K)
+    n_obs = 3 * p * (0.5 + rng.random(K))
+    w2 = 0.05 * (0.5 + rng.random((K, Gn)))
+    d2 = (rng.random((K, Gn)) < 0.3) * 0.2
+    X0 = np.zeros((K, p))
+    for c in range(K):
+        for g in rng.choice(Gn, 10, replace=False):
+            X0[c, gptr[g]:gptr[g + 1]] = rng.standard_normal(sizes[g])
+    X0[0] *= 1e-3                                                    # far from the optimum, strong penalty:
+    w2[0] *= 40.0                                                    # the line search has to backtrack
+    return Gs, gptr, fold, n_obs, X0, w2, d2
+
+
+@pytest.mark.parametrize("ridge", [False, True])
+def test_newton_reference_matches_newton_phase_after_one_step(ridge):
+    """tests/newton_reference.py (float64 numpy / scipy, the kernels' line-search formulas) against the torch
+    model of the phase after one step: same accept decisions, same points up to rounding."""
+    import newton_reference as NR
+
+    Gs, gptr, fold, n_obs, X0, w2, d2 = _step_problem(11)
+    d2 = d2 if ridge else None
+    K, p = X0.shape
+    gid = torch.from_numpy(NR.group_ids(gptr))
+    Xn, info = newton_phase(torch.from_numpy(Gs), torch.from_numpy(fold), torch.from_numpy(n_obs), torch.from_numpy(X0),
+                            torch.from_numpy(w2), None if d2 is None else torch.from_numpy(d2), gid, torch.ones(K),
+                            1e-10, max_steps=1)
+    Xn = Xn.numpy()
+    ts = []
+    for c in range(K):
+        ref = NR.newton_step(Gs[fold[c]], p, n_obs[c], X0[c], w2[c], None if d2 is None else d2[c], gptr)
+        assert ref["ok"] and ref["accepted"] == bool(info["steps"][c] == 1)
+        assert np.abs(Xn[c] - ref["x_new"]).max() <= 1e-10 * np.abs(X0[c]).max()
+        assert np.array_equal(Xn[c] != 0, X0[c] != 0)
+        ts.append(ref["t"])
+        if ref["accepted"]:
+            assert NR.objective_change(Gs[fold[c]], p, n_obs[c], X0[c], ref["x_new"], w2[c],
+                                       None if d2 is None else d2[c], gptr) <= NR.ARMIJO / 2 * ref["t"] * -ref["dec"]
+    assert min(ts) < 1.0 and max(ts) == 1.0                           # a backtracked and a full step among them
