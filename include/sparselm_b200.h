@@ -253,7 +253,8 @@ int slm_intercepts(slm_ctx* ctx, const double* G_dev, int64_t pa, int64_t p,
                    const double* B_dev, int64_t ldz, int32_t K, double* intercept_dev,
                    void* stream);
 
-/* Second-order phase of the batched solve (pure group penalties; DESIGN section 2 item 13): ONE
+/* Second-order phase of the batched solve (pure group penalties; slm_newton_step_l1 below adds the l1 term;
+ * DESIGN section 2 item 13): ONE
  * lock-step damped Newton step on the active groups of k columns, in this library's kernels --
  * Hessian assembly from the Gram, batched blocked Cholesky (trailing updates on the tensor-core
  * GEMM), blocked triangular solves, Armijo line search on objective differences.
@@ -267,6 +268,19 @@ int slm_newton_step(slm_ctx* ctx, const double* G_dev, int64_t g_stride, int64_t
                     int32_t k, const int32_t* fold_host, const double* nobs_dev, double* X_dev,
                     const double* W2_dev, const double* D2_dev, const int32_t* gptr_dev, const int32_t* gid_dev,
                     int32_t n_groups, void* work_dev, size_t work_bytes, double* out_dev, void* stream);
+
+/* The same step for penalties with an l1 term (Lasso, SparseGroupLasso and their adaptive variants):
+ * W1_dev [k][ldv] holds every column's per-coordinate l1 weights in solver feature order (NULL: pure group
+ * penalty, bitwise the same as slm_newton_step).  On the manifold of fixed signs a coordinate is active iff it
+ * is non-zero; the line search starts from min(1, t_cross), t_cross the first step length at which a
+ * coordinate changes sign, and a step accepted at t_cross stores the coordinates that reach zero as exact
+ * zeros (out_dev[c][1] reports the step taken).  Without a group structure pass one group of all p
+ * coordinates with zero weight.  Same workspace as slm_newton_step. */
+int slm_newton_step_l1(slm_ctx* ctx, const double* G_dev, int64_t g_stride, int64_t pa, int64_t p, int n_folds,
+                       int32_t k, const int32_t* fold_host, const double* nobs_dev, double* X_dev,
+                       const double* W2_dev, const double* D2_dev, const double* W1_dev, const int32_t* gptr_dev,
+                       const int32_t* gid_dev, int32_t n_groups, void* work_dev, size_t work_bytes, double* out_dev,
+                       void* stream);
 
 /* Unpenalised least squares on a Gram (OrdinaryLeastSquares, reference model/_ols.py:57-65:
  * argmin 1/(2n) ||X b - y||^2): conjugate gradients on G b = c, c = row p of the Gram, every

@@ -99,6 +99,8 @@ SYMBOLS = {
     "slm_newton_workspace": (c_sz, [c_i64, c_i32, c_i32, ctypes.c_int]),
     "slm_newton_step": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, ctypes.c_int, c_i32, ctypes.POINTER(c_i32), c_vp, c_vp,
                                        c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_sz, c_vp, c_vp]),
+    "slm_newton_step_l1": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, ctypes.c_int, c_i32, ctypes.POINTER(c_i32), c_vp,
+                                          c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_sz, c_vp, c_vp]),
     "slm_gram_cg_workspace": (c_sz, [c_i64]),
     "slm_gram_cg": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_dbl, c_i32, c_vp, c_sz, c_vp, ctypes.POINTER(c_i32), ctypes.POINTER(c_dbl), c_vp]),
     "slm_rowsparse_workspace": (c_sz, [c_i64, c_i64, ctypes.c_int]),

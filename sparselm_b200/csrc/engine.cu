@@ -1960,10 +1960,11 @@ size_t slm_newton_workspace(int64_t p, int32_t n_groups, int32_t k, int n_folds)
     return d * sizeof(double) + (4 * kk + kk * ldh + 64) * sizeof(int) + 256;  // fold, slot, info, MS, ACT
 }
 
-int slm_newton_step(slm_ctx* ctx, const double* G, int64_t g_stride, int64_t pa, int64_t p, int n_folds,
-                    int32_t k, const int32_t* fold_host, const double* nobs_dev, double* X, const double* W2,
-                    const double* D2, const int32_t* gptr, const int32_t* gid, int32_t n_groups, void* work,
-                    size_t work_bytes, double* out, void* stream) {
+// slm_newton_step is the W1 = NULL case of slm_newton_step_l1 (the kernels branch on W1 only)
+static int newton_step_impl(slm_ctx* ctx, const double* G, int64_t g_stride, int64_t pa, int64_t p, int n_folds,
+                            int32_t k, const int32_t* fold_host, const double* nobs_dev, double* X, const double* W2,
+                            const double* D2, const double* W1, const int32_t* gptr, const int32_t* gid,
+                            int32_t n_groups, void* work, size_t work_bytes, double* out, void* stream) {
     if (!ctx || !G || !fold_host || !nobs_dev || !X || !W2 || !gptr || !gid || !work || !out)
         return fail(ctx, 1, "slm_newton_step: null argument");
     if (k <= 0) return 0;
@@ -2010,14 +2011,14 @@ int slm_newton_step(slm_ctx* ctx, const double* G, int64_t g_stride, int64_t pa,
         ctx->newton_smem_set = true;
     }
     const dim3 vgrid((unsigned)((p + NW_T - 1) / NW_T), (unsigned)k);
-    newton_prepare_kernel<<<k, NW_T, 0, s>>>((int)p, n_groups, gptr, X, ldv, W2, D2, NRM, U, KK, DP, ACT, MS);
+    newton_prepare_kernel<<<k, NW_T, 0, s>>>((int)p, n_groups, gptr, X, ldv, W2, D2, W1, NRM, U, KK, DP, ACT, MS);
     std::vector<int> ms((size_t)k);
     CUDA_OK(cudaMemcpyAsync(ms.data(), MS, sizeof(int) * (size_t)k, cudaMemcpyDeviceToHost, s));
     newton_pack_kernel<<<vgrid, NW_T, 0, s>>>((int)p, fold_dev, slot_dev, X, ldv, Z, ldz);
     LAUNCH_OK("newton prepare/pack kernels");
     if (int rc = apply_batched(ctx, G, g_stride, pa, p, n_folds, Kf.data(), Z, ldz, GZ, s, -1.0, FAM_LIPS)) return rc;
     newton_grad_kernel<<<vgrid, NW_T, 0, s>>>((int)p, G, g_stride, pa, fold_dev, slot_dev, nobs_dev, X, GZ, ldz, ldv, KK,
-                                              DP, GS, GRAD);
+                                              DP, W1, GS, GRAD);
     // the host learns the matrix sizes (the gradient's Gram apply runs meanwhile): the factorisation works on
     // the active coordinates of every column, sum_c m_c^3/3 flops instead of k p^3/3
     CUDA_OK(cudaStreamSynchronize(s));
@@ -2088,10 +2089,26 @@ int slm_newton_step(slm_ctx* ctx, const double* G, int64_t g_stride, int64_t pa,
         return fail(ctx, 1, "slm_newton_step: design too large for the solve / line-search kernels");
     chol_solve_kernel<<<k, NW_TS, solve_smem, s>>>(H, ldh, (int)p, ACT, MS, INV, npan, GRAD, DIR, ldv);
     newton_linesearch_kernel<<<k, NW_T, 2 * sizeof(double) * (size_t)n_groups, s>>>(
-        (int)p, n_groups, gptr, X, DIR, GS, GRAD, U, KK, DP, ldv, W2, NRM, info, out);
+        (int)p, n_groups, gptr, X, DIR, GS, GRAD, U, KK, DP, ldv, W2, NRM, W1, info, out);
     LAUNCH_OK("newton solve / line-search kernels");
     ctx->launches += 1;
     return 0;
+}
+
+int slm_newton_step(slm_ctx* ctx, const double* G, int64_t g_stride, int64_t pa, int64_t p, int n_folds,
+                    int32_t k, const int32_t* fold_host, const double* nobs_dev, double* X, const double* W2,
+                    const double* D2, const int32_t* gptr, const int32_t* gid, int32_t n_groups, void* work,
+                    size_t work_bytes, double* out, void* stream) {
+    return newton_step_impl(ctx, G, g_stride, pa, p, n_folds, k, fold_host, nobs_dev, X, W2, D2, nullptr, gptr, gid,
+                            n_groups, work, work_bytes, out, stream);
+}
+
+int slm_newton_step_l1(slm_ctx* ctx, const double* G, int64_t g_stride, int64_t pa, int64_t p, int n_folds,
+                       int32_t k, const int32_t* fold_host, const double* nobs_dev, double* X, const double* W2,
+                       const double* D2, const double* W1, const int32_t* gptr, const int32_t* gid, int32_t n_groups,
+                       void* work, size_t work_bytes, double* out, void* stream) {
+    return newton_step_impl(ctx, G, g_stride, pa, p, n_folds, k, fold_host, nobs_dev, X, W2, D2, W1, gptr, gid,
+                            n_groups, work, work_bytes, out, stream);
 }
 
 int slm_adaptive_update(slm_ctx* ctx, const double* B, int64_t p, int64_t ldz, int32_t K, int32_t n_groups,

@@ -16,6 +16,15 @@
 // Layouts: X, GX, U, KK, DP, GRAD, DIR are [k][ldv] (one row per column, solver feature order); ACT is
 // [k][ldv] int; H is [k][ldh][ldh] row-major over the compacted coordinates (ldh from the largest m_c), upper
 // triangle = the factor U after factorisation; group tables W2, D2, NRM are [k][Gn].
+//
+// Penalties with an l1 term (W1 [k][ldv] of per-coordinate l1 weights; NULL = pure group penalty): on the manifold
+// where the signs s_j of the non-zero coordinates are fixed the objective gains the linear term sum_j w1_j s_j x_j,
+//     grad += w1 * s   (no curvature: H is unchanged),
+// and a coordinate is active iff x_j != 0 (a zero coordinate of an active group is inactive).  The line search
+// starts from t0 = min(1, t_cross), t_cross = min{ -x_j/d_j : x_j d_j < 0 } the first sign change along the ray,
+// so the l1 term stays linear over every tried step; a step accepted at t_cross stores the coordinates that reach
+// zero as exact zeros (the support shrinks; it never grows here, that is the first-order iterations' job).
+// Lasso has no group table: the caller passes one group of all p coordinates with zero weight.
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
@@ -39,10 +48,43 @@ __device__ __forceinline__ double nw_block_sum(double v, double* red) {
     return t;
 }
 
-// per column: group norms, activity, u = x/||x_g||, kk = w_g/||x_g||, dp = d_g (active coordinates)
+__device__ __forceinline__ double nw_block_min(double v, double* red) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(0xffffffffu, v, o));
+    const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+    __syncthreads();
+    if (l == 0) red[w] = v;
+    __syncthreads();
+    double t = (l < NW_T / 32) ? red[l] : INFINITY;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) t = fmin(t, __shfl_xor_sync(0xffffffffu, t, o));
+    return t;
+}
+
+// step length at which coordinate j of x + t d reaches zero; +inf when it moves away from zero or stays
+__device__ __forceinline__ double nw_cross(double xj, double dj) { return xj * dj < 0.0 ? -xj / dj : INFINITY; }
+
+// u, kk, dp of one coordinate of a group with norm nrm, weight w, ridge d (kk = -1 marks an inactive coordinate)
+__device__ __forceinline__ void nw_coord(long long e, double xj, double nrm, double w, double d, bool l1,
+                                         double* __restrict__ U, double* __restrict__ KK, double* __restrict__ DP) {
+    if (nrm > 0.0 && (!l1 || xj != 0.0)) {
+        U[e] = xj / nrm;
+        KK[e] = w / nrm;
+        DP[e] = d;
+    } else {
+        U[e] = 0.0;
+        KK[e] = -1.0;
+        DP[e] = 0.0;
+    }
+}
+
+// per column: group norms, activity, u = x/||x_g||, kk = w_g/||x_g||, dp = d_g (active coordinates); with l1
+// weights (W1 != NULL) a zero coordinate is inactive even in an active group.  A single group with l1 weights
+// (Lasso's zero-weight group of all p coordinates) is worked on by the whole block instead of one thread.
 __global__ void __launch_bounds__(NW_T) newton_prepare_kernel(int p, int Gn, const int* __restrict__ gptr,
                                                               const double* __restrict__ X, long long ldv,
                                                               const double* __restrict__ W2, const double* __restrict__ D2,
+                                                              const double* __restrict__ W1,
                                                               double* __restrict__ NRM, double* __restrict__ U,
                                                               double* __restrict__ KK, double* __restrict__ DP,
                                                               int* __restrict__ ACT, int* __restrict__ MS) {
@@ -50,7 +92,18 @@ __global__ void __launch_bounds__(NW_T) newton_prepare_kernel(int p, int Gn, con
     const double* x = X + (long long)c * ldv;
     __shared__ int wtot[NW_T / 32];
     __shared__ int base_s;
-    for (int g = threadIdx.x; g < Gn; g += NW_T) {
+    __shared__ double red[NW_T / 32];
+    const bool l1 = W1 != nullptr, whole = l1 && Gn == 1;
+    if (whole) {
+        const int ja = gptr[0], jb = gptr[1];
+        double ss = 0.0;
+        for (int j = ja + threadIdx.x; j < jb; j += NW_T) ss += x[j] * x[j];
+        const double nrm = sqrt(nw_block_sum(ss, red));
+        if (threadIdx.x == 0) NRM[c] = nrm;
+        const double w = W2[c], d = D2 ? D2[c] : 0.0;
+        for (int j = ja + threadIdx.x; j < jb; j += NW_T) nw_coord((long long)c * ldv + j, x[j], nrm, w, d, true, U, KK, DP);
+    }
+    for (int g = whole ? Gn : threadIdx.x; g < Gn; g += NW_T) {
         const int ja = gptr[g], jb = gptr[g + 1];
         double ss = 0.0;
         for (int j = ja; j < jb; ++j) ss += x[j] * x[j];
@@ -58,18 +111,7 @@ __global__ void __launch_bounds__(NW_T) newton_prepare_kernel(int p, int Gn, con
         NRM[(long long)c * Gn + g] = nrm;
         const double w = W2[(long long)c * Gn + g];
         const double d = D2 ? D2[(long long)c * Gn + g] : 0.0;
-        for (int j = ja; j < jb; ++j) {
-            const long long e = (long long)c * ldv + j;
-            if (nrm > 0.0) {
-                U[e] = x[j] / nrm;
-                KK[e] = w / nrm;
-                DP[e] = d;
-            } else {
-                U[e] = 0.0;
-                KK[e] = -1.0;  // marks an inactive coordinate
-                DP[e] = 0.0;
-            }
-        }
+        for (int j = ja; j < jb; ++j) nw_coord((long long)c * ldv + j, x[j], nrm, w, d, l1, U, KK, DP);
     }
     // ordered list of the active coordinates (block-wide compaction, 256 coordinates per round)
     if (threadIdx.x == 0) base_s = 0;
@@ -105,15 +147,15 @@ __global__ void __launch_bounds__(NW_T) newton_pack_kernel(int p, const int* __r
     Z[((long long)fold[c] * p + j) * ldz + slot[c]] = X[(long long)c * ldv + j];
 }
 
-// gradient on the active coordinates from GX = G x:  grad = (Gx - c)/n + kk x + dp x  (kk x = w u)
-// gs (the quadratic part, stored in GS) is kept for the line search; GZ = G Z in the apply's layout
+// gradient on the active coordinates from GX = G x:  grad = (Gx - c)/n + kk x + dp x  (kk x = w u), plus w1 sign(x)
+// with l1 weights; gs (the quadratic part, stored in GS) is kept for the line search; GZ = G Z in the apply's layout
 __global__ void __launch_bounds__(NW_T) newton_grad_kernel(int p, const double* __restrict__ G, long long g_stride,
                                                            long long pa, const int* __restrict__ fold,
                                                            const int* __restrict__ slot, const double* __restrict__ nobs,
                                                            const double* __restrict__ X, const double* __restrict__ GZ,
                                                            long long ldz, long long ldv, const double* __restrict__ KK,
-                                                           const double* __restrict__ DP, double* __restrict__ GS,
-                                                           double* __restrict__ GRAD) {
+                                                           const double* __restrict__ DP, const double* __restrict__ W1,
+                                                           double* __restrict__ GS, double* __restrict__ GRAD) {
     const int c = blockIdx.y;
     const int j = blockIdx.x * NW_T + threadIdx.x;
     if (j >= p) return;
@@ -129,7 +171,9 @@ __global__ void __launch_bounds__(NW_T) newton_grad_kernel(int p, const double* 
     const double gx = GZ[((long long)fold[c] * p + j) * ldz + slot[c]];  // (G x)_j in the apply's layout
     const double gs = (gx - cj) / n;
     GS[e] = gs;
-    GRAD[e] = gs + (kk + DP[e]) * X[e];
+    double g = gs + (kk + DP[e]) * X[e];
+    if (W1) g += copysign(W1[e], X[e]);  // active: x_j != 0
+    GRAD[e] = g;
 }
 
 // H[c][i][j] over the compacted coordinates i, j < m_c (original indices ACT[c][i], ACT[c][j]): the upper
@@ -433,6 +477,8 @@ __global__ void __launch_bounds__(NW_TS) chol_solve_kernel(const double* __restr
 
 // Armijo backtracking on phi(x + t d) - phi(x) (formed without cancellation), one block per column.
 // q2 = d'(G_AA/n)d comes from the Newton system itself: d'Hd = -grad'd, H = G_AA/n + curvature terms.
+// With l1 weights backtracking starts at min(1, t_cross) and the l1 difference t sum_j w1_j s_j d_j joins dphi;
+// a step accepted at t_cross sets the coordinates that cross (nw_cross(x_j, d_j) <= t) to exactly zero.
 // out[c] = {accepted (0/1), t, decrement = -grad'd, 0}.  X is updated in place when accepted.
 __global__ void __launch_bounds__(NW_T) newton_linesearch_kernel(int p, int Gn, const int* __restrict__ gptr,
                                                                  double* __restrict__ X, const double* __restrict__ DIR,
@@ -440,7 +486,8 @@ __global__ void __launch_bounds__(NW_T) newton_linesearch_kernel(int p, int Gn, 
                                                                  const double* __restrict__ U, const double* __restrict__ KK,
                                                                  const double* __restrict__ DP, long long ldv,
                                                                  const double* __restrict__ W2, const double* __restrict__ NRM,
-                                                                 const int* __restrict__ info, double* __restrict__ out) {
+                                                                 const double* __restrict__ W1, const int* __restrict__ info,
+                                                                 double* __restrict__ out) {
     extern __shared__ double sh[];  // g1[Gn], g2[Gn]
     __shared__ double red[NW_T / 32];
     __shared__ double tsel;
@@ -450,7 +497,35 @@ __global__ void __launch_bounds__(NW_T) newton_linesearch_kernel(int p, int Gn, 
     double* x = X + (long long)c * ldv;
     const double* d = DIR + (long long)c * ldv;
     double q1 = 0.0, gd = 0.0, r1 = 0.0, r2 = 0.0, cdd = 0.0;
-    for (int g = tid; g < Gn; g += NW_T) {
+    const bool whole = W1 != nullptr && Gn == 1;  // Lasso's single group: the whole block walks its coordinates
+    if (whole) {
+        double a1 = 0.0, a2 = 0.0, ud = 0.0;
+        for (int j = gptr[0] + tid; j < gptr[1]; j += NW_T) {
+            const long long e = (long long)c * ldv + j;
+            const double dj = d[j], xj = x[j];
+            a1 += xj * dj;
+            a2 += dj * dj;
+            q1 += GS[e] * dj;
+            gd += GRAD[e] * dj;
+            const double kk = KK[e];
+            if (kk >= 0.0) {
+                r1 += DP[e] * xj * dj;
+                r2 += DP[e] * dj * dj;
+                cdd += (kk + DP[e]) * dj * dj;
+                ud += U[e] * dj;
+            }
+        }
+        a1 = nw_block_sum(a1, red);
+        a2 = nw_block_sum(a2, red);
+        ud = nw_block_sum(ud, red);
+        if (tid == 0) {
+            const double nrm = NRM[c];
+            cdd -= (nrm > 0.0 ? W2[c] / nrm : 0.0) * ud * ud;  // the group's kk, as newton_prepare_kernel forms it
+            g1[0] = a1;
+            g2[0] = a2;
+        }
+    }
+    for (int g = whole ? Gn : tid; g < Gn; g += NW_T) {
         const int ja = gptr[g], jb = gptr[g + 1];
         double a1 = 0.0, a2 = 0.0, ud = 0.0, kkg = 0.0;
         for (int j = ja; j < jb; ++j) {
@@ -482,6 +557,18 @@ __global__ void __launch_bounds__(NW_T) newton_linesearch_kernel(int p, int Gn, 
     const double q2 = dec - cdd;  // d'(G_AA/n)d
     const bool usable = info[c] == 0 && dec > 0.0 && isfinite(dec);
     double t = 1.0;
+    double l1d = 0.0;  // sum_j w1_j s_j d_j: the l1 term's slope along d up to the first sign change
+    if (W1) {
+        double tc = INFINITY;
+        for (int j = tid; j < p; j += NW_T) {
+            const long long e = (long long)c * ldv + j;
+            if (KK[e] >= 0.0) l1d += copysign(W1[e], x[j]) * d[j];
+            tc = fmin(tc, nw_cross(x[j], d[j]));
+        }
+        l1d = nw_block_sum(l1d, red);
+        tc = nw_block_min(tc, red);
+        t = fmin(1.0, tc);
+    }
     bool accepted = false;
     if (usable) {
         for (int ls = 0; ls < 24 && !accepted; ++ls) {
@@ -494,7 +581,8 @@ __global__ void __launch_bounds__(NW_T) newton_linesearch_kernel(int p, int Gn, 
                 dpen += W2[(long long)c * Gn + g] * dsq / (nn + safe);
             }
             dpen = nw_block_sum(dpen, red);
-            const double dphi = t * q1 + 0.5 * t * t * q2 + t * r1 + 0.5 * t * t * r2 + dpen;
+            double dphi = t * q1 + 0.5 * t * t * q2 + t * r1 + 0.5 * t * t * r2 + dpen;
+            if (W1) dphi += t * l1d;
             if (dphi <= 1e-4 * t * gd)
                 accepted = true;
             else
@@ -504,8 +592,13 @@ __global__ void __launch_bounds__(NW_T) newton_linesearch_kernel(int p, int Gn, 
     if (tid == 0) tsel = accepted ? t : 0.0;
     __syncthreads();
     const double ts = tsel;
-    if (ts > 0.0)
-        for (int j = tid; j < p; j += NW_T) x[j] += ts * d[j];
+    if (ts > 0.0) {
+        if (W1) {
+            for (int j = tid; j < p; j += NW_T) x[j] = nw_cross(x[j], d[j]) <= ts ? 0.0 : x[j] + ts * d[j];
+        } else {
+            for (int j = tid; j < p; j += NW_T) x[j] += ts * d[j];
+        }
+    }
     if (tid == 0) {
         out[4 * c + 0] = accepted ? 1.0 : 0.0;
         out[4 * c + 1] = ts;

@@ -188,6 +188,10 @@ class Engine:
     # 200/100 457 ms per search)
     NEWTON_FIRST = int(os.environ.get("SLM_NEWTON_FIRST", 300))
     NEWTON_LATER = int(os.environ.get("SLM_NEWTON_LATER", 100))
+    # an l1 phase that removed coordinates from a column's support counts as progress, not as one of the three failed
+    # phases after which the column stays first-order: a truncated step drops about one coordinate, so a support with
+    # many spurious coordinates needs several phases (profiles/r03_newton_l1_probe.jsonl: with / without this rule)
+    NEWTON_L1_SHRINK_IS_PROGRESS = True
 
     def __init__(self, device: int | None = None):
         import torch
@@ -697,7 +701,9 @@ class Engine:
         (sparselm_b200/newton.py) between further stretches.  None (default) = on for
         160 < p <= 2048: below, the fused small-design kernel iterates at ~0.3 us per iteration;
         above, one p x p factorisation per column and step costs more than the iterations it saves
-        unless the problem is known to be ill-conditioned (then pass True).
+        unless the problem is known to be ill-conditioned (then pass True).  "l1": the same phase for
+        every penalty, including those with an l1 term (Lasso, SparseGroupLasso and their adaptive
+        variants: Newton steps on the manifold of fixed signs); for a pure group penalty the same as True.
 
         W1_init: optional device tensor [F, p, ldz] of per-coordinate l1 weights (instead of the
         per-column lam1; sparselm_b200/split.py).
@@ -784,6 +790,25 @@ class Engine:
                             n_obs=[float(v) for v in n_obs], Ks=Ks, status=status, n_iter=n_iter,
                             primal=primal, get_W2=lambda: W2, D2=D2, p=p, ldz=ldz, F=F, tol=tol, floor_rel=floor_rel,
                             stats={"phases": 0, "factorizations": 0, "newton_columns": 0, "ms": 0.0})
+        has_l1 = W1_init is not None or (ad is not None and ad.get("a1") is not None) or bool(np.any(np.concatenate(
+            [np.asarray(g.lam1, dtype=float).ravel() for g in grids]) != 0.0))
+        if nctx is None and isinstance(newton, str) and newton == "l1" and has_l1 and (g0.gptr is not None or (W2 is None and D2 is None)):
+            if g0.gptr is None:  # no group table (Lasso): one group of all p coordinates with zero weight
+                ngptr = np.array([0, p], dtype=np.int64)
+                zero_w2 = torch.zeros((F, 1, ldz), dtype=torch.float64, device=dev)
+                get_W2 = lambda: zero_w2  # noqa: E731
+            else:
+                ngptr = np.asarray(g0.gptr, dtype=np.int64)
+                get_W2 = lambda: W2 if W2 is not None else torch.zeros((F, Gn, ldz), dtype=torch.float64, device=dev)  # noqa: E731
+            lam1_full = lam1[:, None, :].expand(F, p, ldz)  # the per-column l1 weight, broadcast (no copy)
+            # the l1 weights the iterations use: W1_init, else lam1 until the adaptive passes allocate W1
+            get_W1 = lambda: W1 if W1 is not None else (W1_init if W1_init is not None and ad is None else lam1_full)  # noqa: E731
+            gid = torch.from_numpy(np.repeat(np.arange(len(ngptr) - 1), np.diff(ngptr)).astype(np.int64)).to(dev)
+            nctx = dict(Gs=Gs, B=B, gid=gid, gid32=gid.to(torch.int32),
+                        gptr_dev=self.to_device(ngptr.astype(np.int32)), n_obs=[float(v) for v in n_obs], Ks=Ks,
+                        status=status, n_iter=n_iter, primal=primal, get_W2=get_W2, get_W1=get_W1, D2=D2, p=p,
+                        ldz=ldz, F=F, tol=tol, floor_rel=floor_rel,
+                        stats={"phases": 0, "factorizations": 0, "newton_columns": 0, "ms": 0.0})
         n_pass = np.ones((F, ldz), dtype=np.int64)
         total_iters = 0
         if ad is None:
@@ -940,13 +965,15 @@ class Engine:
                     break
                 frozen |= ~slow
                 skip_ph.copy_(torch.from_numpy(frozen.astype(np.int32)))
-                # a column that three Newton phases did not finish stays with the iterations (bounded extra cost
-                # on problems the phase does not help); with no candidate left the next stretch runs to max_iter
+                # a column that three Newton phases did not finish (l1: nor shrink its support) stays with the
+                # iterations (bounded extra cost on problems the phase does not help); with no candidate left the
+                # next stretch runs to max_iter
                 fi, ki = np.nonzero(slow & (fails < 3))
                 if len(fi) == 0:
                     last = True
                     continue
                 W2, D2 = nctx["get_W2"](), nctx["D2"]
+                W1 = nctx["get_W1"]() if "get_W1" in nctx else None
                 prim = nctx["primal"].cpu().numpy()
                 floor = max(nctx["floor_rel"], 4e-15 / nctx["tol"])
                 yty = Gs[:, p, p].cpu().numpy()
@@ -961,15 +988,19 @@ class Engine:
                     X = B[fc, :, kc]
                     w2 = W2[fc, :, kc]
                     d2 = None if D2 is None else D2[fc, :, kc]
+                    w1 = None if W1 is None else W1[fc, :, kc]
                     nn = torch.tensor([nctx["n_obs"][f] for f in fi[c0:c0 + chunk]], dtype=torch.float64, device=self.device)
                     sc = torch.from_numpy(scale[c0:c0 + chunk]).to(self.device)
                     if "gptr_dev" in nctx and os.environ.get("SLM_NEWTON_TORCH", "0") != "1":
                         Xn, info = newton_phase_device(self, Gs, fc, nn, X, w2, d2, nctx["gptr_dev"], nctx["gid32"], sc,
-                                                       nctx["tol"])
+                                                       nctx["tol"], w1=w1)
                     else:  # SLM_NEWTON_TORCH=1: the torch / cuSOLVER model of the same iteration (A/B runs)
-                        Xn, info = newton_phase(Gs, fc, nn, X, w2, d2, nctx["gid"], sc, nctx["tol"])
+                        Xn, info = newton_phase(Gs, fc, nn, X, w2, d2, nctx["gid"], sc, nctx["tol"], w1=w1)
                     B[fc, :, kc] = Xn
-                    nf = ~info["finished"].cpu().numpy()
+                    nf = ~info["finished"]
+                    if w1 is not None and self.NEWTON_L1_SHRINK_IS_PROGRESS:
+                        nf &= (Xn != 0).sum(1) >= (X != 0).sum(1)
+                    nf = nf.cpu().numpy()
                     fails[fi[c0:c0 + chunk][nf], ki[c0:c0 + chunk][nf]] += 1
                     nctx["stats"]["factorizations"] += int(info["factorizations"])
                 ev1.record()

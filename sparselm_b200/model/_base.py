@@ -120,7 +120,9 @@ class EngineRegressor(RegressorMixin, BaseEstimator, metaclass=ABCMeta):
         solver (str | None): accepted and ignored (there is one solver: the engine).
         solver_options (dict | None): engine options: ``tol`` (relative duality
             gap, default 1e-10), ``max_iter``, ``check_every``, ``floor_rel``,
-            ``device``.
+            ``device``, ``newton`` (second-order phase: None = automatic for pure
+            group penalties, True / False forces it, ``"l1"`` also runs it for
+            penalties with an l1 term).
     """
 
     _parameter_constraints: dict = {
@@ -173,6 +175,9 @@ class EngineRegressor(RegressorMixin, BaseEstimator, metaclass=ABCMeta):
         if not isinstance(opts, dict):
             raise TypeError("solver_options must be a dictionary")
         known = {"tol", "max_iter", "check_every", "floor_rel", "device", "newton"}
+        nw = opts.get("newton")
+        if not (nw is None or isinstance(nw, (bool, np.bool_)) or (isinstance(nw, str) and nw == "l1")):
+            raise ValueError(f"solver_options['newton'] must be None, True, False or 'l1', got {nw!r}")
         return {k: v for k, v in opts.items() if k in known}
 
     # ---- sklearn API ---------------------------------------------------------

@@ -29,7 +29,13 @@ decreases phi (Armijo test on the *difference* of objective values, formed witho
 Scope: pure group penalties (no l1 term) with optional ridge: GroupLasso, OverlapGroupLasso,
 RidgedGroupLasso and their adaptive variants (also in whitened variables, standardize=True).
 On by default for 160 < p <= 2048 (engine.Engine.solve); ``solver_options={"newton": True / False}``
-forces it.  Measured on C4 (AdaptiveOverlapGroupLasso, 20 alphas x 5 folds x 3 passes, p_ext = 1961): 0.41 s per
+forces it.  ``solver_options={"newton": "l1"}`` also runs it for penalties with an l1 term (Lasso,
+SparseGroupLasso and their adaptive variants; not the method-of-multipliers path of standardize=True):
+steps on the manifold of fixed signs (``slm_newton_step_l1``), active set = the non-zero coordinates,
+backtracking from min(1, t_cross) and exact zeros where a coordinate reaches zero -- the support only
+shrinks.  Measured on an AR(1) rho = 0.99 design (n = 5000, p = 1000, DESIGN.md section 4,
+profiles/r03_newton_l1_probe.jsonl): AdaptiveLasso fit 85 -> 58 ms (2717 -> 300 iterations), Lasso 20 x 5
+search 384 -> 222 ms, SparseGroupLasso 20 x 5 search 430 -> 398 ms, answers equal to 2e-10.  Measured on C4 (AdaptiveOverlapGroupLasso, 20 alphas x 5 folds x 3 passes, p_ext = 1961): 0.41 s per
 search against 12.4 s first-order only (round 1 with torch / cuSOLVER: 1.25 s), 1155 iterations against 129 350,
 no column left on max_iter (6 before), scores equal to 3e-8 relative; 1384 factorisations per search on the active
 coordinates of every column (DESIGN.md section 4).
@@ -52,7 +58,7 @@ def _gsum(v, gid, n_groups):
     return out
 
 
-def newton_phase(Gs, fold, n_obs, X, w2, d2, gid, scale, tol, max_steps=12, chol_batched=True):
+def newton_phase(Gs, fold, n_obs, X, w2, d2, gid, scale, tol, max_steps=12, chol_batched=True, w1=None):
     """Lock-step damped Newton iteration for K columns.
 
     Gs [F, pa, pa] Grams (rows/cols < p: X'X, row p: X'y), fold [K] int64 (Gram of every column),
@@ -60,6 +66,11 @@ def newton_phase(Gs, fold, n_obs, X, w2, d2, gid, scale, tol, max_steps=12, chol
     weights, d2 [K, Gn] ridge weights or None, gid [p] int64 group of every feature, scale [K] =
     max(|P|, floor) of the engine's relative test, tol its tolerance: a column is finished once the
     Newton decrement says phi - phi* <= 1e-3 * tol * scale after a full step.
+
+    w1 [K, p]: per-coordinate l1 weights (None: pure group penalty).  Then the step works on the manifold of
+    fixed signs: only the non-zero coordinates are active, the gradient gains w1 * sign(x), backtracking starts
+    from min(1, t_cross) (the first sign change along the direction) and a step accepted at t_cross stores the
+    coordinates that reach zero as exact zeros.
 
     Returns (X_new [K, p], info) with info = dict(steps [K], factorizations int, finished [K] bool).
     """
@@ -86,6 +97,9 @@ def newton_phase(Gs, fold, n_obs, X, w2, d2, gid, scale, tol, max_steps=12, chol
         nrm_g = torch.sqrt(_gsum(x * x, gid, Gn))                     # [k, Gn]
         act_g = nrm_g > 0
         act = act_g.index_select(1, gid)                              # [k, p]
+        if w1 is not None:
+            w1l = w1.index_select(0, live)
+            act = act & (x != 0)
         actf = act.to(dt)
         safe = torch.where(act_g, nrm_g, torch.ones_like(nrm_g))
         nrm = safe.index_select(1, gid)
@@ -98,6 +112,8 @@ def newton_phase(Gs, fold, n_obs, X, w2, d2, gid, scale, tol, max_steps=12, chol
         Gx = torch.bmm(GA, x[:, :, None])[:, :, 0]
         gs = (Gx - cA) * actf                                         # gradient of the quadratic part
         grad = gs + wp * u + dp * x
+        if w1 is not None:
+            grad = grad + w1l * torch.sign(x)
         H = GA * actf[:, :, None] * actf[:, None, :]
         H -= same[None] * (kk * u)[:, :, None] * u[:, None, :]
         H.diagonal(dim1=1, dim2=2).add_(kk + dp + (1.0 - actf))       # identity on the inactive coordinates
@@ -123,6 +139,10 @@ def newton_phase(Gs, fold, n_obs, X, w2, d2, gid, scale, tol, max_steps=12, chol
         r1, r2 = (dp * xd).sum(1), (dp * dd).sum(1)
         g1, g2 = _gsum(xd, gid, Gn), _gsum(dd, gid, Gn)
         t = torch.ones(k, dtype=dt, device=dev)
+        if w1 is not None:
+            l1d = (w1l * torch.sign(x) * dlt).sum(1)                  # slope of the l1 term up to t_cross
+            cross = torch.where(x * dlt < 0, -x / dlt, torch.full_like(x, float("inf")))
+            t = torch.clamp(cross.min(1).values, max=1.0)
         accepted = torch.zeros(k, dtype=torch.bool, device=dev)
         usable = ok & (dec > 0)
         for _ls in range(24):                                         # Armijo backtracking, per column
@@ -130,6 +150,8 @@ def newton_phase(Gs, fold, n_obs, X, w2, d2, gid, scale, tol, max_steps=12, chol
             new_nrm = torch.sqrt(torch.clamp(nrm_g * nrm_g + dsq, min=0.0))
             dpen = (w * dsq / (new_nrm + safe)).sum(1)
             dphi = t * q1 + 0.5 * t * t * q2 + t * r1 + 0.5 * t * t * r2 + dpen
+            if w1 is not None:
+                dphi = dphi + t * l1d
             good = usable & ~accepted & (dphi <= 1e-4 * t * gd)
             accepted |= good
             t = torch.where(accepted | ~usable, t, 0.5 * t)
@@ -137,6 +159,8 @@ def newton_phase(Gs, fold, n_obs, X, w2, d2, gid, scale, tol, max_steps=12, chol
                 break
         t = torch.where(accepted, t, torch.zeros_like(t))
         x_new = x + t[:, None] * dlt
+        if w1 is not None:                                            # the coordinates that reach zero at t_cross
+            x_new = torch.where(cross <= t[:, None], torch.zeros_like(x_new), x_new)
         X.index_copy_(0, live, x_new)
         steps.index_add_(0, live, accepted.to(torch.int64))
         full = accepted & (t == 1.0)
@@ -150,10 +174,11 @@ def newton_phase(Gs, fold, n_obs, X, w2, d2, gid, scale, tol, max_steps=12, chol
     return X, {"steps": steps, "factorizations": n_fact, "finished": finished}
 
 
-def newton_phase_device(engine, Gs, fold, n_obs, X, w2, d2, gptr_dev, gid_dev, scale, tol, max_steps=12):
+def newton_phase_device(engine, Gs, fold, n_obs, X, w2, d2, gptr_dev, gid_dev, scale, tol, max_steps=12, w1=None):
     """The same lock-step iteration as ``newton_phase`` with every step done by the engine's kernels
-    (``slm_newton_step``).  Gs [F, pa, pa] device Grams, fold [K] int64, n_obs [K], X [K, p] start points,
-    w2 [K, Gn], d2 [K, Gn] or None, gptr_dev int32 [Gn+1], gid_dev int32 [p], scale [K], tol.
+    (``slm_newton_step``; ``slm_newton_step_l1`` with l1 weights).  Gs [F, pa, pa] device Grams, fold [K] int64,
+    n_obs [K], X [K, p] start points, w2 [K, Gn], d2 [K, Gn] or None, gptr_dev int32 [Gn+1], gid_dev int32 [p],
+    scale [K], tol, w1 [K, p] or None.
     One small device-to-host read per step (accepted / step length / decrement of every column)."""
     import ctypes
 
@@ -175,6 +200,10 @@ def newton_phase_device(engine, Gs, fold, n_obs, X, w2, d2, gptr_dev, gid_dev, s
     n_obs = n_obs.to(dt).contiguous()
     w2 = w2.contiguous()
     d2 = None if d2 is None else d2.contiguous()
+    W1w = None
+    if w1 is not None:
+        W1w = torch.zeros((K, ldv), dtype=dt, device=dev)
+        W1w[:, :p] = w1
     nbytes = engine.lib.slm_newton_workspace(p, Gn, K, F)
     work = torch.empty(nbytes, dtype=torch.uint8, device=dev)
     out = torch.zeros((K, 4), dtype=dt, device=dev)
@@ -191,11 +220,18 @@ def newton_phase_device(engine, Gs, fold, n_obs, X, w2, d2, gptr_dev, gid_dev, s
         nn_s = n_obs.index_select(0, ld).contiguous()
         w2_s = w2.index_select(0, ld).contiguous()
         d2_s = None if d2 is None else d2.index_select(0, ld).contiguous()
-        engine._ck(engine.lib.slm_newton_step(
-            engine.h, engine._ptr(Gs), pa * pa, pa, p, F, k, fh.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)),
-            engine._ptr(nn_s), engine._ptr(xs), engine._ptr(w2_s), engine._ptr(d2_s),
-            engine._ptr(gptr_dev), engine._ptr(gid_dev), Gn, engine._ptr(work), nbytes, engine._ptr(out), engine.stream),
-            "slm_newton_step")
+        fp = fh.ctypes.data_as(ctypes.POINTER(ctypes.c_int32))
+        if W1w is None:
+            engine._ck(engine.lib.slm_newton_step(
+                engine.h, engine._ptr(Gs), pa * pa, pa, p, F, k, fp, engine._ptr(nn_s), engine._ptr(xs),
+                engine._ptr(w2_s), engine._ptr(d2_s), engine._ptr(gptr_dev), engine._ptr(gid_dev), Gn,
+                engine._ptr(work), nbytes, engine._ptr(out), engine.stream), "slm_newton_step")
+        else:
+            w1_s = W1w.index_select(0, ld).contiguous()
+            engine._ck(engine.lib.slm_newton_step_l1(
+                engine.h, engine._ptr(Gs), pa * pa, pa, p, F, k, fp, engine._ptr(nn_s), engine._ptr(xs),
+                engine._ptr(w2_s), engine._ptr(d2_s), engine._ptr(w1_s), engine._ptr(gptr_dev), engine._ptr(gid_dev),
+                Gn, engine._ptr(work), nbytes, engine._ptr(out), engine.stream), "slm_newton_step_l1")
         info = out[:k].cpu()  # the step's only host synchronisation
         n_fact += k
         accepted = info[:, 0] > 0
