@@ -89,6 +89,16 @@ int slm_gram_blocks(slm_ctx* ctx, const double* Xa_dev, int64_t lda, const int64
 int slm_gram_block_add(slm_ctx* ctx, const double* Xa_dev, int64_t lda, int64_t r0, int64_t r1,
                        double* G_dev, void* stream);
 
+/* Gram of an arbitrary row set, for n_problems problems at once (CV splits that are not one partition of the
+ * rows): G[s] (+|-)= Xa[idx_s]^T Xa[idx_s], FP64 DMMA, upper tiles + mirror.  Xa_dev is [n][lda]; the row lists
+ * are rows_dev[row_ptr[s] .. row_ptr[s+1]) (device int32, ascending; row_ptr is a HOST array of n_problems + 1
+ * offsets); Gram s is at G_dev + s * g_stride.  accumulate == 0: G[s] is overwritten; != 0: the product is added
+ * to what G[s] holds (as slm_gram_block_add).  negate != 0: the product enters with a minus sign (with
+ * accumulate: a downdate G[s] -= Xa[idx]^T Xa[idx]).  An empty list leaves G[s] untouched.  Bit-reproducible. */
+int slm_gram_rows_update(slm_ctx* ctx, const double* Xa_dev, int64_t n, int64_t lda, int n_problems,
+                         const int64_t* row_ptr, const int32_t* rows_dev, double* G_dev, int64_t g_stride,
+                         int accumulate, int negate, void* stream);
+
 /* in place: Gtot = sum_f Gblk[f]; Gblk[f] <- Gtot - Gblk[f]  (training Gram of fold f
  * when the blocks are the CV test folds, model_selection.py:304-323). */
 int slm_gram_complement(slm_ctx* ctx, double* Gblk_dev, int n_blocks, int64_t pa,
@@ -245,6 +255,14 @@ int slm_cv_score(slm_ctx* ctx, const double* Xa_dev, int64_t lda, int64_t p, int
 int slm_cv_score_many(slm_ctx* ctx, const double* Xa_dev, int64_t lda, int64_t p, int32_t n,
                       const int64_t* r0, const int64_t* r1, const double* const* B_dev, const int64_t* ldb,
                       const int32_t* K, const double* const* intercept_dev, int32_t rows_scaled,
+                      double* const* yhat_dev, const int64_t* ldy, double* const* out_dev, void* stream);
+
+/* slm_cv_score_many with a row list per problem instead of a row range: problem i scores the n_rows[i] rows
+ * rows_dev[i][0 .. n_rows[i]) of Xa (device int32 array; rows_dev[i] is a device pointer, the other arrays are
+ * HOST arrays of length n as in slm_cv_score_many).  yhat[i] is scratch [n_rows[i] + 256][ldy[i]]. */
+int slm_cv_score_rows(slm_ctx* ctx, const double* Xa_dev, int64_t lda, int64_t p, int32_t n,
+                      const int32_t* const* rows_dev, const int64_t* n_rows, const double* const* B_dev,
+                      const int64_t* ldb, const int32_t* K, const double* const* intercept_dev, int32_t rows_scaled,
                       double* const* yhat_dev, const int64_t* ldy, double* const* out_dev, void* stream);
 
 /* intercept[k] = ybar - mu^T B[:,k] from the (uncentred) training Gram's ones row

@@ -74,6 +74,8 @@ SYMBOLS = {
     "slm_pack_design": (ctypes.c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_vp]),
     "slm_gram_blocks": (ctypes.c_int, [c_vp, c_vp, c_i64, ctypes.POINTER(c_i64), ctypes.c_int, c_vp, c_vp]),
     "slm_gram_block_add": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_vp]),
+    "slm_gram_rows_update": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, ctypes.c_int, ctypes.POINTER(c_i64), c_vp, c_vp, c_i64,
+                                            ctypes.c_int, ctypes.c_int, c_vp]),
     "slm_gram_complement": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, c_i64, c_vp, c_vp]),
     "slm_tri_size": (c_i64, [c_i64]),
     "slm_tri_pack": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, ctypes.c_int, c_vp, c_vp]),
@@ -94,6 +96,7 @@ SYMBOLS = {
     "slm_fold_back": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i32, c_vp, c_vp]),
     "slm_cv_score": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp]),
     "slm_cv_score_many": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp]),
+    "slm_cv_score_rows": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp]),
     "slm_intercepts": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp]),
     "slm_gram_apply": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, ctypes.c_int, ctypes.POINTER(c_i32), c_vp, c_i64, c_vp, c_vp]),
     "slm_newton_workspace": (c_sz, [c_i64, c_i32, c_i32, ctypes.c_int]),

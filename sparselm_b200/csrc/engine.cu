@@ -194,10 +194,10 @@ static void fill_units(GemmBatch& b, int bm, int bn, bool sym, int max_ctas, int
 }
 
 template <int WM, int WN, int MI, int NI, bool AM, bool SYM, int MINB, bool KSP = false, int BK = kBK,
-          int STAGES = kStages>
+          int STAGES = kStages, bool AG = false>
 static cudaError_t launch_gemm_t(slm_ctx* ctx, GemmBatch& b, cudaStream_t s) {
     using Cfg = GemmCfg<WM, WN, MI, NI, BK, STAGES, AM>;
-    auto kern = gemm_f64_kernel<WM, WN, MI, NI, BK, STAGES, AM, SYM, MINB, KSP>;
+    auto kern = gemm_f64_kernel<WM, WN, MI, NI, BK, STAGES, AM, SYM, MINB, KSP, AG>;
     // resident CTAs per SM (the spin-wait fix-up needs co-residency); the shared-memory limit is raised per device
     static int occupancy_of[kMaxDevices] = {};
     if (ctx->device >= kMaxDevices) return cudaErrorInvalidDevice;
@@ -217,8 +217,8 @@ static cudaError_t launch_gemm_t(slm_ctx* ctx, GemmBatch& b, cudaStream_t s) {
     if (b.n_flags > ctx->n_flags_cap) return cudaErrorInvalidValue;
     b.flags = ctx->d_flags;
     int grid = b.full_waves > 0 ? ctx->sm_count * occupancy : (b.total_units + b.units_per_cta - 1) / b.units_per_cta;
-    // row-sparse: the k extents live on the device, the CTAs partition the units themselves
-    if (KSP) grid = (int)std::min<long long>((long long)ctx->sm_count * occupancy, b.total_units);
+    // row-sparse apply: the k extents live on the device, the CTAs partition the units themselves
+    if (KSP && !SYM) grid = (int)std::min<long long>((long long)ctx->sm_count * occupancy, b.total_units);
     cudaError_t e = cudaMemsetAsync(b.flags, 0, sizeof(int) * (size_t)b.n_flags, s);
     if (e != cudaSuccess) return e;
     kern<<<grid, Cfg::NT, Cfg::SMEM, s>>>(b);
@@ -290,7 +290,7 @@ static cudaError_t launch_gemm_tma_w(slm_ctx* ctx, GemmBatch& b, cudaStream_t s)
         !make_map(ctx, &mq, b.baseQ, b.rowsQ, b.pr[0].ldq, box_rows, Cfg::B_COLS, !WIDE))
         return cudaErrorInvalidValue;
     int grid = b.full_waves > 0 ? ctx->sm_count * occupancy : (b.total_units + b.units_per_cta - 1) / b.units_per_cta;
-    if (KSP) grid = (int)std::min<long long>((long long)ctx->sm_count * occupancy, b.total_units);
+    if (KSP && !SYM) grid = (int)std::min<long long>((long long)ctx->sm_count * occupancy, b.total_units);
     cudaError_t e = cudaMemsetAsync(b.flags, 0, sizeof(int) * (size_t)b.n_flags, s);
     if (e != cudaSuccess) return e;
     kern<<<grid, Cfg::NT, Cfg::SMEM, s>>>(b, mp, mq);
@@ -429,6 +429,23 @@ static cudaError_t launch_syrk_shape(slm_ctx* ctx, int id, GemmBatch& b, cudaStr
     return cudaErrorInvalidValue;
 }
 constexpr int kNumSyrkShapes = 4;
+// gathered Gram (slm_gram_rows_update): the 128 x 128, 32-deep-slab shape of the Gram build, its rows
+// gathered by the TMA unit (tile::gather4) or by the cp.async copies
+static cudaError_t launch_syrk_rows(slm_ctx* ctx, GemmBatch& b, cudaStream_t s) {
+    if (tma_prepare(ctx, b, 1)) return launch_gemm_tma_t<2, 4, 8, 4, true, 1, true, 32, 3>(ctx, b, s);
+    return launch_gemm_t<2, 4, 8, 4, false, true, 1, true, 32, 3>(ctx, b, s);
+}
+// scoring GEMM over gathered rows of Xa (slm_cv_score_rows): the scoring menu, A rows gathered
+static cudaError_t launch_score_rows_shape(slm_ctx* ctx, int id, GemmBatch& b, cudaStream_t s) {
+    switch (id) {
+        case 0: return launch_gemm_t<2, 4, 8, 4, true, false, 1, false, kBK, kStages, true>(ctx, b, s);
+        case 1: return launch_gemm_t<4, 2, 4, 4, true, false, 2, false, kBK, kStages, true>(ctx, b, s);
+        case 2: return launch_gemm_t<8, 1, 2, 4, true, false, 2, false, kBK, kStages, true>(ctx, b, s);
+        case 3: return launch_gemm_t<8, 1, 2, 2, true, false, 2, false, kBK, kStages, true>(ctx, b, s);
+        case 4: return launch_gemm_t<8, 1, 2, 1, true, false, 2, false, kBK, kStages, true>(ctx, b, s);
+    }
+    return cudaErrorInvalidValue;
+}
 
 struct ProblemDims {
     int M, N;
@@ -834,11 +851,14 @@ __global__ void fold_back_kernel(const double* __restrict__ Be, const int* __res
 
 // K10: residual reductions, two deterministic stages.
 constexpr int SCORE_RB = 128;  // row blocks
+// GATHER: row i of the problem is row ridx[i] of Xa (r0 unused), else row r0 + i
+template <bool GATHER = false>
 __global__ void __launch_bounds__(256) score_partial_kernel(const double* __restrict__ Xa, long long lda, int p,
                                                             long long r0, long long m,
                                                             const double* __restrict__ yhat, long long ldz,
                                                             int K, const double* __restrict__ icpt,
-                                                            int rows_scaled, double* __restrict__ part) {
+                                                            int rows_scaled, double* __restrict__ part,
+                                                            const int* __restrict__ ridx = nullptr) {
     // block = 8 columns x 32 row lanes; grid = (ceil(K/8), SCORE_RB)
     const int c = threadIdx.x & 7, r = threadIdx.x >> 3;
     const int k = blockIdx.x * 8 + c;
@@ -847,7 +867,7 @@ __global__ void __launch_bounds__(256) score_partial_kernel(const double* __rest
     if (k < K) {
         const double b0 = icpt ? icpt[k] : 0.0;
         for (long long i = (long long)blockIdx.y * 32 + r; i < m; i += (long long)SCORE_RB * 32) {
-            const double* row = Xa + (r0 + i) * lda;
+            const double* row = Xa + (GATHER ? (long long)ridx[i] : r0 + i) * lda;
             double d = row[p] - yhat[i * ldz + k] - b0 * row[p + 1];
             // rows packed as sqrt(sw_i) [x_i, y_i, 1]: the scorer wants the unweighted residual
             if (rows_scaled) d /= row[p + 1];
@@ -1139,6 +1159,46 @@ static int gram_blocks_impl(slm_ctx* ctx, const double* Xa, int64_t lda, const i
         FamTimer tm(ctx, FAM_GRAM, s, flops);
         cudaError_t e = launch_syrk_shape(ctx, sid, b, s);
         if (e != cudaSuccess) return fail(ctx, 100 + (int)e, std::string("gram build: ") + cudaGetErrorString(e));
+        ctx->launches++;
+    }
+    return 0;
+}
+
+int slm_gram_rows_update(slm_ctx* ctx, const double* Xa, int64_t n, int64_t lda, int n_problems, const int64_t* row_ptr,
+                         const int32_t* rows, double* G, int64_t g_stride, int accumulate, int negate, void* stream) {
+    if (!ctx || !Xa || !row_ptr || !G) return fail(ctx, 1, "slm_gram_rows_update: null argument");
+    if (lda % 8) return fail(ctx, 1, "slm_gram_rows_update: lda must be a multiple of 8");
+    if (n_problems < 0 || g_stride < lda * lda) return fail(ctx, 1, "slm_gram_rows_update: bad problem count or stride");
+    cudaStream_t s = (cudaStream_t)stream;
+    int i = 0;
+    while (i < n_problems) {
+        GemmBatch b;
+        memset(&b, 0, sizeof(b));
+        b.accumulate = accumulate != 0;
+        b.negate = negate != 0;
+        b.baseP = b.baseQ = Xa;
+        b.rowsP = b.rowsQ = n;
+        double flops = 0.0;
+        int np = 0;
+        for (; i < n_problems && np < kMaxGemmProblems; ++i) {
+            const int64_t m = row_ptr[i + 1] - row_ptr[i];
+            if (m < 0 || m > (1LL << 30)) return fail(ctx, 1, "slm_gram_rows_update: bad row list length");
+            if (m == 0) continue;  // an empty list leaves its Gram untouched
+            if (!rows) return fail(ctx, 1, "slm_gram_rows_update: null row lists");
+            GemmProblem& pr = b.pr[np++];
+            pr.P = pr.Q = Xa;
+            pr.kidx = rows + row_ptr[i];
+            pr.C = G + (int64_t)i * g_stride;
+            pr.ldp = pr.ldq = pr.ldc = lda;
+            pr.M = pr.N = (int)lda;
+            pr.Kd = (int)m;
+            flops += (double)m * (double)lda * (double)(lda + 1);  // SYRK count
+        }
+        if (np == 0) continue;
+        b.n_problems = np;
+        FamTimer tm(ctx, FAM_GRAM, s, flops);
+        cudaError_t e = launch_syrk_rows(ctx, b, s);
+        if (e != cudaSuccess) return fail(ctx, 100 + (int)e, std::string("gram rows update: ") + cudaGetErrorString(e));
         ctx->launches++;
     }
     return 0;
@@ -2224,6 +2284,66 @@ int slm_cv_score_many(slm_ctx* ctx, const double* Xa, int64_t lda, int64_t p, in
             dim3 grid((unsigned)((K[i] + 7) / 8), SCORE_RB);
             score_partial_kernel<<<grid, 256, 0, s>>>(Xa, lda, (int)p, r0[i], m, yhat[i], ldy[i], K[i], icpt ? icpt[i] : nullptr,
                                                       rows_scaled, part);
+            score_final_kernel<<<(unsigned)((K[i] + 127) / 128), 128, 0, s>>>(part, ldy[i], K[i], out[i]);
+        }
+        LAUNCH_OK("score kernels");
+    }
+    return 0;
+}
+
+// the same with a device row list per problem instead of a row range (arbitrary CV splits)
+int slm_cv_score_rows(slm_ctx* ctx, const double* Xa, int64_t lda, int64_t p, int32_t n, const int32_t* const* rows,
+                      const int64_t* n_rows, const double* const* B, const int64_t* ldb, const int32_t* K,
+                      const double* const* icpt, int32_t rows_scaled, double* const* yhat, const int64_t* ldy,
+                      double* const* out, void* stream) {
+    if (!ctx || !Xa || !rows || !n_rows || !B || !ldb || !K || !yhat || !ldy || !out)
+        return fail(ctx, 1, "slm_cv_score_rows: null argument");
+    cudaStream_t s = (cudaStream_t)stream;
+    for (int i0 = 0; i0 < n; i0 += kMaxGemmProblems) {
+        const int nb = std::min<int>(n - i0, kMaxGemmProblems);
+        GemmBatch b;
+        memset(&b, 0, sizeof(b));
+        ProblemDims pd[kMaxGemmProblems];
+        int np = 0;
+        double flops = 0.0;
+        for (int i = i0; i < i0 + nb; ++i) {
+            const int64_t m = n_rows[i];
+            if (m <= 0 || K[i] <= 0) continue;
+            if (m > (1LL << 30)) return fail(ctx, 1, "slm_cv_score_rows: row list too long");
+            if (!rows[i] || !B[i] || !yhat[i] || !out[i] || (ldb[i] & 1) || (ldy[i] % 8) || ((uintptr_t)B[i] & 15))
+                return fail(ctx, 1, "slm_cv_score_rows: bad problem (null pointer, odd leading dimension or unaligned B)");
+            GemmProblem& pr = b.pr[np];
+            pr.P = Xa;
+            pr.kidx = rows[i];
+            pr.Q = B[i];
+            pr.C = yhat[i];
+            pr.ldp = lda;
+            pr.ldq = ldb[i];
+            pr.ldc = ldy[i];
+            pr.M = (int)m;
+            pr.N = (int)std::min<int64_t>(round_up(K[i], 8), ldy[i]);
+            pr.qlim = pr.N;
+            pr.Kd = (int)p;
+            pd[np] = {pr.M, pr.N};
+            flops += 2.0 * (double)m * (double)p * (double)K[i];
+            ++np;
+        }
+        if (np == 0) continue;
+        b.n_problems = np;
+        const int sid = pick_shape(kScoreShapes, kNumScoreShapes, pd, np, ctx->sm_count);
+        {
+            FamTimer tm(ctx, FAM_SCORE, s, flops);
+            cudaError_t e = launch_score_rows_shape(ctx, sid, b, s);
+            if (e != cudaSuccess) return fail(ctx, 100 + (int)e, std::string("score gemm: ") + cudaGetErrorString(e));
+            ctx->launches++;
+        }
+        for (int i = i0; i < i0 + nb; ++i) {
+            const int64_t m = n_rows[i];
+            if (m <= 0 || K[i] <= 0) continue;
+            double* part = yhat[i] + m * ldy[i];
+            dim3 grid((unsigned)((K[i] + 7) / 8), SCORE_RB);
+            score_partial_kernel<true><<<grid, 256, 0, s>>>(Xa, lda, (int)p, 0, m, yhat[i], ldy[i], K[i],
+                                                            icpt ? icpt[i] : nullptr, rows_scaled, part, rows[i]);
             score_final_kernel<<<(unsigned)((K[i] + 127) / 128), 128, 0, s>>>(part, ldy[i], K[i], out[i]);
         }
         LAUNCH_OK("score kernels");

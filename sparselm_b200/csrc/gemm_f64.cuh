@@ -32,6 +32,14 @@
 // loads) and, because the list length is only known on the device, every CTA
 // derives the stream-K unit partition itself from the counts.
 //
+// Gathered Gram (SYM && KSPARSE): C = Xa[idx]^T Xa[idx] for a row list idx whose length is known on
+// the host.  The contraction gathers rows as above, but the unit partition is the host-made hybrid
+// one (data-parallel waves + stream-K remainder): the device-derived pure stream-K partition of the
+// apply reads the operands once per tile instead of once per wave.
+//
+// Gathered A rows (AGATHER, A_MMAJOR only): row m of the M-major A operand is row kidx[m] of P
+// (scoring of an arbitrary row set: predictions of the rows kidx[0..M)).
+//
 // Shared-memory tiles are padded by 4 doubles per row: for the m8n8k4 fragment
 // pattern (k = lane%4, x = lane/4) a row stride == 4 or 12 (mod 16) doubles makes
 // every half-warp hit 16 distinct 8-byte banks.
@@ -120,10 +128,13 @@ struct GemmCfg {
 // SYM: problem is C = A^T A with P == Q; only tiles with tn >= tm exist and each
 // is also written transposed.
 template <int WARPS_M, int WARPS_N, int MI, int NI, int BK, int STAGES, bool A_MMAJOR, bool SYM, int MINB,
-          bool KSPARSE = false>
+          bool KSPARSE = false, bool AGATHER = false>
 __global__ void __launch_bounds__(WARPS_M* WARPS_N * 32, MINB)
     gemm_f64_kernel(const __grid_constant__ GemmBatch batch) {
-    static_assert(!(KSPARSE && (A_MMAJOR || SYM)), "row-sparse mode is for the K-major apply");
+    static_assert(!(KSPARSE && A_MMAJOR), "row-sparse mode is for the K-major contractions");
+    static_assert(!AGATHER || (A_MMAJOR && !SYM && !KSPARSE), "gathered A rows are for the M-major scoring GEMM");
+    // device-derived unit partition: the row-sparse apply, whose list lengths only the device knows
+    constexpr bool DEV_PART = KSPARSE && !SYM;
     using Cfg = GemmCfg<WARPS_M, WARPS_N, MI, NI, BK, STAGES, A_MMAJOR>;
     constexpr int BM = Cfg::BM, BN = Cfg::BN, NT = Cfg::NT;
     extern __shared__ __align__(16) double smem[];
@@ -135,10 +146,10 @@ __global__ void __launch_bounds__(WARPS_M* WARPS_N * 32, MINB)
     const int lk = lane & 3, lx = lane >> 2;
 
     // unit partition: host-made, or derived here from the device-side row counts
-    __shared__ int s_ub[KSPARSE ? kMaxGemmProblems + 1 : 1];
-    __shared__ int s_kd[KSPARSE ? kMaxGemmProblems : 1];
+    __shared__ int s_ub[DEV_PART ? kMaxGemmProblems + 1 : 1];
+    __shared__ int s_kd[DEV_PART ? kMaxGemmProblems : 1];
     int upc = batch.units_per_cta, total_units = batch.total_units;
-    if (KSPARSE) {
+    if (DEV_PART) {
         if (tid < batch.n_problems) s_kd[tid] = min(batch.pr[tid].Kd, __ldcg(batch.pr[tid].kcount));
         __syncthreads();
         if (tid == 0) {
@@ -153,11 +164,11 @@ __global__ void __launch_bounds__(WARPS_M* WARPS_N * 32, MINB)
         total_units = s_ub[batch.n_problems];
         upc = (total_units + (int)gridDim.x - 1) / (int)gridDim.x;
     }
-    const int rem0 = KSPARSE ? 0 : batch.rem_unit_begin;  // first unit of the stream-K part
+    const int rem0 = DEV_PART ? 0 : batch.rem_unit_begin;  // first unit of the stream-K part
     int u = rem0 + blockIdx.x * upc;
     const int u_end = min(total_units, u + upc);
     int wave = 0;
-    const int full_waves = KSPARSE ? 0 : batch.full_waves;
+    const int full_waves = DEV_PART ? 0 : batch.full_waves;
 
 #pragma unroll 1
     while (wave < full_waves || u < u_end) {
@@ -178,10 +189,10 @@ __global__ void __launch_bounds__(WARPS_M* WARPS_N * 32, MINB)
         } else {
 #pragma unroll 1
             for (int i = 1; i < batch.n_problems; ++i)
-                if (u >= (KSPARSE ? s_ub[i] : batch.pr[i].unit_begin)) pi = i;
-            Kd = KSPARSE ? s_kd[pi] : batch.pr[pi].Kd;
-            KT = KSPARSE ? max(1, (Kd + BK - 1) / BK) : batch.pr[pi].kt;
-            unit_begin = KSPARSE ? s_ub[pi] : batch.pr[pi].unit_begin;
+                if (u >= (DEV_PART ? s_ub[i] : batch.pr[i].unit_begin)) pi = i;
+            Kd = DEV_PART ? s_kd[pi] : batch.pr[pi].Kd;
+            KT = DEV_PART ? max(1, (Kd + BK - 1) / BK) : batch.pr[pi].kt;
+            unit_begin = DEV_PART ? s_ub[pi] : batch.pr[pi].unit_begin;
             const int local = u - unit_begin;
             tl = local / KT;
             kt0 = local - tl * KT;
@@ -276,11 +287,33 @@ __global__ void __launch_bounds__(WARPS_M* WARPS_N * 32, MINB)
                 }
             }
         };
+        // AGATHER: the source rows of the A tile are the same for every slab of the tile
+        constexpr int AG_IT = AGATHER ? (BM * (BK / 2) + NT - 1) / NT : 1;
+        long long arow[AG_IT];
+        if (AGATHER) {
+#pragma unroll
+            for (int i = 0; i < AG_IT; ++i) {
+                const int r = (tid + i * NT) / (BK / 2);
+                arow[i] = (r < BM && m0 + r < M) ? (long long)__ldg(kidx + m0 + r) : -1;
+            }
+        }
         auto load_stage = [&](int kt, int stage) {
             const int k0 = kt * BK;
             double* as = As + (size_t)stage * Cfg::A_STAGE;
             double* bs = Bs + (size_t)stage * Cfg::B_STAGE;
-            if (!A_MMAJOR) {
+            if (AGATHER) {
+                constexpr int CPR = BK / 2;
+#pragma unroll
+                for (int i = 0; i < AG_IT; ++i) {
+                    const int c = tid + i * NT;
+                    if (c < BM * CPR) {
+                        const int r = c / CPR, x = (c - r * CPR) * 2;
+                        const bool ok = arow[i] >= 0 && (k0 + x + 2 <= ldp);
+                        const double* src = ok ? (P + arow[i] * ldp + k0 + x) : P;
+                        cp_async16(as + r * Cfg::A_LD + x, src, ok);
+                    }
+                }
+            } else if (!A_MMAJOR) {
                 constexpr int CPR = BM / 2;  // 16-byte chunks per row
                 for (int c = tid; c < BK * CPR; c += NT) {
                     int r = c / CPR, x = (c - r * CPR) * 2;

@@ -114,7 +114,8 @@ struct TmaCfg {
     static_assert(A_BYTES % 128 == 0 && STAGE_BYTES % 128 == 0, "TMA destinations are 128-byte aligned");
 };
 
-// A operand K-major only (Gram build, Gram apply).  SYM / KSPARSE as in gemm_f64_kernel.
+// A operand K-major only (Gram build, Gram apply).  SYM / KSPARSE as in gemm_f64_kernel (SYM && KSPARSE:
+// the gathered Gram, host-made hybrid partition).
 // mapP / mapQ: 2-D tensor maps over the whole operand matrices (P: [rows][ldp], Q: [rows][ldq]),
 // box [BK][16] for the tiled mode, [1][16] for the gather mode.  A problem addresses its rows
 // through prow0 / qrow0 and its first P / Q columns through pcol0 / qcol0.
@@ -133,9 +134,10 @@ __global__ void __launch_bounds__((WARPS_M * WARPS_N + 4) * 32, MINB)
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
-    // unit partition: host-made, or derived here from the device-side row counts
-    __shared__ int s_ub[KSPARSE ? kMaxGemmProblems + 1 : 1];
-    __shared__ int s_kd[KSPARSE ? kMaxGemmProblems : 1];
+    // unit partition: host-made, or derived here from the device-side row counts (row-sparse apply)
+    constexpr bool DEV_PART = KSPARSE && !SYM;
+    __shared__ int s_ub[DEV_PART ? kMaxGemmProblems + 1 : 1];
+    __shared__ int s_kd[DEV_PART ? kMaxGemmProblems : 1];
     int upc = batch.units_per_cta, total_units = batch.total_units;
     if (tid == 0) {
         for (int s = 0; s < STAGES; ++s) {
@@ -144,7 +146,7 @@ __global__ void __launch_bounds__((WARPS_M * WARPS_N + 4) * 32, MINB)
         }
         mbar_fence_init();
     }
-    if (KSPARSE) {
+    if (DEV_PART) {
         if (tid < batch.n_problems) s_kd[tid] = min(batch.pr[tid].Kd, __ldcg(batch.pr[tid].kcount));
         __syncthreads();
         if (tid == 0) {
@@ -157,15 +159,15 @@ __global__ void __launch_bounds__((WARPS_M * WARPS_N + 4) * 32, MINB)
         }
     }
     __syncthreads();
-    if (KSPARSE) {
+    if (DEV_PART) {
         total_units = s_ub[batch.n_problems];
         upc = (total_units + (int)gridDim.x - 1) / (int)gridDim.x;
     }
-    const int rem0 = KSPARSE ? 0 : batch.rem_unit_begin;
+    const int rem0 = DEV_PART ? 0 : batch.rem_unit_begin;
     int u = rem0 + blockIdx.x * upc;
     const int u_end = min(total_units, u + upc);
     int wave = 0;
-    const int full_waves = KSPARSE ? 0 : batch.full_waves;
+    const int full_waves = DEV_PART ? 0 : batch.full_waves;
 
     // (problem, tile, slab range) of the next segment of this CTA -- walked identically by the
     // producer warp and by the consumer warps
@@ -190,10 +192,10 @@ __global__ void __launch_bounds__((WARPS_M * WARPS_N + 4) * 32, MINB)
         } else {
 #pragma unroll 1
             for (int i = 1; i < batch.n_problems; ++i)
-                if (u >= (KSPARSE ? s_ub[i] : batch.pr[i].unit_begin)) pi = i;
-            sg.Kd = KSPARSE ? s_kd[pi] : batch.pr[pi].Kd;
-            sg.KT = KSPARSE ? max(1, (sg.Kd + BK - 1) / BK) : batch.pr[pi].kt;
-            sg.unit_begin = KSPARSE ? s_ub[pi] : batch.pr[pi].unit_begin;
+                if (u >= (DEV_PART ? s_ub[i] : batch.pr[i].unit_begin)) pi = i;
+            sg.Kd = DEV_PART ? s_kd[pi] : batch.pr[pi].Kd;
+            sg.KT = DEV_PART ? max(1, (sg.Kd + BK - 1) / BK) : batch.pr[pi].kt;
+            sg.unit_begin = DEV_PART ? s_ub[pi] : batch.pr[pi].unit_begin;
             const int local = u - sg.unit_begin;
             sg.tl = local / sg.KT;
             sg.kt0 = local - sg.tl * sg.KT;

@@ -17,7 +17,7 @@ import numpy as np
 
 from . import _lib
 
-__all__ = ["Engine", "PenaltyGrid", "FoldData", "EngineError", "get_engine"]
+__all__ = ["Engine", "PenaltyGrid", "FoldData", "SplitData", "EngineError", "get_engine", "plan_splits", "split_chunks"]
 
 
 class EngineError(RuntimeError):
@@ -175,6 +175,94 @@ class FoldData:
                     one = torch.ones((), dtype=torch.float64, device=engine.device)
                 parts.append(one)
         return torch.stack(parts).clamp_min(1e-300) * engine.to_device(scale)
+
+
+@dataclass
+class SplitData:
+    """Device-resident problem data of a CV search whose splits are arbitrary row sets (not one
+    partition of the rows): repeated / shuffled splits, leave-one-out, time-series and grouped splits.
+
+    The training Grams are not kept: Engine.split_chunk builds those of at most SLM_MAX_FOLDS splits at
+    a time, so memory stays O(SLM_MAX_FOLDS pa^2) whatever the number of splits.  Split s is built
+    either directly from its training rows (direct[s]) or as a downdate of the full Gram by the rows
+    outside its training set (test rows and rows in neither set), whichever list is shorter; only
+    that list is stored, in one CSR array per mode (splits in order)."""
+
+    n: int
+    p: int
+    pa: int
+    Xa: object                 # torch [n, pa] augmented design, original row order
+    G_raw: object              # torch [pa, pa] uncentred Gram of all rows
+    full: FoldData             # refit data: G_full = the full Gram, centred if fit_intercept
+    direct: np.ndarray         # bool (S,): build split s from its training rows (else downdate)
+    direct_ptr: np.ndarray     # int64 CSR offsets into direct_dev, over the direct splits in order
+    direct_dev: object         # torch int32: training rows of the direct splits
+    out_ptr: np.ndarray        # int64 CSR offsets into out_dev, over the downdate splits in order
+    out_dev: object            # torch int32: rows outside the training set of the downdate splits
+    test_ptr: np.ndarray       # int64 (S+1,) CSR offsets into test_dev
+    test_dev: object           # torch int32: test rows of every split
+    n_obs: np.ndarray          # (S,) n of the 1/(2n) data term: training rows, or sum of their weights
+    n_train: np.ndarray        # (S,) training rows
+    fit_intercept: bool
+    weighted: bool
+
+    @property
+    def n_splits(self):
+        return len(self.direct)
+
+    def test_rows(self, s):
+        """Device int32 view of the test rows of split s."""
+        return self.test_dev[int(self.test_ptr[s]):int(self.test_ptr[s + 1])]
+
+    def build_rows(self, s):
+        """Device int32 view of the list split s is built from: its training rows (direct) or the rows
+        outside its training set (downdate)."""
+        j = int(np.count_nonzero(self.direct[:s]))
+        if self.direct[s]:
+            return self.direct_dev[int(self.direct_ptr[j]):int(self.direct_ptr[j + 1])]
+        k = s - j
+        return self.out_dev[int(self.out_ptr[k]):int(self.out_ptr[k + 1])]
+
+
+def split_chunks(n_splits):
+    """[s0, s1) ranges of at most SLM_MAX_FOLDS splits: the unit of the Gram build and of the solve."""
+    return [(s0, min(n_splits, s0 + _lib.SLM_MAX_FOLDS)) for s0 in range(0, n_splits, _lib.SLM_MAX_FOLDS)]
+
+
+def plan_splits(splits, n, sample_weight=None):
+    """Host side of Engine.prepare_splits: per split its build mode and the one row list that mode
+    needs, the test lists and n_obs.  splits: (train, test) index arrays, each without repeated rows.
+    Returns a dict of numpy arrays (CSR lists as int32 values and int64 offsets)."""
+    direct, dl, ol, tl, n_obs, n_train = [], [], [], [], [], []
+    for train, test in splits:
+        tr = np.sort(np.asarray(train, dtype=np.int64))
+        te = np.sort(np.asarray(test, dtype=np.int64))
+        if len(tr) and (tr[0] < 0 or tr[-1] >= n) or len(te) and (te[0] < 0 or te[-1] >= n):
+            raise ValueError("split indices out of range")
+        if np.any(np.diff(tr) == 0) or np.any(np.diff(te) == 0):
+            raise ValueError("a split repeats a row")
+        d = len(tr) <= n - len(tr)  # the training rows are at most as many as the rows outside them
+        direct.append(d)
+        if d:
+            dl.append(tr)
+        else:
+            keep = np.ones(n, dtype=bool)
+            keep[tr] = False
+            ol.append(np.flatnonzero(keep))
+        tl.append(te)
+        n_train.append(float(len(tr)))
+        n_obs.append(float(len(tr)) if sample_weight is None else float(np.asarray(sample_weight, dtype=np.float64)[tr].sum()))
+
+    def csr(lists):
+        ptr = np.concatenate([[0], np.cumsum([len(v) for v in lists])]).astype(np.int64)
+        vals = np.concatenate(lists).astype(np.int32) if lists else np.zeros(0, dtype=np.int32)
+        return ptr, vals
+
+    dptr, dvals = csr(dl)
+    optr, ovals = csr(ol)
+    tptr, tvals = csr(tl)
+    return dict(direct=np.array(direct, dtype=bool), direct_ptr=dptr, direct_rows=dvals, out_ptr=optr, out_rows=ovals,
+                test_ptr=tptr, test_rows=tvals, n_obs=np.array(n_obs), n_train=np.array(n_train))
 
 
 class Engine:
@@ -539,6 +627,81 @@ class Engine:
                                           ctypes.c_void_p(fd.Xa.data_ptr() + 8 * a * fd.pa), fd.pa, self.stream),
                  "slm_pack_design")
         part.discard(f)
+
+    def prepare_splits(self, X, y, splits, fit_intercept=False, sample_weight=None, col_perm=None):
+        """Pack the design in its original row order and build the full Gram, for a CV search over
+        arbitrary splits (list of (train, test) index arrays, no row repeated inside a split).  The
+        training Grams are built chunk by chunk later (split_chunk).  Returns a SplitData."""
+        torch = self.torch
+        if isinstance(X, torch.Tensor):
+            n, p = X.shape
+        else:
+            X = np.asarray(X)
+            n, p = X.shape
+        sw = None if sample_weight is None else np.asarray(sample_weight, dtype=np.float64)
+        plan = plan_splits(splits, n, sw)
+        row_ptr = np.array([0, n], dtype=np.int64)
+        if not (isinstance(X, torch.Tensor) and X.is_cuda) and n >= 4096:
+            Xa, allG, _ = self._prepare_pipelined(X, y, sw, col_perm, row_ptr, [(0, n)])
+        else:
+            Xa = self.pack(X, y, sw, col_perm)
+            allG = self.gram_blocks(Xa, row_ptr)
+        G_raw = allG[0]
+        G_full = G_raw
+        if fit_intercept:
+            G_full = G_raw.clone()
+            self.gram_center(G_full, p)
+        extra = {"n_obs_full": float(sw.sum()), "weighted": True} if sw is not None else {}
+        finite = torch.isfinite(G_raw[p + 1]).all()  # checked at the next host sync
+        full = FoldData(n=n, p=p, pa=Xa.shape[1], Xa=Xa, row_ptr=row_ptr, G_train=allG[:0], G_full=G_full,
+                        n_train=np.zeros(0), fit_intercept=bool(fit_intercept), extra=extra, _finite=finite)
+        dev = lambda a: self.to_device(a) if len(a) else torch.zeros(1, dtype=torch.int32, device=self.device)  # noqa: E731
+        return SplitData(n=n, p=p, pa=Xa.shape[1], Xa=Xa, G_raw=G_raw, full=full, direct=plan["direct"],
+                         direct_ptr=plan["direct_ptr"], direct_dev=dev(plan["direct_rows"]), out_ptr=plan["out_ptr"],
+                         out_dev=dev(plan["out_rows"]), test_ptr=plan["test_ptr"], test_dev=dev(plan["test_rows"]),
+                         n_obs=plan["n_obs"], n_train=plan["n_train"], fit_intercept=bool(fit_intercept),
+                         weighted=sw is not None)
+
+    def split_chunk(self, sd, s0, s1, buf):
+        """Training Grams of splits s0..s1-1 of `sd` (at most SLM_MAX_FOLDS) in buf [>= s1-s0, pa, pa],
+        centred if fit_intercept.  The direct splits take the first slots, the downdate splits the
+        others.  Returns (order, fd): order[j] = split in slot j; fd a FoldData whose G_train are those
+        slots (solve_specs, scoring and the refit take it as they take a partition's)."""
+        c = s1 - s0
+        assert 0 < c <= min(_lib.SLM_MAX_FOLDS, buf.shape[0])
+        d = sd.direct[s0:s1]
+        order = np.concatenate([s0 + np.flatnonzero(d), s0 + np.flatnonzero(~d)])
+        a = int(d.sum())
+        j0 = int(sd.direct[:s0].sum())  # direct splits before the chunk = its first entry of the direct CSR
+        k0 = s0 - j0
+        G = buf[:c]
+        if a:
+            self.gram_rows_update(sd.Xa, sd.direct_ptr[j0:j0 + a + 1], sd.direct_dev, G[:a])
+        if a < c:
+            G[a:].copy_(sd.G_raw.expand(c - a, sd.pa, sd.pa))
+            self.gram_rows_update(sd.Xa, sd.out_ptr[k0:k0 + c - a + 1], sd.out_dev, G[a:], accumulate=True, negate=True)
+        if sd.fit_intercept:
+            self.gram_center(G, sd.p)
+        extra = dict(sd.full.extra)
+        extra["n_obs_train"] = sd.n_obs[order]
+        fd = FoldData(n=sd.n, p=sd.p, pa=sd.pa, Xa=sd.Xa, row_ptr=None, G_train=G, G_full=sd.full.G_full,
+                      n_train=sd.n_train[order], fit_intercept=sd.fit_intercept, extra=extra, _finite=sd.full._finite)
+        return order, fd
+
+    def gram_rows_update(self, Xa, row_ptr, rows_dev, G, accumulate=False, negate=False):
+        """G[s] (+|-)= Xa[rows_s]^T Xa[rows_s] for every s (slm_gram_rows_update): rows_s =
+        rows_dev[row_ptr[s]:row_ptr[s+1]] (device int32, ascending; row_ptr a host array of absolute
+        offsets); accumulate=False overwrites G[s]; an empty list leaves G[s] untouched."""
+        row_ptr = np.ascontiguousarray(row_ptr, dtype=np.int64)
+        S = len(row_ptr) - 1
+        pa = Xa.shape[1]
+        Gs = G.reshape(-1, pa, pa)
+        assert Gs.shape[0] >= S and Gs.stride(0) == pa * pa and Gs.is_contiguous()
+        self._ck(self.lib.slm_gram_rows_update(self.h, self._ptr(Xa), Xa.shape[0], pa, S,
+                                               row_ptr.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)),
+                                               self._ptr(rows_dev), self._ptr(Gs), pa * pa, int(bool(accumulate)),
+                                               int(bool(negate)), self.stream), "slm_gram_rows_update")
+        return G
 
     def _gram_block_into(self, Xa, lo, hi, out, accumulate=False):
         """out (+)= Xa[lo:hi]^T Xa[lo:hi] (out untouched when the range is empty)."""
@@ -1168,6 +1331,32 @@ class Engine:
         op = vp(*[out.data_ptr() + 8 * i * 2 * ldo for i in range(n)])
         self._ck(self.lib.slm_cv_score_many(self.h, self._ptr(Xa), Xa.shape[1], p, n, r0, r1, Bp, ldb, K, ic,
                                             1 if rows_scaled else 0, yp, ldy, op, self.stream), "slm_cv_score_many")
+        return out
+
+    def cv_score_rows(self, Xa, p, items, rows_scaled=False):
+        """cv_score_many over row lists: items are (rows, B, K, intercept) with rows a device int32 view of the
+        rows of Xa to score.  Returns a device tensor [len(items), 2, ldo] (sse, sae in the first K entries)."""
+        torch = self.torch
+        n = len(items)
+        ldo = max([max(8, _round_up(int(it[2]), 8)) for it in items], default=8)
+        out = torch.zeros((max(n, 1), 2, ldo), dtype=torch.float64, device=self.device)
+        if n == 0:
+            return out
+        rows = [int(it[0].numel()) for it in items]
+        offs = np.concatenate([[0], np.cumsum([(m + 256) * ldo for m in rows])]).astype(np.int64)
+        yhat = torch.empty(int(offs[-1]), dtype=torch.float64, device=self.device)
+        i64, i32, vp = ctypes.c_int64 * n, ctypes.c_int32 * n, ctypes.c_void_p * n
+        rp = vp(*[it[0].data_ptr() for it in items])
+        nr = i64(*rows)
+        Bp = vp(*[it[1].data_ptr() for it in items])
+        ldb = i64(*[int(it[1].stride(0)) for it in items])
+        K = i32(*[int(it[2]) for it in items])
+        ic = vp(*[(None if it[3] is None else it[3].data_ptr()) for it in items])
+        yp = vp(*[yhat.data_ptr() + 8 * int(o) for o in offs[:-1]])
+        ldy = i64(*([ldo] * n))
+        op = vp(*[out.data_ptr() + 8 * i * 2 * ldo for i in range(n)])
+        self._ck(self.lib.slm_cv_score_rows(self.h, self._ptr(Xa), Xa.shape[1], p, n, rp, nr, Bp, ldb, K, ic,
+                                            1 if rows_scaled else 0, yp, ldy, op, self.stream), "slm_cv_score_rows")
         return out
 
 

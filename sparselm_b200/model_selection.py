@@ -9,13 +9,20 @@ the batched accelerated proximal-gradient solve, and the CV scores are computed
 on the device.  Anything the batched seam does not cover (foreign estimators,
 fit params, exotic scorers or splitters) takes sklearn's generic per-fit path,
 which still fits on the engine through ``estimator.fit``.
+
+Splits that are not one partition of the rows into at most 15 folds (repeated, shuffled,
+leave-one-out, time-series and grouped splitters) are batched too: the full Gram is built once
+and the training Grams of at most 16 splits at a time are built from their rows or as a
+downdate of the full Gram (``batched_cv_splits``).
 """
 
 from __future__ import annotations
 
+import hashlib
 import numbers
 import re
 import time
+import warnings
 from copy import deepcopy
 
 import numpy as np
@@ -27,7 +34,7 @@ from sklearn.model_selection import ParameterGrid, check_cv
 from sklearn.model_selection._search import BaseSearchCV
 from sklearn.utils.validation import check_X_y
 
-from .engine import EngineError, get_engine
+from .engine import EngineError, get_engine, split_chunks
 from .model._base import EngineRegressor, _to_original_order, solve_specs
 
 __all__ = ["GridSearchCV", "LineSearchCV"]
@@ -96,6 +103,24 @@ def _is_partition(splits, n):
     return bool(np.all(seen == 1))
 
 
+def _split_route(splits, n, world=1):
+    """How a search runs its CV splits: "partition" (one partition of the rows into 2..15 folds: the fold path
+    of batched_cv), "splits" (arbitrary row sets: batched_cv_splits) or None (sklearn's per-fit loop: sharded
+    searches, an empty test set, fewer than two training rows, a row repeated inside a split)."""
+    if 2 <= len(splits) <= 15 and _is_partition(splits, n):
+        return "partition"
+    if world > 1 or not splits:
+        return None
+    for train, test in splits:
+        tr, te = np.asarray(train), np.asarray(test)
+        if len(te) == 0 or len(tr) < 2 or tr.dtype.kind not in "iu" or te.dtype.kind not in "iu":
+            return None
+        both = np.concatenate([tr, te])
+        if both.min() < 0 or both.max() >= n or len(np.unique(both)) != len(both):
+            return None
+    return "splits"
+
+
 def _metric(scoring, sse, sae, n_rows, sst):
     """Score per column from residual sums (greater is better, sklearn convention)."""
     if scoring == "neg_root_mean_squared_error":
@@ -108,6 +133,17 @@ def _metric(scoring, sse, sae, n_rows, sst):
     if sst == 0.0:
         return np.where(sse == 0.0, 1.0, 0.0)
     return 1.0 - sse / sst
+
+
+def _split_metric(scoring, sse, sae, n_rows, sst):
+    """_metric of the arbitrary-split path, with sklearn's rule for r2 on fewer than two rows: NaN and an
+    UndefinedMetricWarning (LeaveOneOut with scoring="r2")."""
+    if scoring == "r2" and n_rows < 2:
+        from sklearn.exceptions import UndefinedMetricWarning
+
+        warnings.warn("R^2 score is not well-defined with less than two samples.", UndefinedMetricWarning)
+        return np.full(np.shape(sse), np.nan)
+    return _metric(scoring, sse, sae, n_rows, sst)
 
 
 class _WarmStarts:
@@ -160,6 +196,143 @@ def prepare_folds(engine, X, yv, test_folds, est, spec, cache=None, cache_key=No
     if ck is not None:
         cache[ck] = fd
     return fd
+
+
+def _splits_cache_key(cache, Xv, yv, sw):
+    """Data part of the SplitData cache key of a LineSearchCV: the identity of X (check_X_y returns the float64 design
+    it was given) and the content of y and of the weights (check_X_y returns a new y object at every line)."""
+    if cache is None:
+        return None
+    return (id(Xv), hashlib.sha1(np.ascontiguousarray(yv).tobytes()).hexdigest(),
+            None if sw is None else hashlib.sha1(sw.tobytes()).hexdigest())
+
+
+def prepare_split_data(engine, X, yv, splits, est, spec, cache=None, cache_key=None, sample_weight=None):
+    """Device-resident design + full Gram for arbitrary splits (Engine.prepare_splits), through the FoldData
+    cache of a LineSearchCV when there is one.  Only enqueues GPU work."""
+    ck = None
+    if cache is not None and cache_key is not None:
+        # keyed on the full content of every split, training and test rows alike: repeated / shuffled splitters
+        # can draw new splits per line, and rows in neither set make the test rows alone ambiguous
+        h = hashlib.sha1()
+        for train, test in splits:
+            for a in (train, test):
+                a = np.asarray(a, dtype=np.int64)
+                h.update(np.int64(len(a)).tobytes())
+                h.update(a.tobytes())
+        ck = ("splits", cache_key, _fold_key(est, spec), len(splits), h.hexdigest())
+        if ck in cache:
+            return cache[ck]
+    sd = engine.prepare_splits(X, yv, splits, est.fit_intercept, sample_weight, col_perm=spec.col_perm)
+    if ck is not None:
+        cache[ck] = sd
+    return sd
+
+
+def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_train_score=False, cache=None,
+                      cache_key=None, sds=None, sample_weight=None):
+    """batched_cv for arbitrary splits (list of (train, test) index arrays, see _split_route): the training Grams of
+    at most 16 splits at a time are built (Engine.split_chunk), their Lipschitz constants estimated and every
+    candidate solved on them as one batch (solve_specs), then the test lists are scored (slm_cv_score_rows).
+    Train scores: a split built from its training rows scores that list; a downdated split scores all rows
+    minus the rows outside its training set (the residual sums are additive).
+    Returns the same dict as batched_cv; its "fds" hold the refit data (SplitData.full)."""
+    torch = engine.torch
+    yv = np.asarray(y, dtype=np.float64)
+    n = yv.shape[0]
+    p = X.shape[1]
+    n_splits, n_cand = len(splits), len(specs)
+    multi = not isinstance(scoring, str)
+    metrics = dict(scoring) if multi else {"score": scoring}
+    want_train = bool(return_train_score)
+    SSE, SAE = np.zeros((n_cand, n_splits)), np.zeros((n_cand, n_splits))
+    TSSE, TSAE = (np.zeros((n_cand, n_splits)), np.zeros((n_cand, n_splits))) if want_train else (None, None)
+    fit_time = np.zeros(n_cand)
+    score_time = np.zeros(n_cand)
+    info = dict(n_iter=np.zeros((n_cand, n_splits), dtype=int), status=np.zeros((n_cand, n_splits), dtype=int),
+                gap=np.zeros((n_cand, n_splits)), n_pass=np.zeros((n_cand, n_splits), dtype=int))
+    need_r2 = "r2" in metrics.values()
+
+    def sst(rows):
+        v = yv[rows]
+        return float(((v - v.mean()) ** 2).sum()) if need_r2 and len(v) else 0.0
+
+    sst_test = np.array([sst(np.asarray(te)) for _, te in splits])
+    sst_train = np.array([sst(np.asarray(tr)) for tr, _ in splits]) if want_train else None
+    n_unconverged, iters_run, newton_stats = 0, 0, {}
+    sds = {} if sds is None else dict(sds)
+    warm = _WarmStarts()
+    batches = {}
+    for ci, s in enumerate(specs):
+        batches.setdefault(s.key, []).append(ci)
+    chunks = split_chunks(n_splits)
+    buf = None  # training Grams of one chunk, reused by every chunk and batch
+    for key, idxs in batches.items():
+        s0_, e0 = specs[idxs[0]], ests[idxs[0]]
+        fkey = _fold_key(e0, s0_)
+        if fkey not in sds:
+            sds[fkey] = prepare_split_data(engine, X, yv, splits, e0, s0_, cache, cache_key, sample_weight)
+        sd = sds[fkey]
+        if buf is None:
+            buf = torch.empty((chunks[0][1] - chunks[0][0], sd.pa, sd.pa), dtype=torch.float64, device=engine.device)
+        idxs = np.asarray(sorted(idxs, key=lambda ci: (specs[ci].strength, ci)))
+        K = len(idxs)
+        bspecs = [specs[ci] for ci in idxs]
+        for c0, c1 in chunks:
+            t0 = time.perf_counter()
+            order, fd = engine.split_chunk(sd, c0, c1, buf)
+            out = solve_specs(engine, fd, bspecs, **opts)
+            t1 = time.perf_counter()
+            if c0 == 0:
+                warm.add(out["B"], idxs, [np.arange(K)] * (c1 - c0))
+            icpt = (lambda f: out["intercept"][f]) if sd.fit_intercept else (lambda f: None)
+            rows_items, rows_where, range_items, range_where = [], [], [], []
+            for f, s in enumerate(order):
+                rows_items.append((sd.test_rows(s), out["coef"][f], K, icpt(f)))
+                rows_where.append((0, s, 1.0))
+                if want_train:
+                    rows_items.append((sd.build_rows(s), out["coef"][f], K, icpt(f)))
+                    if sd.direct[s]:
+                        rows_where.append((1, s, 1.0))
+                    else:
+                        rows_where.append((1, s, -1.0))
+                        range_items.append((0, n, out["coef"][f], K, icpt(f)))
+                        range_where.append((1, s, 1.0))
+            res = engine.cv_score_rows(sd.Xa, p, rows_items, rows_scaled=sd.weighted)
+            res_r = engine.cv_score_many(sd.Xa, p, range_items, rows_scaled=sd.weighted) if range_items else None
+            res = res.cpu().numpy()  # one D2H each
+            res_r = None if res_r is None else res_r.cpu().numpy()
+            for r, wh in ((res, rows_where), (res_r, range_where)):
+                for i, (kind, s, sign) in enumerate(wh):
+                    if kind == 0:
+                        SSE[idxs, s] += sign * r[i, 0, :K]
+                        SAE[idxs, s] += sign * r[i, 1, :K]
+                    else:
+                        TSSE[idxs, s] += sign * r[i, 0, :K]
+                        TSAE[idxs, s] += sign * r[i, 1, :K]
+            t2 = time.perf_counter()
+            for f, s in enumerate(order):
+                info["n_iter"][idxs, s] = out["n_iter"][f, :K]
+                info["status"][idxs, s] = out["status"][f, :K]
+                info["gap"][idxs, s] = out["gap"][f, :K]
+                info["n_pass"][idxs, s] = out["n_pass"][f, :K]
+            fit_time[idxs] += (t1 - t0) / (K * n_splits)
+            score_time[idxs] += (t2 - t1) / (K * n_splits)
+            n_unconverged += int(out["n_unconverged"])
+            iters_run += int(out["iters_run"])
+            for k, v in (out.get("newton") or {}).items():
+                newton_stats[k] = newton_stats.get(k, 0) + v
+    test_tabs = {m: np.empty((n_cand, n_splits)) for m in metrics}
+    train_tabs = {m: np.empty((n_cand, n_splits)) for m in metrics} if want_train else None
+    for s, (tr, te) in enumerate(splits):
+        for m, scorer in metrics.items():
+            test_tabs[m][:, s] = _split_metric(scorer, SSE[:, s], SAE[:, s], len(te), sst_test[s])
+            if want_train:
+                train_tabs[m][:, s] = _split_metric(scorer, TSSE[:, s], TSAE[:, s], len(tr), sst_train[s])
+    return dict(test_scores=test_tabs if multi else test_tabs["score"],
+                train_scores=None if not want_train else (train_tabs if multi else train_tabs["score"]),
+                fit_time=fit_time, score_time=score_time, info=info, fds={k: v.full for k, v in sds.items()},
+                n_unconverged=n_unconverged, iters_run=iters_run, warm=warm, newton=newton_stats)
 
 
 def batched_cv(engine, X, y, test_folds, ests, specs, opts, scoring, return_train_score=False, cache=None,
@@ -418,14 +591,17 @@ class GridSearchCV(_SkGridSearchCV):
         if not isinstance(est, EngineRegressor) or y is None or not getattr(est, "_batchable", True):
             return None
         # fit params: only sample_weight is understood by the batched seam (strictly positive:
-        # the unweighted CV scores are recovered from the sqrt(sw)-scaled rows)
-        sw = None
+        # the unweighted CV scores are recovered from the sqrt(sw)-scaled rows); groups only reach the splitter
+        sw = groups = None
         for k, v in params.items():
             if v is None:
                 continue
-            if k != "sample_weight":
+            if k == "groups":
+                groups = v
+            elif k == "sample_weight":
+                sw = v
+            else:
                 return None
-            sw = v
         if _device_metrics(self.scoring) is None:
             return None
         if callable(self.refit) or hasattr(X, "columns"):
@@ -450,8 +626,13 @@ class GridSearchCV(_SkGridSearchCV):
             if sw.shape[0] != n or not np.all(np.isfinite(sw)) or not np.all(sw > 0):
                 return None
         cv = check_cv(self.cv, yv, classifier=False)
-        splits = list(cv.split(Xv, yv, None))
-        if len(splits) < 2 or len(splits) > 15 or not _is_partition(splits, n):
+        try:
+            splits = list(cv.split(Xv, yv, groups))
+        except Exception:
+            return None  # sklearn's loop raises the splitter's own error
+        shard = getattr(self, "_shard", None)
+        route = _split_route(splits, n, 1 if shard is None else shard.world)
+        if route is None:
             return None
         candidates = list(ParameterGrid(self.param_grid))
         valid = set(est.get_params(deep=False))
@@ -486,7 +667,12 @@ class GridSearchCV(_SkGridSearchCV):
                     opts0 = est._engine_options()
                     engine = get_engine(opts0.pop("device", None))
                     cache = getattr(self, "_fd_cache", None)
-                    shard = getattr(self, "_shard", None)
+                    cache_key = None if cache is None else (id(Xv), id(yv), None if sw is None else sw.tobytes())
+                    if route == "splits":
+                        cache_key = _splits_cache_key(cache, Xv, yv, sw)
+                        pre_fds[_fold_key(ests[0], specs[0])] = prepare_split_data(
+                            engine, Xv, yv, splits, ests[0], specs[0], cache, cache_key, sw)
+                        continue
                     score_folds = None
                     if shard is not None and shard.world > 1 and cache is None:
                         # host rows this rank needs: its slice of every fold (Gram build and scoring
@@ -494,14 +680,13 @@ class GridSearchCV(_SkGridSearchCV):
                         score_folds = set()
                     pre_fds[_fold_key(ests[0], specs[0])] = prepare_folds(
                         engine, Xv, yv, [np.asarray(test) for _, test in splits], ests[0], specs[0], cache,
-                        None if cache is None else (id(Xv), id(yv), None if sw is None else sw.tobytes()),
-                        shard, sw, score_folds)
+                        cache_key, shard, sw, score_folds)
         except (NotImplementedError, EngineError):
             raise
         except Exception:
             return None  # sklearn's loop applies error_score semantics per candidate
         return dict(X=Xv, y=yv, n=n, p=p, splits=splits, candidates=candidates, ests=ests, specs=specs,
-                    fds=pre_fds, sample_weight=sw)
+                    fds=pre_fds, sample_weight=sw, route=route)
 
     def _fit_batched(self, plan):
         Xv, yv, n, p = plan["X"], plan["y"], plan["n"], plan["p"]
@@ -515,10 +700,18 @@ class GridSearchCV(_SkGridSearchCV):
         test_folds = [np.asarray(test) for _, test in splits]
         cache = getattr(self, "_fd_cache", None)
         sw = plan.get("sample_weight")
-        cache_key = None if cache is None else (id(plan["X"]), id(plan["y"]), None if sw is None else sw.tobytes())
-        res = batched_cv(engine, Xv, yv, test_folds, ests, specs, opts, scoring,
-                         return_train_score=self.return_train_score, cache=cache, cache_key=cache_key,
-                         shard=getattr(self, "_shard", None), fds=plan.get("fds"), sample_weight=sw)
+        if plan["route"] == "splits":
+            cache_key = _splits_cache_key(cache, plan["X"], plan["y"], sw)
+        else:
+            cache_key = None if cache is None else (id(plan["X"]), id(plan["y"]), None if sw is None else sw.tobytes())
+        if plan["route"] == "splits":
+            res = batched_cv_splits(engine, Xv, yv, splits, ests, specs, opts, scoring,
+                                    return_train_score=self.return_train_score, cache=cache, cache_key=cache_key,
+                                    sds=plan.get("fds"), sample_weight=sw)
+        else:
+            res = batched_cv(engine, Xv, yv, test_folds, ests, specs, opts, scoring,
+                             return_train_score=self.return_train_score, cache=cache, cache_key=cache_key,
+                             shard=getattr(self, "_shard", None), fds=plan.get("fds"), sample_weight=sw)
         test_scores, train_scores = res["test_scores"], res["train_scores"]
         fit_time, score_time, info, fds = res["fit_time"], res["score_time"], res["info"], res["fds"]
         if res["n_unconverged"]:
