@@ -265,6 +265,30 @@ int slm_cv_score_rows(slm_ctx* ctx, const double* Xa_dev, int64_t lda, int64_t p
                       const int64_t* ldb, const int32_t* K, const double* const* intercept_dev, int32_t rows_scaled,
                       double* const* yhat_dev, const int64_t* ldy, double* const* out_dev, void* stream);
 
+/* Residual statistics beyond the two sums, for the CV scorers that need them (neg_max_error,
+ * neg_mean_absolute_percentage_error, neg_median_absolute_error).  rows_dev == NULL: problem i is the row range
+ * [r0[i], r1[i]) as in slm_cv_score_many; else the row list rows_dev[i] of n_rows[i] rows as in slm_cv_score_rows
+ * (r0 / r1 may then be NULL, and n_rows may be NULL with ranges).  out[i] is [5][ldy[i]]:
+ *   row 0: sum r^2, row 1: sum |r| (bitwise what slm_cv_score_many / slm_cv_score_rows return),
+ *   row 2: max |r|                        (SLM_STAT_MAX),
+ *   row 3: sum |r| / max(|y|, DBL_EPSILON) (SLM_STAT_MAPE; y recovered like r when rows_scaled),
+ *   row 4: median |r|                     (SLM_STAT_MEDIAN; the mean of the two middle values when the count is
+ *                                          even, as numpy.median).
+ * r is the residual of the sums (divided by the row's sqrt(sw) column when rows_scaled).  Rows 2-4 are written
+ * only when their bit of `stats` is set; stats == 0 is slm_cv_score_many / slm_cv_score_rows.  With stats != 0,
+ * rows [0, m) of yhat[i] hold the residuals that were reduced when the call's work completes.  max and median are
+ * exact (the median is a radix select on the bit patterns, no arithmetic but the final (a + b) / 2; a NaN residual
+ * makes both NaN); the percentage sum uses the fixed two-stage order of the sums: every result is bit-reproducible.
+ * yhat[i] is scratch [m + 256][ldy[i]] as in slm_cv_score_many. */
+#define SLM_STAT_MAX (1 << 2)
+#define SLM_STAT_MAPE (1 << 3)
+#define SLM_STAT_MEDIAN (1 << 4)
+int slm_cv_score_stats(slm_ctx* ctx, const double* Xa_dev, int64_t lda, int64_t p, int32_t n,
+                       const int64_t* r0, const int64_t* r1, const int32_t* const* rows_dev, const int64_t* n_rows,
+                       const double* const* B_dev, const int64_t* ldb, const int32_t* K,
+                       const double* const* intercept_dev, int32_t rows_scaled, int32_t stats,
+                       double* const* yhat_dev, const int64_t* ldy, double* const* out_dev, void* stream);
+
 /* intercept[k] = ybar - mu^T B[:,k] from the (uncentred) training Gram's ones row
  * (LinearModel._set_intercept, _base.py:202). */
 int slm_intercepts(slm_ctx* ctx, const double* G_dev, int64_t pa, int64_t p,

@@ -13,6 +13,7 @@ import os
 from . import _build
 
 SLM_MAX_FOLDS = 16
+SLM_STAT_MAX, SLM_STAT_MAPE, SLM_STAT_MEDIAN = 1 << 2, 1 << 3, 1 << 4
 
 c_i32, c_i64, c_dbl, c_vp, c_sz = (
     ctypes.c_int32, ctypes.c_int64, ctypes.c_double, ctypes.c_void_p, ctypes.c_size_t,
@@ -97,6 +98,8 @@ SYMBOLS = {
     "slm_cv_score": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp]),
     "slm_cv_score_many": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp]),
     "slm_cv_score_rows": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp]),
+    "slm_cv_score_stats": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32,
+                                          c_i32, c_vp, c_vp, c_vp, c_vp]),
     "slm_intercepts": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp]),
     "slm_gram_apply": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, ctypes.c_int, ctypes.POINTER(c_i32), c_vp, c_i64, c_vp, c_vp]),
     "slm_newton_workspace": (c_sz, [c_i64, c_i32, c_i32, ctypes.c_int]),

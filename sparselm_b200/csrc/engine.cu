@@ -11,7 +11,9 @@
 //   K8  reweighting     adaptive_kernel
 //   K9  fold back       fold_back_kernel
 //   K10 scoring         gemm_f64_kernel<A_MMAJOR> + score_kernel
+//   K10b statistics     stat_residual/final/median_kernel (max, percentage sum, median of |r|)
 #include <cuda_runtime.h>
+#include <float.h>
 #include <math.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -901,6 +903,164 @@ __global__ void score_final_kernel(const double* __restrict__ part, long long ld
     }
     out[k] = sse;
     out[ldz + k] = sae;
+}
+
+// K10b (slm_cv_score_stats): residual statistics beyond the two sums, for the problem table of one scoring batch.
+// They run after score_final_kernel, so the partial-sum rows of every scratch are free again.
+struct StatProblem {
+    double* yhat;         // [m][ldy]: predictions in, residuals out; [2 * SCORE_RB][ldy] partials from row m
+    const int* ridx;      // row list, or NULL: rows r0 + i
+    const double* icpt;   // [K] or NULL
+    double* out;          // [5][ldy]
+    long long r0, m, ldy;
+    int K;
+};
+struct StatTable {
+    StatProblem pr[kMaxGemmProblems];
+};
+
+// grid (ceil(K_max / 8), SCORE_RB, problems): the residual of score_partial_kernel replaces the prediction, and the
+// block writes its partial max |r| (as bits: for non-negative doubles the bit pattern orders like the value, and a
+// NaN sorts above +inf) and its partial sum of |r| / max(|y|, eps), same row split and tree as the residual sums
+__global__ void __launch_bounds__(256) stat_residual_kernel(const double* __restrict__ Xa, long long lda, int p,
+                                                            int rows_scaled, const __grid_constant__ StatTable t) {
+    const StatProblem& q = t.pr[blockIdx.z];
+    if ((int)blockIdx.x * 8 >= q.K) return;
+    const int c = threadIdx.x & 7, r = threadIdx.x >> 3;
+    const int k = blockIdx.x * 8 + c;
+    __shared__ unsigned long long rmax[32][8];
+    __shared__ double rpct[32][8];
+    unsigned long long amax = 0;
+    double pct = 0.0;
+    if (k < q.K) {
+        const double b0 = q.icpt ? q.icpt[k] : 0.0;
+        for (long long i = (long long)blockIdx.y * 32 + r; i < q.m; i += (long long)SCORE_RB * 32) {
+            const double* row = Xa + (q.ridx ? (long long)q.ridx[i] : q.r0 + i) * lda;
+            double* yh = q.yhat + i * q.ldy + k;
+            double d = row[p] - *yh - b0 * row[p + 1];
+            double yv = row[p];
+            if (rows_scaled) {
+                d /= row[p + 1];
+                yv /= row[p + 1];
+            }
+            *yh = d;
+            const double a = fabs(d);
+            amax = max(amax, (unsigned long long)__double_as_longlong(a));
+            pct += a / fmax(fabs(yv), DBL_EPSILON);
+        }
+    }
+    rmax[r][c] = amax;
+    rpct[r][c] = pct;
+    __syncthreads();
+    for (int s = 16; s > 0; s >>= 1) {
+        if (r < s) {
+            rmax[r][c] = max(rmax[r][c], rmax[r + s][c]);
+            rpct[r][c] += rpct[r + s][c];
+        }
+        __syncthreads();
+    }
+    if (r == 0 && k < q.K) {
+        unsigned long long* part = reinterpret_cast<unsigned long long*>(q.yhat + q.m * q.ldy);
+        part[((long long)blockIdx.y * 2 + 0) * q.ldy + k] = rmax[0][c];
+        reinterpret_cast<double*>(part)[((long long)blockIdx.y * 2 + 1) * q.ldy + k] = rpct[0][c];
+    }
+}
+// grid (ceil(K_max / 128), problems): out rows 2 (max |r|) and 3 (percentage sum), fixed order over the row blocks
+__global__ void stat_final_kernel(int stats, const __grid_constant__ StatTable t) {
+    const StatProblem& q = t.pr[blockIdx.y];
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= q.K) return;
+    const double* part = q.yhat + q.m * q.ldy;
+    unsigned long long amax = 0;
+    double pct = 0.0;
+    for (int b = 0; b < SCORE_RB; ++b) {
+        amax = max(amax, reinterpret_cast<const unsigned long long*>(part)[(long long)b * 2 * q.ldy + k]);
+        pct += part[((long long)b * 2 + 1) * q.ldy + k];
+    }
+    if (stats & SLM_STAT_MAX) q.out[2 * q.ldy + k] = __longlong_as_double((long long)amax);
+    if (stats & SLM_STAT_MAPE) q.out[3 * q.ldy + k] = pct;
+}
+
+// grid (ceil(K_max / 8), problems): exact median of |r| per column by a most-significant-digit-first radix select on
+// the bit patterns (8 passes of 8-bit digits), the two middle order statistics at once.  A block owns 8 adjacent
+// columns (64-byte row segments); thread (c, r) reads column c of rows r, r + 32, ...; warp w finds column w's digits.
+constexpr int MED_UNROLL = 4;
+__global__ void __launch_bounds__(256) stat_median_kernel(const __grid_constant__ StatTable t) {
+    const StatProblem& q = t.pr[blockIdx.y];
+    if ((int)blockIdx.x * 8 >= q.K) return;
+    const int c = threadIdx.x & 7, r = threadIdx.x >> 3, lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int k = blockIdx.x * 8 + c;
+    const bool col = k < q.K;
+    __shared__ unsigned int hist[2][8][256];
+    __shared__ unsigned long long pfx[2][8];  // digits of the two order statistics found so far
+    __shared__ long long rnk[2][8];           // their ranks among the values that share that prefix
+    __shared__ int has_nan[8];
+    for (int j = threadIdx.x; j < 2 * 8 * 256; j += 256) (&hist[0][0][0])[j] = 0u;
+    if (threadIdx.x < 16) {
+        const int tt = threadIdx.x >> 3, cc = threadIdx.x & 7;
+        pfx[tt][cc] = 0ull;
+        rnk[tt][cc] = tt == 0 ? (q.m - 1) / 2 : q.m / 2;  // np.median: ranks (m-1)/2 and m/2
+    }
+    if (threadIdx.x < 8) has_nan[threadIdx.x] = 0;
+    __syncthreads();
+    for (int shift = 56; shift >= 0; shift -= 8) {
+        const unsigned long long hmask = shift == 56 ? 0ull : ~0ull << (shift + 8);
+        const unsigned long long p0 = pfx[0][c], p1 = pfx[1][c];
+        // the trip count is uniform over a warp (its 4 row lanes share i0): every lane takes part in the matches
+        for (long long i0 = 0; i0 < q.m; i0 += 32 * MED_UNROLL) {
+            unsigned long long v[MED_UNROLL];
+            bool ok[MED_UNROLL];
+#pragma unroll
+            for (int u = 0; u < MED_UNROLL; ++u) {
+                const long long i = i0 + r + 32 * u;
+                ok[u] = col && i < q.m;
+                v[u] = ok[u] ? (unsigned long long)__double_as_longlong(fabs(q.yhat[i * q.ldy + k])) : 0ull;
+            }
+#pragma unroll
+            for (int u = 0; u < MED_UNROLL; ++u) {
+                const unsigned dig = (unsigned)(v[u] >> shift) & 255u;
+#pragma unroll
+                for (int tt = 0; tt < 2; ++tt) {
+                    const bool in = ok[u] && (v[u] & hmask) == (tt ? p1 : p0);
+                    // lanes adding to the same bin add once (ties and all-equal columns would serialise otherwise)
+                    const unsigned key = in ? ((unsigned)c << 8 | dig) : 0xffffffffu;
+                    const unsigned peers = __match_any_sync(0xffffffffu, key);
+                    if (in && lane == __ffs(peers) - 1) atomicAdd(&hist[tt][c][dig], (unsigned)__popc(peers));
+                }
+                if (shift == 56 && ok[u] && v[u] > 0x7ff0000000000000ull) has_nan[c] = 1;
+            }
+        }
+        __syncthreads();
+        if (blockIdx.x * 8 + w < q.K) {
+            for (int tt = 0; tt < 2; ++tt) {
+                const unsigned int* h = hist[tt][w];
+                unsigned long long s = 0;
+                for (int j = 0; j < 8; ++j) s += h[lane * 8 + j];
+                unsigned long long incl = s;
+                for (int o = 1; o < 32; o <<= 1) {
+                    const unsigned long long x = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= o) incl += x;
+                }
+                const unsigned long long excl = incl - s;
+                const long long R = rnk[tt][w];
+                __syncwarp();
+                if ((unsigned long long)R >= excl && (unsigned long long)R < incl) {
+                    unsigned long long cum = excl;
+                    int b = lane * 8;
+                    while (b < lane * 8 + 7 && cum + h[b] <= (unsigned long long)R) cum += h[b++];
+                    pfx[tt][w] |= (unsigned long long)b << shift;
+                    rnk[tt][w] = R - (long long)cum;
+                }
+            }
+        }
+        __syncthreads();
+        for (int j = threadIdx.x; j < 2 * 8 * 256; j += 256) (&hist[0][0][0])[j] = 0u;
+        __syncthreads();
+    }
+    if (col && r == 0) {
+        const double a = __longlong_as_double((long long)pfx[0][c]), b = __longlong_as_double((long long)pfx[1][c]);
+        q.out[4 * q.ldy + k] = has_nan[c] ? __longlong_as_double(0x7ff8000000000000ll) : ((q.m & 1) ? a : (a + b) / 2);
+    }
 }
 
 __global__ void __launch_bounds__(256) intercept_kernel(const double* __restrict__ G, long long pa, int p,
@@ -2233,14 +2393,22 @@ int slm_cv_score(slm_ctx* ctx, const double* Xa, int64_t lda, int64_t p, int64_t
 }
 
 // several scoring problems in one GEMM launch (the row-sharded scoring of a sharded grid holds a dozen small
-// ones: a slice of every fold's rows x the columns every rank solved on that fold)
-int slm_cv_score_many(slm_ctx* ctx, const double* Xa, int64_t lda, int64_t p, int32_t n, const int64_t* r0,
-                      const int64_t* r1, const double* const* B, const int64_t* ldb, const int32_t* K,
-                      const double* const* icpt, int32_t rows_scaled, double* const* yhat, const int64_t* ldy,
-                      double* const* out, void* stream) {
-    if (!ctx || !Xa || !r0 || !r1 || !B || !ldb || !K || !yhat || !ldy || !out)
-        return fail(ctx, 1, "slm_cv_score_many: null argument");
+// ones: a slice of every fold's rows x the columns every rank solved on that fold).  rows == NULL: problem i is the
+// row range [r0[i], r1[i]); else the device row list rows[i] of n_rows[i] rows (gathered A rows in the GEMM and in
+// the residual sums).  slm_cv_score_many and slm_cv_score_rows are the stats == 0 cases of slm_cv_score_stats: the
+// statistics kernels run only when stats asks for them.
+static int cv_score_impl(slm_ctx* ctx, const char* fn, const double* Xa, int64_t lda, int64_t p, int32_t n,
+                         const int64_t* r0, const int64_t* r1, const int32_t* const* rows, const int64_t* n_rows,
+                         const double* const* B, const int64_t* ldb, const int32_t* K, const double* const* icpt,
+                         int32_t rows_scaled, int32_t stats, double* const* yhat, const int64_t* ldy,
+                         double* const* out, void* stream) {
+    if (!ctx || !Xa || (rows ? !n_rows : (!r0 || !r1)) || !B || !ldb || !K || !yhat || !ldy || !out)
+        return fail(ctx, 1, std::string(fn) + ": null argument");
+    if (stats & ~(3 | SLM_STAT_MAX | SLM_STAT_MAPE | SLM_STAT_MEDIAN))
+        return fail(ctx, 1, std::string(fn) + ": unknown statistic in the stats mask");
+    stats &= SLM_STAT_MAX | SLM_STAT_MAPE | SLM_STAT_MEDIAN;  // the two sums are always computed
     cudaStream_t s = (cudaStream_t)stream;
+    auto rows_of = [&](int i) -> int64_t { return rows ? n_rows[i] : r1[i] - r0[i]; };
     for (int i0 = 0; i0 < n; i0 += kMaxGemmProblems) {
         const int nb = std::min<int>(n - i0, kMaxGemmProblems);
         GemmBatch b;
@@ -2249,12 +2417,15 @@ int slm_cv_score_many(slm_ctx* ctx, const double* Xa, int64_t lda, int64_t p, in
         int np = 0;
         double flops = 0.0;
         for (int i = i0; i < i0 + nb; ++i) {
-            const int64_t m = r1[i] - r0[i];
+            const int64_t m = rows_of(i);
             if (m <= 0 || K[i] <= 0) continue;
-            if (!B[i] || !yhat[i] || !out[i] || (ldb[i] & 1) || (ldy[i] % 8) || ((uintptr_t)B[i] & 15))
-                return fail(ctx, 1, "slm_cv_score_many: bad problem (null pointer, odd leading dimension or unaligned B)");
+            if (rows && m > (1LL << 30)) return fail(ctx, 1, std::string(fn) + ": row list too long");
+            if ((rows && !rows[i]) || !B[i] || !yhat[i] || !out[i] || (ldb[i] & 1) || (ldy[i] % 8) ||
+                ((uintptr_t)B[i] & 15))
+                return fail(ctx, 1, std::string(fn) + ": bad problem (null pointer, odd leading dimension or unaligned B)");
             GemmProblem& pr = b.pr[np];
-            pr.P = Xa + r0[i] * lda;
+            pr.P = rows ? Xa : Xa + r0[i] * lda;
+            if (rows) pr.kidx = rows[i];
             pr.Q = B[i];
             pr.C = yhat[i];
             pr.ldp = lda;
@@ -2273,22 +2444,48 @@ int slm_cv_score_many(slm_ctx* ctx, const double* Xa, int64_t lda, int64_t p, in
         const int sid = pick_shape(kScoreShapes, kNumScoreShapes, pd, np, ctx->sm_count);
         {
             FamTimer tm(ctx, FAM_SCORE, s, flops);
-            cudaError_t e = launch_score_shape(ctx, sid, b, s);
+            cudaError_t e = rows ? launch_score_rows_shape(ctx, sid, b, s) : launch_score_shape(ctx, sid, b, s);
             if (e != cudaSuccess) return fail(ctx, 100 + (int)e, std::string("score gemm: ") + cudaGetErrorString(e));
             ctx->launches++;
         }
+        StatTable st;
+        int nst = 0, kmax = 0;
         for (int i = i0; i < i0 + nb; ++i) {
-            const int64_t m = r1[i] - r0[i];
+            const int64_t m = rows_of(i);
             if (m <= 0 || K[i] <= 0) continue;
             double* part = yhat[i] + m * ldy[i];
             dim3 grid((unsigned)((K[i] + 7) / 8), SCORE_RB);
-            score_partial_kernel<<<grid, 256, 0, s>>>(Xa, lda, (int)p, r0[i], m, yhat[i], ldy[i], K[i], icpt ? icpt[i] : nullptr,
-                                                      rows_scaled, part);
+            if (rows)
+                score_partial_kernel<true><<<grid, 256, 0, s>>>(Xa, lda, (int)p, 0, m, yhat[i], ldy[i], K[i],
+                                                                icpt ? icpt[i] : nullptr, rows_scaled, part, rows[i]);
+            else
+                score_partial_kernel<<<grid, 256, 0, s>>>(Xa, lda, (int)p, r0[i], m, yhat[i], ldy[i], K[i],
+                                                          icpt ? icpt[i] : nullptr, rows_scaled, part);
             score_final_kernel<<<(unsigned)((K[i] + 127) / 128), 128, 0, s>>>(part, ldy[i], K[i], out[i]);
+            st.pr[nst++] = {yhat[i], rows ? rows[i] : nullptr, icpt ? icpt[i] : nullptr, out[i], rows ? 0 : r0[i], m,
+                            ldy[i], K[i]};
+            kmax = std::max<int>(kmax, K[i]);
         }
         LAUNCH_OK("score kernels");
+        if (stats == 0) continue;
+        // one launch of each statistics kernel for the whole table
+        stat_residual_kernel<<<dim3((unsigned)((kmax + 7) / 8), SCORE_RB, (unsigned)nst), 256, 0, s>>>(
+            Xa, lda, (int)p, rows_scaled, st);
+        if (stats & (SLM_STAT_MAX | SLM_STAT_MAPE))
+            stat_final_kernel<<<dim3((unsigned)((kmax + 127) / 128), (unsigned)nst), 128, 0, s>>>(stats, st);
+        if (stats & SLM_STAT_MEDIAN)
+            stat_median_kernel<<<dim3((unsigned)((kmax + 7) / 8), (unsigned)nst), 256, 0, s>>>(st);
+        LAUNCH_OK("score statistics kernels");
     }
     return 0;
+}
+
+int slm_cv_score_many(slm_ctx* ctx, const double* Xa, int64_t lda, int64_t p, int32_t n, const int64_t* r0,
+                      const int64_t* r1, const double* const* B, const int64_t* ldb, const int32_t* K,
+                      const double* const* icpt, int32_t rows_scaled, double* const* yhat, const int64_t* ldy,
+                      double* const* out, void* stream) {
+    return cv_score_impl(ctx, "slm_cv_score_many", Xa, lda, p, n, r0, r1, nullptr, nullptr, B, ldb, K, icpt,
+                         rows_scaled, 0, yhat, ldy, out, stream);
 }
 
 // the same with a device row list per problem instead of a row range (arbitrary CV splits)
@@ -2296,59 +2493,17 @@ int slm_cv_score_rows(slm_ctx* ctx, const double* Xa, int64_t lda, int64_t p, in
                       const int64_t* n_rows, const double* const* B, const int64_t* ldb, const int32_t* K,
                       const double* const* icpt, int32_t rows_scaled, double* const* yhat, const int64_t* ldy,
                       double* const* out, void* stream) {
-    if (!ctx || !Xa || !rows || !n_rows || !B || !ldb || !K || !yhat || !ldy || !out)
-        return fail(ctx, 1, "slm_cv_score_rows: null argument");
-    cudaStream_t s = (cudaStream_t)stream;
-    for (int i0 = 0; i0 < n; i0 += kMaxGemmProblems) {
-        const int nb = std::min<int>(n - i0, kMaxGemmProblems);
-        GemmBatch b;
-        memset(&b, 0, sizeof(b));
-        ProblemDims pd[kMaxGemmProblems];
-        int np = 0;
-        double flops = 0.0;
-        for (int i = i0; i < i0 + nb; ++i) {
-            const int64_t m = n_rows[i];
-            if (m <= 0 || K[i] <= 0) continue;
-            if (m > (1LL << 30)) return fail(ctx, 1, "slm_cv_score_rows: row list too long");
-            if (!rows[i] || !B[i] || !yhat[i] || !out[i] || (ldb[i] & 1) || (ldy[i] % 8) || ((uintptr_t)B[i] & 15))
-                return fail(ctx, 1, "slm_cv_score_rows: bad problem (null pointer, odd leading dimension or unaligned B)");
-            GemmProblem& pr = b.pr[np];
-            pr.P = Xa;
-            pr.kidx = rows[i];
-            pr.Q = B[i];
-            pr.C = yhat[i];
-            pr.ldp = lda;
-            pr.ldq = ldb[i];
-            pr.ldc = ldy[i];
-            pr.M = (int)m;
-            pr.N = (int)std::min<int64_t>(round_up(K[i], 8), ldy[i]);
-            pr.qlim = pr.N;
-            pr.Kd = (int)p;
-            pd[np] = {pr.M, pr.N};
-            flops += 2.0 * (double)m * (double)p * (double)K[i];
-            ++np;
-        }
-        if (np == 0) continue;
-        b.n_problems = np;
-        const int sid = pick_shape(kScoreShapes, kNumScoreShapes, pd, np, ctx->sm_count);
-        {
-            FamTimer tm(ctx, FAM_SCORE, s, flops);
-            cudaError_t e = launch_score_rows_shape(ctx, sid, b, s);
-            if (e != cudaSuccess) return fail(ctx, 100 + (int)e, std::string("score gemm: ") + cudaGetErrorString(e));
-            ctx->launches++;
-        }
-        for (int i = i0; i < i0 + nb; ++i) {
-            const int64_t m = n_rows[i];
-            if (m <= 0 || K[i] <= 0) continue;
-            double* part = yhat[i] + m * ldy[i];
-            dim3 grid((unsigned)((K[i] + 7) / 8), SCORE_RB);
-            score_partial_kernel<true><<<grid, 256, 0, s>>>(Xa, lda, (int)p, 0, m, yhat[i], ldy[i], K[i],
-                                                            icpt ? icpt[i] : nullptr, rows_scaled, part, rows[i]);
-            score_final_kernel<<<(unsigned)((K[i] + 127) / 128), 128, 0, s>>>(part, ldy[i], K[i], out[i]);
-        }
-        LAUNCH_OK("score kernels");
-    }
-    return 0;
+    if (!rows) return fail(ctx, 1, "slm_cv_score_rows: null argument");
+    return cv_score_impl(ctx, "slm_cv_score_rows", Xa, lda, p, n, nullptr, nullptr, rows, n_rows, B, ldb, K, icpt,
+                         rows_scaled, 0, yhat, ldy, out, stream);
+}
+
+int slm_cv_score_stats(slm_ctx* ctx, const double* Xa, int64_t lda, int64_t p, int32_t n, const int64_t* r0,
+                       const int64_t* r1, const int32_t* const* rows, const int64_t* n_rows, const double* const* B,
+                       const int64_t* ldb, const int32_t* K, const double* const* icpt, int32_t rows_scaled,
+                       int32_t stats, double* const* yhat, const int64_t* ldy, double* const* out, void* stream) {
+    return cv_score_impl(ctx, "slm_cv_score_stats", Xa, lda, p, n, r0, r1, rows, n_rows, B, ldb, K, icpt, rows_scaled,
+                         stats, yhat, ldy, out, stream);
 }
 
 int slm_intercepts(slm_ctx* ctx, const double* G, int64_t pa, int64_t p, const double* B, int64_t ldz,

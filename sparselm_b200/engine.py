@@ -1309,55 +1309,63 @@ class Engine:
         items: list of (r0, r1, B, K, intercept) with B a device view [p, >= K] whose row stride is even and
         whose first element is 16-byte aligned (a column slice of a wider table is fine), intercept a device
         view [K] or None.  Returns a device tensor [len(items), 2, ldo] (sse, sae in the first K entries)."""
-        torch = self.torch
-        n = len(items)
-        ldo = max([max(8, _round_up(int(it[3]), 8)) for it in items], default=8)
-        ldys = [ldo] * n  # one leading dimension for every problem: slot i of the result is a plain [2, ldo] block
-        out = torch.zeros((max(n, 1), 2, ldo), dtype=torch.float64, device=self.device)
-        if n == 0:
-            return out
-        rows = [max(0, int(it[1]) - int(it[0])) for it in items]
-        offs = np.concatenate([[0], np.cumsum([(m + 256) * ld for m, ld in zip(rows, ldys)])]).astype(np.int64)
-        yhat = torch.empty(int(offs[-1]), dtype=torch.float64, device=self.device)
-        i64, i32, vp = ctypes.c_int64 * n, ctypes.c_int32 * n, ctypes.c_void_p * n
-        r0 = i64(*[int(it[0]) for it in items])
-        r1 = i64(*[int(it[1]) for it in items])
-        Bp = vp(*[it[2].data_ptr() for it in items])
-        ldb = i64(*[int(it[2].stride(0)) for it in items])
-        K = i32(*[int(it[3]) for it in items])
-        ic = vp(*[(None if it[4] is None else it[4].data_ptr()) for it in items])
-        yp = vp(*[yhat.data_ptr() + 8 * int(o) for o in offs[:-1]])
-        ldy = i64(*ldys)
-        op = vp(*[out.data_ptr() + 8 * i * 2 * ldo for i in range(n)])
-        self._ck(self.lib.slm_cv_score_many(self.h, self._ptr(Xa), Xa.shape[1], p, n, r0, r1, Bp, ldb, K, ic,
-                                            1 if rows_scaled else 0, yp, ldy, op, self.stream), "slm_cv_score_many")
-        return out
+        return self._cv_score(Xa, p, items, rows_scaled, None)[0]
 
     def cv_score_rows(self, Xa, p, items, rows_scaled=False):
         """cv_score_many over row lists: items are (rows, B, K, intercept) with rows a device int32 view of the
         rows of Xa to score.  Returns a device tensor [len(items), 2, ldo] (sse, sae in the first K entries)."""
+        return self._cv_score(Xa, p, items, rows_scaled, None)[0]
+
+    def cv_score_stats(self, Xa, p, items, rows_scaled=False, stats=0, return_residuals=False):
+        """cv_score_many (items (r0, r1, B, K, intercept)) or cv_score_rows (items (rows, B, K, intercept)) with the
+        residual statistics of the `stats` bit mask (_lib.SLM_STAT_MAX | SLM_STAT_MAPE | SLM_STAT_MEDIAN).
+        Returns a device tensor [len(items), 5, ldo]: sse, sae, max |r|, sum |r| / max(|y|, eps), median |r| in
+        the first K entries (rows whose bit is not set are zero); with return_residuals also, per item, the
+        device view [m, ldo] of the residuals that were reduced (first K columns)."""
+        out, res = self._cv_score(Xa, p, items, rows_scaled, int(stats))
+        return (out, res) if return_residuals else out
+
+    def _cv_score(self, Xa, p, items, rows_scaled, stats):
+        """One call of slm_cv_score_many / _rows (stats None) or slm_cv_score_stats: range items are 5-tuples,
+        row-list items 4-tuples.  Returns (out [len(items), 2 or 5, ldo], per-item [m, ldo] scratch views)."""
         torch = self.torch
         n = len(items)
-        ldo = max([max(8, _round_up(int(it[2]), 8)) for it in items], default=8)
-        out = torch.zeros((max(n, 1), 2, ldo), dtype=torch.float64, device=self.device)
+        ranges = n > 0 and len(items[0]) == 5
+        ldo = max([max(8, _round_up(int(it[-2]), 8)) for it in items], default=8)
+        nrow = 2 if stats is None else 5
+        # one leading dimension for every problem: slot i of the result is a plain [nrow, ldo] block
+        out = torch.zeros((max(n, 1), nrow, ldo), dtype=torch.float64, device=self.device)
         if n == 0:
-            return out
-        rows = [int(it[0].numel()) for it in items]
+            return out, []
+        rows = [max(0, int(it[1]) - int(it[0])) if ranges else int(it[0].numel()) for it in items]
         offs = np.concatenate([[0], np.cumsum([(m + 256) * ldo for m in rows])]).astype(np.int64)
         yhat = torch.empty(int(offs[-1]), dtype=torch.float64, device=self.device)
         i64, i32, vp = ctypes.c_int64 * n, ctypes.c_int32 * n, ctypes.c_void_p * n
-        rp = vp(*[it[0].data_ptr() for it in items])
-        nr = i64(*rows)
-        Bp = vp(*[it[1].data_ptr() for it in items])
-        ldb = i64(*[int(it[1].stride(0)) for it in items])
-        K = i32(*[int(it[2]) for it in items])
-        ic = vp(*[(None if it[3] is None else it[3].data_ptr()) for it in items])
+        B, K, ic = ([it[j] for it in items] for j in (-3, -2, -1))
+        Bp = vp(*[b.data_ptr() for b in B])
+        ldb = i64(*[int(b.stride(0)) for b in B])
+        Kc = i32(*[int(k) for k in K])
+        icp = vp(*[(None if c is None else c.data_ptr()) for c in ic])
         yp = vp(*[yhat.data_ptr() + 8 * int(o) for o in offs[:-1]])
         ldy = i64(*([ldo] * n))
-        op = vp(*[out.data_ptr() + 8 * i * 2 * ldo for i in range(n)])
-        self._ck(self.lib.slm_cv_score_rows(self.h, self._ptr(Xa), Xa.shape[1], p, n, rp, nr, Bp, ldb, K, ic,
-                                            1 if rows_scaled else 0, yp, ldy, op, self.stream), "slm_cv_score_rows")
-        return out
+        op = vp(*[out.data_ptr() + 8 * i * nrow * ldo for i in range(n)])
+        if ranges:
+            r0, r1 = i64(*[int(it[0]) for it in items]), i64(*[int(it[1]) for it in items])
+            rp = nr = None
+        else:
+            r0 = r1 = None
+            rp, nr = vp(*[it[0].data_ptr() for it in items]), i64(*rows)
+        sc = 1 if rows_scaled else 0
+        if stats is not None:
+            self._ck(self.lib.slm_cv_score_stats(self.h, self._ptr(Xa), Xa.shape[1], p, n, r0, r1, rp, nr, Bp, ldb,
+                                                 Kc, icp, sc, stats, yp, ldy, op, self.stream), "slm_cv_score_stats")
+        elif ranges:
+            self._ck(self.lib.slm_cv_score_many(self.h, self._ptr(Xa), Xa.shape[1], p, n, r0, r1, Bp, ldb, Kc, icp, sc,
+                                                yp, ldy, op, self.stream), "slm_cv_score_many")
+        else:
+            self._ck(self.lib.slm_cv_score_rows(self.h, self._ptr(Xa), Xa.shape[1], p, n, rp, nr, Bp, ldb, Kc, icp, sc,
+                                                yp, ldy, op, self.stream), "slm_cv_score_rows")
+        return out, [yhat[int(o):int(o) + m * ldo].view(m, ldo) for o, m in zip(offs[:-1], rows)]
 
 
 _engines: dict = {}

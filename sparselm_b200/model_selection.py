@@ -39,8 +39,23 @@ from .model._base import EngineRegressor, _to_original_order, solve_specs
 
 __all__ = ["GridSearchCV", "LineSearchCV"]
 
+# scorers that need a residual statistic beyond the two sums: the row of slm_cv_score_stats' output that holds it
+_STAT_ROWS = {"neg_max_error": 2, "neg_mean_absolute_percentage_error": 3, "neg_median_absolute_error": 4}
 _DEVICE_SCORERS = {None, "r2", "neg_root_mean_squared_error", "neg_mean_squared_error",
-                   "neg_mean_absolute_error"}
+                   "neg_mean_absolute_error", "d2_absolute_error_score"} | set(_STAT_ROWS)
+# scorers a sharded search leaves to sklearn's loop: a median of row-sharded residuals needs a residual exchange
+_UNSHARDED_SCORERS = set(_STAT_ROWS) | {"d2_absolute_error_score"}
+
+
+def _stat_mask(metrics):
+    """slm_cv_score_stats bit mask of the statistics the metrics {name: scorer} need (0: the two sums suffice)."""
+    return sum(1 << r for v, r in _STAT_ROWS.items() if v in set(metrics.values()))
+
+
+def _abs_dev_median(v):
+    """sum |v - median(v)|: the denominator of d2_absolute_error_score (np.median equals sklearn's
+    _weighted_percentile(v, 1, 50, average=True))."""
+    return float(np.abs(v - np.median(v)).sum()) if len(v) else 0.0
 
 
 def _device_metrics(scoring):
@@ -121,8 +136,27 @@ def _split_route(splits, n, world=1):
     return "splits"
 
 
-def _metric(scoring, sse, sae, n_rows, sst):
-    """Score per column from residual sums (greater is better, sklearn convention)."""
+def _metric(scoring, sse, sae, n_rows, sst, stats=None):
+    """Score per column from residual sums (greater is better, sklearn convention).  stats: what the other
+    scorers need, {"max", "mape", "median"}: per-column max |r|, sum |r| / max(|y|, eps) and median |r|;
+    "sad": sum |y - median(y)| over the scored rows."""
+    if scoring == "neg_median_absolute_error":
+        return -stats["median"]
+    if scoring == "neg_max_error":
+        return -stats["max"]
+    if scoring == "neg_mean_absolute_percentage_error":
+        return -stats["mape"] / n_rows
+    if scoring == "d2_absolute_error_score":
+        # sklearn's d2_pinball_score(alpha=0.5): NaN on fewer than two rows, force-finite otherwise
+        if n_rows < 2:
+            from sklearn.exceptions import UndefinedMetricWarning
+
+            warnings.warn("D^2 score is not well-defined with less than two samples.", UndefinedMetricWarning)
+            return np.full(np.shape(sae), np.nan)
+        sae = np.asarray(sae, dtype=np.float64)
+        if stats["sad"] == 0.0:
+            return np.where(sae == 0.0, 1.0, 0.0)
+        return np.where(sae == 0.0, 1.0, 1.0 - sae / stats["sad"])
     if scoring == "neg_root_mean_squared_error":
         return -np.sqrt(sse / n_rows)
     if scoring == "neg_mean_squared_error":
@@ -135,7 +169,7 @@ def _metric(scoring, sse, sae, n_rows, sst):
     return 1.0 - sse / sst
 
 
-def _split_metric(scoring, sse, sae, n_rows, sst):
+def _split_metric(scoring, sse, sae, n_rows, sst, stats=None):
     """_metric of the arbitrary-split path, with sklearn's rule for r2 on fewer than two rows: NaN and an
     UndefinedMetricWarning (LeaveOneOut with scoring="r2")."""
     if scoring == "r2" and n_rows < 2:
@@ -143,7 +177,7 @@ def _split_metric(scoring, sse, sae, n_rows, sst):
 
         warnings.warn("R^2 score is not well-defined with less than two samples.", UndefinedMetricWarning)
         return np.full(np.shape(sse), np.nan)
-    return _metric(scoring, sse, sae, n_rows, sst)
+    return _metric(scoring, sse, sae, n_rows, sst, stats)
 
 
 class _WarmStarts:
@@ -229,13 +263,23 @@ def prepare_split_data(engine, X, yv, splits, est, spec, cache=None, cache_key=N
     return sd
 
 
+def _stats_of(ext, s, sad):
+    """The stats argument of _metric for split s: columns of the [3][n_cand][n_splits] statistics table (or None)."""
+    d = {"sad": sad}
+    if ext is not None:
+        d.update(max=ext[0][:, s], mape=ext[1][:, s], median=ext[2][:, s])
+    return d
+
+
 def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_train_score=False, cache=None,
                       cache_key=None, sds=None, sample_weight=None):
     """batched_cv for arbitrary splits (list of (train, test) index arrays, see _split_route): the training Grams of
     at most 16 splits at a time are built (Engine.split_chunk), their Lipschitz constants estimated and every
-    candidate solved on them as one batch (solve_specs), then the test lists are scored (slm_cv_score_rows).
+    candidate solved on them as one batch (solve_specs), then the test lists are scored (slm_cv_score_rows, or
+    slm_cv_score_stats when a scorer needs a residual statistic).
     Train scores: a split built from its training rows scores that list; a downdated split scores all rows
-    minus the rows outside its training set (the residual sums are additive).
+    minus the rows outside its training set (the residual sums are additive), or, when a statistic is needed (a
+    median does not downdate), the explicit list of its training rows, made for the chunk and dropped after it.
     Returns the same dict as batched_cv; its "fds" hold the refit data (SplitData.full)."""
     torch = engine.torch
     yv = np.asarray(y, dtype=np.float64)
@@ -252,6 +296,11 @@ def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_t
     info = dict(n_iter=np.zeros((n_cand, n_splits), dtype=int), status=np.zeros((n_cand, n_splits), dtype=int),
                 gap=np.zeros((n_cand, n_splits)), n_pass=np.zeros((n_cand, n_splits), dtype=int))
     need_r2 = "r2" in metrics.values()
+    need_d2 = "d2_absolute_error_score" in metrics.values()
+    stat_mask = _stat_mask(metrics)
+    # max |r|, percentage sum, median |r| per (candidate, split): rows 2-4 of slm_cv_score_stats
+    EXT = np.zeros((3, n_cand, n_splits)) if stat_mask else None
+    TEXT = np.zeros((3, n_cand, n_splits)) if stat_mask and want_train else None
 
     def sst(rows):
         v = yv[rows]
@@ -259,6 +308,8 @@ def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_t
 
     sst_test = np.array([sst(np.asarray(te)) for _, te in splits])
     sst_train = np.array([sst(np.asarray(tr)) for tr, _ in splits]) if want_train else None
+    sad_test = [_abs_dev_median(yv[np.asarray(te)]) if need_d2 else 0.0 for _, te in splits]
+    sad_train = [_abs_dev_median(yv[np.asarray(tr)]) if need_d2 else 0.0 for tr, _ in splits] if want_train else None
     n_unconverged, iters_run, newton_stats = 0, 0, {}
     sds = {} if sds is None else dict(sds)
     warm = _WarmStarts()
@@ -290,7 +341,12 @@ def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_t
             for f, s in enumerate(order):
                 rows_items.append((sd.test_rows(s), out["coef"][f], K, icpt(f)))
                 rows_where.append((0, s, 1.0))
-                if want_train:
+                if want_train and stat_mask:
+                    tr = sd.build_rows(s) if sd.direct[s] else engine.to_device(
+                        np.sort(np.asarray(splits[s][0])).astype(np.int32))
+                    rows_items.append((tr, out["coef"][f], K, icpt(f)))
+                    rows_where.append((1, s, 1.0))
+                elif want_train:
                     rows_items.append((sd.build_rows(s), out["coef"][f], K, icpt(f)))
                     if sd.direct[s]:
                         rows_where.append((1, s, 1.0))
@@ -298,7 +354,10 @@ def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_t
                         rows_where.append((1, s, -1.0))
                         range_items.append((0, n, out["coef"][f], K, icpt(f)))
                         range_where.append((1, s, 1.0))
-            res = engine.cv_score_rows(sd.Xa, p, rows_items, rows_scaled=sd.weighted)
+            if stat_mask:
+                res = engine.cv_score_stats(sd.Xa, p, rows_items, rows_scaled=sd.weighted, stats=stat_mask)
+            else:
+                res = engine.cv_score_rows(sd.Xa, p, rows_items, rows_scaled=sd.weighted)
             res_r = engine.cv_score_many(sd.Xa, p, range_items, rows_scaled=sd.weighted) if range_items else None
             res = res.cpu().numpy()  # one D2H each
             res_r = None if res_r is None else res_r.cpu().numpy()
@@ -310,6 +369,8 @@ def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_t
                     else:
                         TSSE[idxs, s] += sign * r[i, 0, :K]
                         TSAE[idxs, s] += sign * r[i, 1, :K]
+                    if stat_mask:  # one item per split and kind: the statistics are not summed
+                        (EXT if kind == 0 else TEXT)[:, idxs, s] = r[i, 2:5, :K]
             t2 = time.perf_counter()
             for f, s in enumerate(order):
                 info["n_iter"][idxs, s] = out["n_iter"][f, :K]
@@ -326,9 +387,11 @@ def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_t
     train_tabs = {m: np.empty((n_cand, n_splits)) for m in metrics} if want_train else None
     for s, (tr, te) in enumerate(splits):
         for m, scorer in metrics.items():
-            test_tabs[m][:, s] = _split_metric(scorer, SSE[:, s], SAE[:, s], len(te), sst_test[s])
+            test_tabs[m][:, s] = _split_metric(scorer, SSE[:, s], SAE[:, s], len(te), sst_test[s],
+                                               _stats_of(EXT, s, sad_test[s]))
             if want_train:
-                train_tabs[m][:, s] = _split_metric(scorer, TSSE[:, s], TSAE[:, s], len(tr), sst_train[s])
+                train_tabs[m][:, s] = _split_metric(scorer, TSSE[:, s], TSAE[:, s], len(tr), sst_train[s],
+                                                    _stats_of(TEXT, s, sad_train[s]))
     return dict(test_scores=test_tabs if multi else test_tabs["score"],
                 train_scores=None if not want_train else (train_tabs if multi else train_tabs["score"]),
                 fit_time=fit_time, score_time=score_time, info=info, fds={k: v.full for k, v in sds.items()},
@@ -371,6 +434,16 @@ def batched_cv(engine, X, y, test_folds, ests, specs, opts, scoring, return_trai
                 gap=np.zeros((n_cand, n_splits)), n_pass=np.zeros((n_cand, n_splits), dtype=int))
     need_r2 = "r2" in metrics.values()
     sst_test = np.array([float(((yv[t] - yv[t].mean()) ** 2).sum()) if need_r2 else 0.0 for t in test_folds])
+    need_d2 = "d2_absolute_error_score" in metrics.values()
+    stat_mask = _stat_mask(metrics)
+    if sharded and (stat_mask or need_d2):
+        raise ValueError("a sharded search scores the residual sums only: statistics and d2 need one rank's residuals")
+    # statistics per (candidate, fold) (rows 2-4 of slm_cv_score_stats); the training rows of fold f are scored as
+    # one row list [0, r0_f) + [r1_f, n) of the packed design, made once per call
+    EXT = np.zeros((3, n_cand, n_splits)) if stat_mask else None
+    TEXT = np.zeros((3, n_cand, n_splits)) if stat_mask and want_train else None
+    train_lists = {}
+    sad_test = [_abs_dev_median(yv[t]) if need_d2 else 0.0 for t in test_folds]
     tot_sum, tot_sq = float(yv.sum()), float((yv * yv).sum())
     n_unconverged = 0
     newton_stats = {}
@@ -422,21 +495,36 @@ def batched_cv(engine, X, y, test_folds, ests, specs, opts, scoring, return_trai
             # needs no exchange of coefficients; the partial tables are summed with the info tables below).
             # All (fold, row range) problems go through one batched scoring launch.
             icpt = (lambda f: out["intercept"][f]) if fd.fit_intercept else (lambda f: None)
-            items, where = [], []
+            items, where, titems, tfolds = [], [], [], []
             for f in range(n_splits):
                 kf = len(mine[f])
                 if kf == 0:
                     continue
                 items.append((fd.row_ptr[f], fd.row_ptr[f + 1], out["coef"][f], kf, icpt(f)))
                 where.append((0, f))
-                if want_train:
+                if want_train and stat_mask:
+                    if f not in train_lists:
+                        train_lists[f] = engine.to_device(np.concatenate(
+                            [np.arange(0, fd.row_ptr[f]), np.arange(fd.row_ptr[f + 1], n)]).astype(np.int32))
+                    titems.append((train_lists[f], out["coef"][f], kf, icpt(f)))
+                    tfolds.append(f)
+                elif want_train:
                     for r0, r1 in ((0, fd.row_ptr[f]), (fd.row_ptr[f + 1], n)):
                         if r1 > r0:
                             items.append((r0, r1, out["coef"][f], kf, icpt(f)))
                             where.append((1, f))
-            sc = np.zeros((n_splits, 2, K))
-            tsc = np.zeros((n_splits, 2, K)) if want_train else None
-            if items:
+            nst = 5 if stat_mask else 2
+            sc = np.zeros((n_splits, nst, K))
+            tsc = np.zeros((n_splits, nst, K)) if want_train else None
+            if items and stat_mask:
+                res = engine.cv_score_stats(fd.Xa, p, items, rows_scaled=wtd, stats=stat_mask).cpu().numpy()
+                if titems:
+                    tres = engine.cv_score_stats(fd.Xa, p, titems, rows_scaled=wtd, stats=stat_mask).cpu().numpy()
+                    for i, f in enumerate(tfolds):
+                        tsc[f] = tres[i][:, :K]
+                for i, (kind, f) in enumerate(where):
+                    sc[f] = res[i][:, :K]
+            elif items:
                 res = engine.cv_score_many(fd.Xa, p, items, rows_scaled=wtd).cpu().numpy()  # one D2H
                 for i, (kind, f) in enumerate(where):
                     tgt = sc if kind == 0 else tsc
@@ -448,6 +536,10 @@ def batched_cv(engine, X, y, test_folds, ests, specs, opts, scoring, return_trai
             SSE[idxs, f], SAE[idxs, f] = sc[f, 0], sc[f, 1]
             if want_train:
                 TSSE[idxs, f], TSAE[idxs, f] = tsc[f, 0], tsc[f, 1]
+            if stat_mask:
+                EXT[:, idxs, f] = sc[f, 2:]
+                if want_train:
+                    TEXT[:, idxs, f] = tsc[f, 2:]
             kf = len(mine[f])
             ci = idxs[mine[f]]
             info["n_iter"][ci, f] = out["n_iter"][f, :kf]
@@ -481,13 +573,19 @@ def batched_cv(engine, X, y, test_folds, ests, specs, opts, scoring, return_trai
     for f in range(n_splits):
         nt = len(test_folds[f])
         for m, scorer in metrics.items():
-            test_tabs[m][:, f] = _metric(scorer, SSE[:, f], SAE[:, f], nt, sst_test[f])
+            test_tabs[m][:, f] = _metric(scorer, SSE[:, f], SAE[:, f], nt, sst_test[f], _stats_of(EXT, f, sad_test[f]))
         if want_train:
             ntr = n - nt
             s_tr = tot_sum - float(yv[test_folds[f]].sum())
             q_tr = tot_sq - float((yv[test_folds[f]] ** 2).sum())
+            sad_tr = 0.0
+            if need_d2:
+                mask = np.ones(n, dtype=bool)
+                mask[test_folds[f]] = False
+                sad_tr = _abs_dev_median(yv[mask])
             for m, scorer in metrics.items():
-                train_tabs[m][:, f] = _metric(scorer, TSSE[:, f], TSAE[:, f], ntr, q_tr - s_tr * s_tr / ntr)
+                train_tabs[m][:, f] = _metric(scorer, TSSE[:, f], TSAE[:, f], ntr, q_tr - s_tr * s_tr / ntr,
+                                              _stats_of(TEXT, f, sad_tr))
     test_scores = test_tabs if multi else test_tabs["score"]
     train_scores = None
     if want_train:
@@ -602,8 +700,13 @@ class GridSearchCV(_SkGridSearchCV):
                 sw = v
             else:
                 return None
-        if _device_metrics(self.scoring) is None:
+        metrics = _device_metrics(self.scoring)
+        if metrics is None:
             return None
+        shard = getattr(self, "_shard", None)
+        if shard is not None and shard.world > 1 and _UNSHARDED_SCORERS & set(
+                [metrics] if isinstance(metrics, str) else metrics.values()):
+            return None  # DESIGN section 7: statistics of row-sharded residuals are not formed
         if callable(self.refit) or hasattr(X, "columns"):
             return None
         if not isinstance(_device_metrics(self.scoring), str) and self.refit is not False and (
@@ -630,7 +733,6 @@ class GridSearchCV(_SkGridSearchCV):
             splits = list(cv.split(Xv, yv, groups))
         except Exception:
             return None  # sklearn's loop raises the splitter's own error
-        shard = getattr(self, "_shard", None)
         route = _split_route(splits, n, 1 if shard is None else shard.world)
         if route is None:
             return None
