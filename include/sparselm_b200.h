@@ -289,6 +289,17 @@ int slm_cv_score_stats(slm_ctx* ctx, const double* Xa_dev, int64_t lda, int64_t 
                        const double* const* intercept_dev, int32_t rows_scaled, int32_t stats,
                        double* const* yhat_dev, const int64_t* ldy, double* const* out_dev, void* stream);
 
+/* ---- K11: stability selection counts (DESIGN section 2 item 17) ------------------------------------
+ * coef_dev is the [F][p][ldz] coefficient table of F fits x K candidate columns (slm_solve_batch / fold-back
+ * layout, F <= SLM_MAX_FOLDS, K <= ldz).  Coefficient j of fit (f, k) is selected iff
+ *   |coef[f][j][k]| > rel_tol * max_j' |coef[f][j'][k]|
+ * (an all-zero fit selects nothing; a NaN coefficient is never selected; columns k >= K are never read).
+ *   counts_dev[j][k] += number of fits f of the call that select j for candidate k   (int32 [p][K])
+ *   union_dev[f][j]   = 1 if some candidate k < K of fit f selects j, else left as is  (uint8 [F][p])
+ * Both accumulate over calls; no atomics on the counts, so the results are deterministic.  Only enqueues work. */
+int slm_support_counts(slm_ctx* ctx, const double* coef_dev, int F, int64_t p, int64_t ldz, int K, double rel_tol,
+                       int32_t* counts_dev, uint8_t* union_dev, void* stream);
+
 /* intercept[k] = ybar - mu^T B[:,k] from the (uncentred) training Gram's ones row
  * (LinearModel._set_intercept, _base.py:202). */
 int slm_intercepts(slm_ctx* ctx, const double* G_dev, int64_t pa, int64_t p,

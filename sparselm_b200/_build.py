@@ -11,7 +11,7 @@ CSRC = os.path.join(_PKG, "csrc")
 LIB_DIR = os.path.join(_PKG, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libsparselm_b200.so")
 SOURCES = ["engine.cu"]
-HEADERS = ["gemm_f64.cuh", "gemm_f64_tma.cuh", "solver_kernels.cuh", "whiten_kernels.cuh", "cg_kernels.cuh", "coop_kernels.cuh", "newton_kernels.cuh", os.path.join("..", "..", "include", "sparselm_b200.h")]
+HEADERS = ["gemm_f64.cuh", "gemm_f64_tma.cuh", "solver_kernels.cuh", "whiten_kernels.cuh", "cg_kernels.cuh", "coop_kernels.cuh", "newton_kernels.cuh", "select_kernels.cuh", os.path.join("..", "..", "include", "sparselm_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

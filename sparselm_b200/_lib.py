@@ -100,6 +100,7 @@ SYMBOLS = {
     "slm_cv_score_rows": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_vp, c_vp, c_vp]),
     "slm_cv_score_stats": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32,
                                           c_i32, c_vp, c_vp, c_vp, c_vp]),
+    "slm_support_counts": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, c_i64, c_i64, ctypes.c_int, c_dbl, c_vp, c_vp, c_vp]),
     "slm_intercepts": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp]),
     "slm_gram_apply": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, ctypes.c_int, ctypes.POINTER(c_i32), c_vp, c_i64, c_vp, c_vp]),
     "slm_newton_workspace": (c_sz, [c_i64, c_i32, c_i32, ctypes.c_int]),

@@ -12,6 +12,7 @@
 //   K9  fold back       fold_back_kernel
 //   K10 scoring         gemm_f64_kernel<A_MMAJOR> + score_kernel
 //   K10b statistics     stat_residual/final/median_kernel (max, percentage sum, median of |r|)
+//   K11 selection       support_colmax_kernel + support_count_kernel (stability selection counts)
 #include <cuda_runtime.h>
 #include <float.h>
 #include <math.h>
@@ -32,6 +33,7 @@
 #include "cg_kernels.cuh"
 #include "coop_kernels.cuh"
 #include "newton_kernels.cuh"
+#include "select_kernels.cuh"
 
 using namespace slm;
 
@@ -70,6 +72,8 @@ struct slm_ctx {
     unsigned long long* h_ratio = nullptr;
     int* h_scount = nullptr;         // pinned copy of the support-list lengths (chunk-width choice)
     double* h_scal = nullptr;        // pinned scalars of the conjugate-gradient loop
+    unsigned long long* d_colmax = nullptr;  // [F][ldz] column maxima of slm_support_counts (grown on demand)
+    size_t colmax_cap = 0;
     double apply_exec_flops = 0.0;   // flops the row-sparse applies executed (useful, unpadded)
     double apply_dense_flops = 0.0;  // 2 p^2 K_active of the same applies
     int chunk_w = 32;                // columns per support chunk (SLM_CHUNK_W)
@@ -1175,6 +1179,7 @@ void slm_destroy(slm_ctx* ctx) {
     if (ctx->h_scal) cudaFreeHost(ctx->h_scal);
     if (ctx->d_flags) cudaFree(ctx->d_flags);
     if (ctx->h_counter) cudaFreeHost(ctx->h_counter);
+    if (ctx->d_colmax) cudaFree(ctx->d_colmax);
     delete ctx;
 }
 
@@ -2351,6 +2356,34 @@ int slm_fold_back(slm_ctx* ctx, const double* Be, const int32_t* inv_ptr, const 
     dim3 grid((unsigned)((K + 127) / 128), (unsigned)p);
     fold_back_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(Be, inv_ptr, inv_idx, (int)p, ldz, K, coef);
     LAUNCH_OK("fold_back_kernel");
+    return 0;
+}
+
+int slm_support_counts(slm_ctx* ctx, const double* coef, int F, int64_t p, int64_t ldz, int K, double rel_tol,
+                       int32_t* counts, uint8_t* uni, void* stream) {
+    if (!ctx || !coef || !counts || !uni) return fail(ctx, 1, "slm_support_counts: null argument");
+    if (F < 0 || F > SLM_MAX_FOLDS || K < 0 || (int64_t)K > ldz || p < 0)
+        return fail(ctx, 1, "slm_support_counts: bad shape (need 0 <= F <= SLM_MAX_FOLDS, 0 <= K <= ldz)");
+    if (!(rel_tol >= 0.0 && rel_tol <= DBL_MAX)) return fail(ctx, 1, "slm_support_counts: rel_tol must be finite and >= 0");
+    if (F == 0 || K == 0 || p == 0) return 0;
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t need = (size_t)F * (size_t)ldz;
+    if (need > ctx->colmax_cap) {
+        // growing synchronises the device (cudaFree): it happens once per larger shape
+        if (ctx->d_colmax) CUDA_OK(cudaFree(ctx->d_colmax));
+        ctx->d_colmax = nullptr;
+        ctx->colmax_cap = 0;
+        CUDA_OK(cudaMalloc(&ctx->d_colmax, need * sizeof(unsigned long long)));
+        ctx->colmax_cap = need;
+    }
+    CUDA_OK(cudaMemsetAsync(ctx->d_colmax, 0, need * sizeof(unsigned long long), s));
+    const int rows_per_block = SEL_ROWS * SEL_RPT;
+    dim3 g1((unsigned)((K + 31) / 32), (unsigned)F, (unsigned)((p + rows_per_block - 1) / rows_per_block));
+    support_colmax_kernel<<<g1, dim3(32, SEL_ROWS), 0, s>>>(coef, p, ldz, K, ctx->d_colmax);
+    LAUNCH_OK("support_colmax_kernel");
+    support_count_kernel<<<(unsigned)((p + SEL_ROWS - 1) / SEL_ROWS), dim3(32, SEL_ROWS), 0, s>>>(
+        coef, F, p, ldz, K, rel_tol, ctx->d_colmax, counts, uni);
+    LAUNCH_OK("support_count_kernel");
     return 0;
 }
 

@@ -1281,6 +1281,18 @@ class Engine:
                                         p, ldz, K, self._ptr(coef), self.stream), "slm_fold_back")
         return coef
 
+    def support_counts(self, coef, K, rel_tol, counts, union):
+        """Selection counts of the [F, p, ldz] coefficient table `coef` (slm_support_counts): counts [p, K] int32
+        += fits that select (j, k); union [F, p] uint8 |= some candidate of fit f selects j.  Selected:
+        |b_j| > rel_tol * max_j' |b_j'| within one fit.  Both accumulate in place on the device."""
+        torch = self.torch
+        F, p, ldz = coef.shape
+        assert coef.dtype == torch.float64 and coef.is_contiguous()
+        assert counts.dtype == torch.int32 and counts.is_contiguous() and tuple(counts.shape) == (p, K)
+        assert union.dtype == torch.uint8 and union.is_contiguous() and tuple(union.shape) == (F, p)
+        self._ck(self.lib.slm_support_counts(self.h, self._ptr(coef), F, p, ldz, int(K), float(rel_tol),
+                                             self._ptr(counts), self._ptr(union), self.stream), "slm_support_counts")
+
     def intercepts(self, G, p, B, K):
         torch = self.torch
         ldz = B.shape[-1]

@@ -642,6 +642,36 @@ def _sharded_residual_sums(engine, shard, fd, out, owner, mine, p, K, n_splits, 
     return part, tpart
 
 
+def describe_candidates(est, candidates, X, y, on_first=None):
+    """(ests, specs) of the candidates (dicts of parameters of `est`) on the design X, y: per candidate a namespace
+    holding its fit_intercept and its ProblemSpec.  on_first(ests[0], specs[0]) runs once the first candidate is
+    described, before the others (GridSearchCV enqueues its device preparation there)."""
+    from types import SimpleNamespace
+
+    p = X.shape[1]
+    ests, specs = [], []
+    # one working estimator re-parametrised per candidate (cloning 100 estimators and
+    # re-deriving their group structure costs more host time than the GPU solve)
+    work = clone(est)
+    for ci, c in enumerate(candidates):
+        work.set_params(**c)
+        if ci == 1:
+            # from the second candidate on only the grid's own parameters are re-validated, and the
+            # group structure memoised for the first candidate is reused without re-hashing `groups`
+            # (the working estimator is private to this loop)
+            work.__dict__["_validate_only"] = set().union(*[set(cc) for cc in candidates])
+            work.__dict__["_groups_frozen"] = True
+        with warnings.catch_warnings():
+            if ci > 0:  # structural warnings (e.g. groups=None) are emitted once
+                warnings.simplefilter("ignore", UserWarning)
+            work._validate_hyperparams(X, y)
+        ests.append(SimpleNamespace(fit_intercept=bool(work.fit_intercept)))
+        specs.append(work._problem_spec(p))
+        if ci == 0 and on_first is not None:
+            on_first(ests[0], specs[0])
+    return ests, specs
+
+
 class GridSearchCV(_SkGridSearchCV):
     """Exhaustive search over a parameter grid, batched on the GPU for engine-backed
     estimators.  Same constructor as the reference (model_selection.py:160-187):
@@ -740,49 +770,30 @@ class GridSearchCV(_SkGridSearchCV):
         valid = set(est.get_params(deep=False))
         if any(not set(c) <= valid for c in candidates):
             return None
-        ests, specs = [], []
         pre_fds = {}
-        try:
-            # one working estimator re-parametrised per candidate (cloning 100 estimators and
-            # re-deriving their group structure costs more host time than the GPU solve)
-            work = clone(est)
-            import warnings as _w
-            from types import SimpleNamespace
 
-            for ci, c in enumerate(candidates):
-                work.set_params(**c)
-                if ci == 1:
-                    # from the second candidate on only the grid's own parameters are re-validated, and the
-                    # group structure memoised for the first candidate is reused without re-hashing `groups`
-                    # (the working estimator is private to this loop)
-                    work.__dict__["_validate_only"] = set().union(*[set(cc) for cc in candidates])
-                    work.__dict__["_groups_frozen"] = True
-                with _w.catch_warnings():
-                    if ci > 0:  # structural warnings (e.g. groups=None) are emitted once
-                        _w.simplefilter("ignore", UserWarning)
-                    work._validate_hyperparams(Xv, yv)
-                ests.append(SimpleNamespace(fit_intercept=bool(work.fit_intercept)))
-                specs.append(work._problem_spec(p))
-                if ci == 0:
-                    # the design of the first candidate starts its way to the device (H2D, packing,
-                    # Gram build are only enqueued) while the host describes the other candidates
-                    opts0 = est._engine_options()
-                    engine = get_engine(opts0.pop("device", None))
-                    cache = getattr(self, "_fd_cache", None)
-                    cache_key = None if cache is None else (id(Xv), id(yv), None if sw is None else sw.tobytes())
-                    if route == "splits":
-                        cache_key = _splits_cache_key(cache, Xv, yv, sw)
-                        pre_fds[_fold_key(ests[0], specs[0])] = prepare_split_data(
-                            engine, Xv, yv, splits, ests[0], specs[0], cache, cache_key, sw)
-                        continue
-                    score_folds = None
-                    if shard is not None and shard.world > 1 and cache is None:
-                        # host rows this rank needs: its slice of every fold (Gram build and scoring
-                        # are both row-sharded)
-                        score_folds = set()
-                    pre_fds[_fold_key(ests[0], specs[0])] = prepare_folds(
-                        engine, Xv, yv, [np.asarray(test) for _, test in splits], ests[0], specs[0], cache,
-                        cache_key, shard, sw, score_folds)
+        def start_prepare(e0, s0):
+            # the design of the first candidate starts its way to the device (H2D, packing,
+            # Gram build are only enqueued) while the host describes the other candidates
+            opts0 = est._engine_options()
+            engine = get_engine(opts0.pop("device", None))
+            cache = getattr(self, "_fd_cache", None)
+            cache_key = None if cache is None else (id(Xv), id(yv), None if sw is None else sw.tobytes())
+            if route == "splits":
+                cache_key = _splits_cache_key(cache, Xv, yv, sw)
+                pre_fds[_fold_key(e0, s0)] = prepare_split_data(engine, Xv, yv, splits, e0, s0, cache, cache_key, sw)
+                return
+            score_folds = None
+            if shard is not None and shard.world > 1 and cache is None:
+                # host rows this rank needs: its slice of every fold (Gram build and scoring
+                # are both row-sharded)
+                score_folds = set()
+            pre_fds[_fold_key(e0, s0)] = prepare_folds(
+                engine, Xv, yv, [np.asarray(test) for _, test in splits], e0, s0, cache,
+                cache_key, shard, sw, score_folds)
+
+        try:
+            ests, specs = describe_candidates(est, candidates, Xv, yv, on_first=start_prepare)
         except (NotImplementedError, EngineError):
             raise
         except Exception:
