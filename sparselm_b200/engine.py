@@ -527,14 +527,14 @@ class Engine:
 
     # ---- data preparation for a CV search / a plain fit --------------------
     def prepare(self, X, y, test_folds=None, fit_intercept=False, sample_weight=None, col_perm=None, shard=None,
-                score_folds=None):
+                own_rows=False):
         """Pack the design, build per-fold training Grams + the full Gram.
 
         test_folds: list of index arrays forming a partition of range(n) (the CV
         test sets), or None for a single fit on all rows.
-        score_folds: (sharded searches on a host-resident X) the test folds this rank will
-        score; rows of other folds are only brought to the device as far as this rank's
-        share of the Gram build needs them.  None = every row.
+        own_rows: (sharded searches on a host-resident X) bring only this rank's slice of
+        every test fold's rows to the device, the rows its share of the Gram build and of the
+        scoring needs.  False = every row.
         """
         if isinstance(X, self.torch.Tensor):
             n, p = X.shape
@@ -564,14 +564,14 @@ class Engine:
         # rows of every test fold whose Gram block this rank builds (all of them unless sharded)
         fold_rows = shard.fold_row_ranges(row_ptr) if sharded else \
             [(int(row_ptr[f]), int(row_ptr[f + 1])) for f in range(F)]
-        partial = False  # did the prepare routine leave rows of unscored folds unpacked?
+        partial = False  # did the prepare routine leave the rows of other ranks unpacked?
         self._complemented = False  # set by the sharded reduce when it already produced training Grams + total
         if on_host and row_perm is None and n >= 4096:
             Xa, allG, partial = self._prepare_pipelined(X, y, sw, col_perm, row_ptr, fold_rows,
-                                                        shard if sharded else None, score_folds if sharded else None)
+                                                        shard if sharded else None, own_rows and sharded)
         elif sharded:
             Xa, allG, partial = self._prepare_sharded(X, y, sw, col_perm, row_perm, row_ptr, fold_rows, shard,
-                                                      score_folds)
+                                                      own_rows)
         else:
             Xa = self.pack(X, y, sw, col_perm, row_perm)
             allG = self.gram_blocks(Xa, row_ptr, extra=1 if F > 1 else 0)
@@ -600,33 +600,12 @@ class Engine:
             if F > 1:
                 self.gram_center(G_train, p)
         if partial:
-            # rows of the other folds reached the device only as far as the Gram build needed
-            extra["partial_folds"] = {f for f in range(F) if f not in score_folds}
-            extra["pack_args"] = (sw, col_perm)
+            # only this rank's slice of every fold's rows reached the device
+            extra["partial_folds"] = True
         finite = self.torch.isfinite(G_full[p + 1]).all()  # checked at the next host sync
         return FoldData(n=n, p=p, pa=pa, Xa=Xa, row_ptr=row_ptr, G_train=G_train, G_full=G_full,
                         n_train=n_train, fit_intercept=bool(fit_intercept), row_perm=row_perm, extra=extra,
                         G_all=allG if F > 1 else None, _finite=finite)
-
-    def ensure_fold_rows(self, fd, X, y, f):
-        """Make every row of test fold f resident in fd.Xa (a sharded prepare only uploads the
-        folds it expects to score; anything else is fetched on demand here)."""
-        part = fd.extra.get("partial_folds")
-        if not part or f not in part:
-            return
-        torch = self.torch
-        sw, col_perm = fd.extra["pack_args"]
-        a, b = int(fd.row_ptr[f]), int(fd.row_ptr[f + 1])
-        Xt = X if isinstance(X, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(X, dtype=np.float64))
-        blk = self.to_device(Xt[a:b], torch.float64)
-        yd = self.to_device(np.asarray(y, dtype=np.float64)[a:b])
-        swd = None if sw is None else self.to_device(np.asarray(sw, dtype=np.float64)[a:b])
-        cp = None if col_perm is None else self.to_device(np.asarray(col_perm, dtype=np.int32))
-        self._ck(self.lib.slm_pack_design(self.h, self._ptr(blk), blk.stride(0), self._ptr(yd), self._ptr(swd),
-                                          self._ptr(cp), ctypes.c_void_p(0), b - a, fd.p,
-                                          ctypes.c_void_p(fd.Xa.data_ptr() + 8 * a * fd.pa), fd.pa, self.stream),
-                 "slm_pack_design")
-        part.discard(f)
 
     def prepare_splits(self, X, y, splits, fit_intercept=False, sample_weight=None, col_perm=None):
         """Pack the design in its original row order and build the full Gram, for a CV search over
@@ -716,14 +695,13 @@ class Engine:
                                           ptr.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), 1,
                                           ctypes.c_void_p(out.data_ptr()), self.stream), "slm_gram_blocks")
 
-    def _prepare_sharded(self, X, y, sw, col_perm, row_perm, row_ptr, fold_rows, shard, score_folds=None):
+    def _prepare_sharded(self, X, y, sw, col_perm, row_perm, row_ptr, fold_rows, shard, own_rows=False):
         """Row-sharded Gram build (SURVEY 8e): this rank contributes, for every test fold, the
         Gram of its own 1/world slice of that fold's rows; the blocks are then summed over the
-        ranks.  Only the rows this rank needs are packed: its slices, plus the whole test folds
-        in `score_folds` (None = everything)."""
+        ranks.  With `own_rows` only this rank's slices are packed (everything otherwise)."""
         torch = self.torch
         F = len(row_ptr) - 1
-        partial = not (score_folds is None or row_perm is not None or F == 1)
+        partial = own_rows and row_perm is None and F > 1
         if not partial:
             Xa = self.pack(X, y, sw, col_perm, row_perm)
         else:
@@ -733,8 +711,7 @@ class Engine:
             cp = None if col_perm is None else self.to_device(np.asarray(col_perm, dtype=np.int32))
             n, p = Xd.shape
             Xa = torch.empty((n, self.padded_cols(p)), dtype=torch.float64, device=self.device)
-            for f in range(F):
-                a, b = (int(row_ptr[f]), int(row_ptr[f + 1])) if f in score_folds else fold_rows[f]
+            for a, b in fold_rows:
                 self._pack_rows(Xd, yd, swd, cp, a, b, Xa)
         pa = Xa.shape[1]
         allG = torch.zeros((F + (1 if F > 1 else 0), pa, pa), dtype=torch.float64, device=self.device)
@@ -785,13 +762,14 @@ class Engine:
                                           ctypes.c_void_p(Xa.data_ptr() + 8 * a * pa), pa, self.stream),
                  "slm_pack_design")
 
-    def _prepare_pipelined(self, X, y, sw, col_perm, row_ptr, fold_rows, shard=None, score_folds=None):
+    def _prepare_pipelined(self, X, y, sw, col_perm, row_ptr, fold_rows, shard=None, own_rows=False):
         """Host-resident X: the rows of one test fold at a time are copied to the device on a
         copy stream while the previous fold is packed and its Gram block is built, so the
         H2D transfer hides behind the FP64 tensor work (needs pinned memory to be truly
         asynchronous; pageable arrays still overlap chunk by chunk).  fold_rows[f] = the rows
         of fold f whose Gram this rank builds; with `shard` the blocks are then summed over the
-        ranks (one all-reduce of the packed upper triangles)."""
+        ranks (one all-reduce of the packed upper triangles); with `own_rows` (F > 1) only those
+        rows travel."""
         torch = self.torch
         Xt = X if isinstance(X, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(X, dtype=np.float64))
         if Xt.dtype != torch.float64:
@@ -814,8 +792,8 @@ class Engine:
         max_rows = max(1024, self.PIPELINE_BLOCK_BYTES // (8 * p))
         for f in range(F):
             a, b = int(row_ptr[f]), int(row_ptr[f + 1])
-            if F > 1 and score_folds is not None and f not in score_folds:
-                a, b = fold_rows[f]  # not scored here: only this rank's slice of the fold travels
+            if F > 1 and own_rows:
+                a, b = fold_rows[f]  # only this rank's slice of the fold travels
                 if b <= a:
                     if shard is not None:
                         blocks.append((a, a))  # nothing to build, but the collective still runs
@@ -852,7 +830,7 @@ class Engine:
                 started.add(f)
         if shard is not None:
             self._complemented = self._allreduce_grams(allG, F, shard)
-        return Xa, allG, bool(F > 1 and score_folds is not None)
+        return Xa, allG, bool(F > 1 and own_rows)
 
     # ---- K5-K8: batched solve ------------------------------------------------
     def solve(self, G, p, n_obs, lipschitz, grids, B0=None, tol=1e-10, floor_rel=1e-14, max_iter=20000,

@@ -35,7 +35,7 @@ from sklearn.model_selection._search import BaseSearchCV
 from sklearn.utils.validation import check_X_y
 
 from .engine import EngineError, get_engine, split_chunks
-from .model._base import EngineRegressor, _to_original_order, solve_specs
+from .model._base import EngineRegressor, solve_specs
 
 __all__ = ["GridSearchCV", "LineSearchCV"]
 
@@ -210,30 +210,32 @@ def _fold_key(est, spec):
     return (bool(est.fit_intercept), None if spec.col_perm is None else spec.col_perm.tobytes())
 
 
-def prepare_folds(engine, X, yv, test_folds, est, spec, cache=None, cache_key=None, shard=None, sample_weight=None,
-                  score_folds=None):
+def prepare_folds(engine, X, yv, test_folds, est, spec, cache=None, cache_key=None, shard=None, sample_weight=None):
     """Device-resident design + Grams for (fit_intercept, column order) of `est`/`spec`,
     through the FoldData cache of a LineSearchCV when there is one.  Only enqueues GPU
-    work (H2D copies, packing, Gram build): the caller can keep working on the host."""
+    work (H2D copies, packing, Gram build): the caller can keep working on the host.
+    A sharded rank uploads only its own slice of every fold's rows (Gram build and scoring are both
+    row-sharded) when the design comes from the host; a design that is already device-resident, or the
+    cached one of a LineSearchCV, is kept whole."""
     ck = None
     if cache is not None and cache_key is not None:
         # keyed on the full content of the split: a shuffling splitter draws a new partition per
         # line, and two partitions can agree in fold sizes and first indices
-        import hashlib
-
         fold_hash = hashlib.sha1(np.concatenate([np.asarray(t, dtype=np.int64) for t in test_folds]).tobytes()).hexdigest()
         ck = (cache_key, _fold_key(est, spec), tuple(len(t) for t in test_folds), fold_hash)
         if ck in cache:
             return cache[ck]
+    own_rows = (shard is not None and shard.world > 1 and cache is None
+                and not (isinstance(X, engine.torch.Tensor) and X.is_cuda))
     fd = engine.prepare(X, yv, test_folds, est.fit_intercept, sample_weight, col_perm=spec.col_perm, shard=shard,
-                        score_folds=score_folds)
+                        own_rows=own_rows)
     if ck is not None:
         cache[ck] = fd
     return fd
 
 
-def _splits_cache_key(cache, Xv, yv, sw):
-    """Data part of the SplitData cache key of a LineSearchCV: the identity of X (check_X_y returns the float64 design
+def _cache_key(cache, Xv, yv, sw):
+    """Data part of the device-data cache key of a LineSearchCV: the identity of X (check_X_y returns the float64 design
     it was given) and the content of y and of the weights (check_X_y returns a new y object at every line)."""
     if cache is None:
         return None
@@ -271,6 +273,142 @@ def _stats_of(ext, s, sad):
     return d
 
 
+def candidate_batches(specs):
+    """{structure key: candidate indices}: the candidates solved as one batch, in order of increasing penalty strength
+    (dense iterates first: the row-sparse apply shares one support list per chunk of adjacent columns)."""
+    batches = {}
+    for ci, s in enumerate(specs):
+        batches.setdefault(s.key, []).append(ci)
+    return {k: np.asarray(sorted(v, key=lambda ci: (specs[ci].strength, ci))) for k, v in batches.items()}
+
+
+class _SolveInfo:
+    """Solver info of a search's (candidate, cell) grid: the n_iter / status / gap / n_pass tables [n_cand, n_cells],
+    the number of unconverged problems, the iterations run and the Newton-phase totals (engine._run_batch)."""
+
+    def __init__(self, n_cand, n_cells):
+        self.tables = dict(n_iter=np.zeros((n_cand, n_cells), dtype=int), status=np.zeros((n_cand, n_cells), dtype=int),
+                           gap=np.zeros((n_cand, n_cells)), n_pass=np.zeros((n_cand, n_cells), dtype=int))
+        self.n_unconverged, self.iters_run, self.newton = 0, 0, {}
+
+    def record(self, out, cells, cands):
+        """Take one solve_specs output whose slot f solved cell cells[f] for the candidates cands[f] (its first
+        len(cands[f]) columns)."""
+        for f, (c, ci) in enumerate(zip(cells, cands)):
+            for k, t in self.tables.items():
+                t[ci, c] = out[k][f, :len(ci)]
+        self.n_unconverged += int(out["n_unconverged"])
+        self.iters_run += int(out["iters_run"])
+        for k, v in (out.get("newton") or {}).items():
+            self.newton[k] = self.newton.get(k, 0) + v
+
+    def allreduce(self, shard, device, resid):
+        """The last exchange of a sharded grid: ONE sum over the ranks of the residual tables `resid` (returned), the
+        info tables and n_unconverged.  iters_run and newton stay this rank's."""
+        tabs = [resid] + [t.astype(np.float64) for t in self.tables.values()] + [np.array([float(self.n_unconverged)])]
+        flat = shard.allreduce_sum_numpy(np.concatenate([t.ravel() for t in tabs]), device)
+        o = resid.size
+        resid = flat[:o].reshape(resid.shape)
+        for k, t in self.tables.items():
+            self.tables[k] = flat[o:o + t.size].reshape(t.shape).astype(t.dtype)
+            o += t.size
+        self.n_unconverged = int(round(float(flat[o])))
+        return resid
+
+
+def _residual_tables(n_cand, n_cells, want_train, stat_mask):
+    """Zeroed residual tables of a search: [kind][row][n_cand][n_cells], kind 0 the test rows and 1 the training rows
+    (only with train scores); rows Σr², Σ|r| and, when a scorer needs a statistic (stat_mask), max |r|, the
+    percentage sum and median |r| (the rows of slm_cv_score_stats)."""
+    return np.zeros((2 if want_train else 1, 5 if stat_mask else 2, n_cand, n_cells))
+
+
+def _split_cells(yv, splits, metrics, want_train):
+    """Per split (n_rows, sst, sad) of its test rows and of its training rows (None without train scores): the inputs
+    of _scores.  sst and sad are 0.0 where no metric needs them (r2, d2_absolute_error_score)."""
+    need_r2 = "r2" in metrics.values()
+    need_d2 = "d2_absolute_error_score" in metrics.values()
+
+    def cell(rows):
+        v = yv[np.asarray(rows)]
+        return (len(v), float(((v - v.mean()) ** 2).sum()) if need_r2 and len(v) else 0.0,
+                _abs_dev_median(v) if need_d2 else 0.0)
+
+    return [cell(te) for _, te in splits], [cell(tr) for tr, _ in splits] if want_train else None
+
+
+def _partition_cells(yv, test_folds, metrics, want_train):
+    """_split_cells of a partition: the sst of a fold's training rows is downdated from the sums over all rows,
+    q_tr - s_tr^2 / n_tr."""
+    need_r2 = "r2" in metrics.values()
+    need_d2 = "d2_absolute_error_score" in metrics.values()
+    n = len(yv)
+    test_cells, train_cells = [], [] if want_train else None
+    tot_sum, tot_sq = float(yv.sum()), float((yv * yv).sum())
+    for t in test_folds:
+        v = yv[t]
+        test_cells.append((len(t), float(((v - v.mean()) ** 2).sum()) if need_r2 else 0.0,
+                           _abs_dev_median(v) if need_d2 else 0.0))
+        if want_train:
+            ntr = n - len(t)
+            s_tr, q_tr = tot_sum - float(v.sum()), tot_sq - float((v ** 2).sum())
+            sad_tr = 0.0
+            if need_d2:
+                mask = np.ones(n, dtype=bool)
+                mask[t] = False
+                sad_tr = _abs_dev_median(yv[mask])
+            train_cells.append((ntr, q_tr - s_tr * s_tr / ntr, sad_tr))
+    return test_cells, train_cells
+
+
+def _scores(scoring, metric, resid, test_cells, train_cells=None):
+    """(test_scores, train_scores) of a search: per metric of `scoring` (one scorer name, or {metric name: scorer
+    name}) a table [n_cand, n_cells] formed by `metric` from the residual tables (_residual_tables) and the per-cell
+    (n_rows, sst, sad) of the test rows and of the training rows (None: no train scores).  `metric` is _metric on a
+    partition and _split_metric on arbitrary splits: they differ in r2 on one row."""
+    multi = not isinstance(scoring, str)
+    metrics = dict(scoring) if multi else {"score": scoring}
+    out = [None, None]
+    for kind, cells in enumerate((test_cells, train_cells)[:len(resid)]):
+        R = resid[kind]
+        tabs = {m: np.empty(R.shape[1:]) for m in metrics}
+        for c, (n_rows, sst, sad) in enumerate(cells):
+            for m, scorer in metrics.items():
+                tabs[m][:, c] = metric(scorer, R[0][:, c], R[1][:, c], n_rows, sst,
+                                       _stats_of(R[2:] if len(R) > 2 else None, c, sad))
+        out[kind] = tabs if multi else tabs["score"]
+    return out
+
+
+def split_batches(engine, X, yv, splits, ests, specs, opts, sds, cache=None, cache_key=None, sample_weight=None):
+    """The (batch, chunk) loop of a search over arbitrary splits.  Per structure key yields (fkey, sd, idxs, chunks):
+    the SplitData of the batch's (fit_intercept, column order), prepared on first use into `sds`; the batch's
+    candidates (candidate_batches); and a generator that yields per chunk of at most 16 splits (c0, order, fd, out, t):
+    the chunk's training Grams (Engine.split_chunk: slot j holds split order[j], c0 the chunk's first split), every
+    candidate of the batch solved on them (solve_specs) and the host time the two took.  One [16, pa, pa] buffer
+    serves every chunk and batch: a batch's chunks are walked before the next batch is asked for."""
+    chunks = split_chunks(len(splits))
+    buf = None
+    for idxs in candidate_batches(specs).values():
+        s0, e0 = specs[idxs[0]], ests[idxs[0]]
+        fkey = _fold_key(e0, s0)
+        if fkey not in sds:
+            sds[fkey] = prepare_split_data(engine, X, yv, splits, e0, s0, cache, cache_key, sample_weight)
+        sd = sds[fkey]
+        if buf is None:
+            buf = engine.torch.empty((chunks[0][1] - chunks[0][0], sd.pa, sd.pa), dtype=engine.torch.float64,
+                                     device=engine.device)
+        yield fkey, sd, idxs, _solved_chunks(engine, sd, [specs[ci] for ci in idxs], chunks, buf, opts)
+
+
+def _solved_chunks(engine, sd, bspecs, chunks, buf, opts):
+    for c0, c1 in chunks:
+        t0 = time.perf_counter()
+        order, fd = engine.split_chunk(sd, c0, c1, buf)
+        out = solve_specs(engine, fd, bspecs, **opts)
+        yield c0, order, fd, out, time.perf_counter() - t0
+
+
 def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_train_score=False, cache=None,
                       cache_key=None, sds=None, sample_weight=None):
     """batched_cv for arbitrary splits (list of (train, test) index arrays, see _split_route): the training Grams of
@@ -281,61 +419,26 @@ def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_t
     minus the rows outside its training set (the residual sums are additive), or, when a statistic is needed (a
     median does not downdate), the explicit list of its training rows, made for the chunk and dropped after it.
     Returns the same dict as batched_cv; its "fds" hold the refit data (SplitData.full)."""
-    torch = engine.torch
     yv = np.asarray(y, dtype=np.float64)
     n = yv.shape[0]
     p = X.shape[1]
     n_splits, n_cand = len(splits), len(specs)
-    multi = not isinstance(scoring, str)
-    metrics = dict(scoring) if multi else {"score": scoring}
+    metrics = {"score": scoring} if isinstance(scoring, str) else dict(scoring)
     want_train = bool(return_train_score)
-    SSE, SAE = np.zeros((n_cand, n_splits)), np.zeros((n_cand, n_splits))
-    TSSE, TSAE = (np.zeros((n_cand, n_splits)), np.zeros((n_cand, n_splits))) if want_train else (None, None)
+    stat_mask = _stat_mask(metrics)
+    resid = _residual_tables(n_cand, n_splits, want_train, stat_mask)
     fit_time = np.zeros(n_cand)
     score_time = np.zeros(n_cand)
-    info = dict(n_iter=np.zeros((n_cand, n_splits), dtype=int), status=np.zeros((n_cand, n_splits), dtype=int),
-                gap=np.zeros((n_cand, n_splits)), n_pass=np.zeros((n_cand, n_splits), dtype=int))
-    need_r2 = "r2" in metrics.values()
-    need_d2 = "d2_absolute_error_score" in metrics.values()
-    stat_mask = _stat_mask(metrics)
-    # max |r|, percentage sum, median |r| per (candidate, split): rows 2-4 of slm_cv_score_stats
-    EXT = np.zeros((3, n_cand, n_splits)) if stat_mask else None
-    TEXT = np.zeros((3, n_cand, n_splits)) if stat_mask and want_train else None
-
-    def sst(rows):
-        v = yv[rows]
-        return float(((v - v.mean()) ** 2).sum()) if need_r2 and len(v) else 0.0
-
-    sst_test = np.array([sst(np.asarray(te)) for _, te in splits])
-    sst_train = np.array([sst(np.asarray(tr)) for tr, _ in splits]) if want_train else None
-    sad_test = [_abs_dev_median(yv[np.asarray(te)]) if need_d2 else 0.0 for _, te in splits]
-    sad_train = [_abs_dev_median(yv[np.asarray(tr)]) if need_d2 else 0.0 for tr, _ in splits] if want_train else None
-    n_unconverged, iters_run, newton_stats = 0, 0, {}
+    info = _SolveInfo(n_cand, n_splits)
     sds = {} if sds is None else dict(sds)
     warm = _WarmStarts()
-    batches = {}
-    for ci, s in enumerate(specs):
-        batches.setdefault(s.key, []).append(ci)
-    chunks = split_chunks(n_splits)
-    buf = None  # training Grams of one chunk, reused by every chunk and batch
-    for key, idxs in batches.items():
-        s0_, e0 = specs[idxs[0]], ests[idxs[0]]
-        fkey = _fold_key(e0, s0_)
-        if fkey not in sds:
-            sds[fkey] = prepare_split_data(engine, X, yv, splits, e0, s0_, cache, cache_key, sample_weight)
-        sd = sds[fkey]
-        if buf is None:
-            buf = torch.empty((chunks[0][1] - chunks[0][0], sd.pa, sd.pa), dtype=torch.float64, device=engine.device)
-        idxs = np.asarray(sorted(idxs, key=lambda ci: (specs[ci].strength, ci)))
+    for _, sd, idxs, chunks in split_batches(engine, X, yv, splits, ests, specs, opts, sds, cache, cache_key,
+                                             sample_weight):
         K = len(idxs)
-        bspecs = [specs[ci] for ci in idxs]
-        for c0, c1 in chunks:
-            t0 = time.perf_counter()
-            order, fd = engine.split_chunk(sd, c0, c1, buf)
-            out = solve_specs(engine, fd, bspecs, **opts)
+        for c0, order, fd, out, t_solve in chunks:
             t1 = time.perf_counter()
             if c0 == 0:
-                warm.add(out["B"], idxs, [np.arange(K)] * (c1 - c0))
+                warm.add(out["B"], idxs, [np.arange(K)] * len(order))
             icpt = (lambda f: out["intercept"][f]) if sd.fit_intercept else (lambda f: None)
             rows_items, rows_where, range_items, range_where = [], [], [], []
             for f, s in enumerate(order):
@@ -363,39 +466,17 @@ def batched_cv_splits(engine, X, y, splits, ests, specs, opts, scoring, return_t
             res_r = None if res_r is None else res_r.cpu().numpy()
             for r, wh in ((res, rows_where), (res_r, range_where)):
                 for i, (kind, s, sign) in enumerate(wh):
-                    if kind == 0:
-                        SSE[idxs, s] += sign * r[i, 0, :K]
-                        SAE[idxs, s] += sign * r[i, 1, :K]
-                    else:
-                        TSSE[idxs, s] += sign * r[i, 0, :K]
-                        TSAE[idxs, s] += sign * r[i, 1, :K]
+                    resid[kind][:2, idxs, s] += sign * r[i, :2, :K]
                     if stat_mask:  # one item per split and kind: the statistics are not summed
-                        (EXT if kind == 0 else TEXT)[:, idxs, s] = r[i, 2:5, :K]
+                        resid[kind][2:, idxs, s] = r[i, 2:5, :K]
             t2 = time.perf_counter()
-            for f, s in enumerate(order):
-                info["n_iter"][idxs, s] = out["n_iter"][f, :K]
-                info["status"][idxs, s] = out["status"][f, :K]
-                info["gap"][idxs, s] = out["gap"][f, :K]
-                info["n_pass"][idxs, s] = out["n_pass"][f, :K]
-            fit_time[idxs] += (t1 - t0) / (K * n_splits)
+            info.record(out, order, [idxs] * len(order))
+            fit_time[idxs] += t_solve / (K * n_splits)
             score_time[idxs] += (t2 - t1) / (K * n_splits)
-            n_unconverged += int(out["n_unconverged"])
-            iters_run += int(out["iters_run"])
-            for k, v in (out.get("newton") or {}).items():
-                newton_stats[k] = newton_stats.get(k, 0) + v
-    test_tabs = {m: np.empty((n_cand, n_splits)) for m in metrics}
-    train_tabs = {m: np.empty((n_cand, n_splits)) for m in metrics} if want_train else None
-    for s, (tr, te) in enumerate(splits):
-        for m, scorer in metrics.items():
-            test_tabs[m][:, s] = _split_metric(scorer, SSE[:, s], SAE[:, s], len(te), sst_test[s],
-                                               _stats_of(EXT, s, sad_test[s]))
-            if want_train:
-                train_tabs[m][:, s] = _split_metric(scorer, TSSE[:, s], TSAE[:, s], len(tr), sst_train[s],
-                                                    _stats_of(TEXT, s, sad_train[s]))
-    return dict(test_scores=test_tabs if multi else test_tabs["score"],
-                train_scores=None if not want_train else (train_tabs if multi else train_tabs["score"]),
-                fit_time=fit_time, score_time=score_time, info=info, fds={k: v.full for k, v in sds.items()},
-                n_unconverged=n_unconverged, iters_run=iters_run, warm=warm, newton=newton_stats)
+    test_scores, train_scores = _scores(scoring, _split_metric, resid, *_split_cells(yv, splits, metrics, want_train))
+    return dict(test_scores=test_scores, train_scores=train_scores, fit_time=fit_time, score_time=score_time,
+                info=info.tables, fds={k: v.full for k, v in sds.items()}, n_unconverged=info.n_unconverged,
+                iters_run=info.iters_run, warm=warm, newton=info.newton)
 
 
 def batched_cv(engine, X, y, test_folds, ests, specs, opts, scoring, return_train_score=False, cache=None,
@@ -415,58 +496,35 @@ def batched_cv(engine, X, y, test_folds, ests, specs, opts, scoring, return_trai
     n, p = X.shape
     n_splits, n_cand = len(test_folds), len(specs)
     yv = np.asarray(y, dtype=np.float64)
-    torch = engine.torch
     # one scorer name, or {metric name: scorer name}: every device scorer derives from the same
     # two residual sums, so a multi-metric search costs nothing extra on the GPU
-    multi = not isinstance(scoring, str)
-    metrics = dict(scoring) if multi else {"score": scoring}
+    metrics = {"score": scoring} if isinstance(scoring, str) else dict(scoring)
     sharded = shard is not None and shard.world > 1
-    # residual sums per (candidate, fold): sum of squares and of absolute values over the test rows
-    # (and over the training rows when train scores are asked for).  A sharded search fills in the
-    # sums of ITS rows of every fold (scoring is row-sharded like the Gram build) and the tables are
-    # summed over the ranks; the metrics are formed from the complete sums afterwards.
     want_train = bool(return_train_score)
-    SSE, SAE = np.zeros((n_cand, n_splits)), np.zeros((n_cand, n_splits))
-    TSSE, TSAE = (np.zeros((n_cand, n_splits)), np.zeros((n_cand, n_splits))) if want_train else (None, None)
+    stat_mask = _stat_mask(metrics)
+    if sharded and (stat_mask or "d2_absolute_error_score" in metrics.values()):
+        raise ValueError("a sharded search scores the residual sums only: statistics and d2 need one rank's residuals")
+    # residual sums per (candidate, fold) over the test rows (and over the training rows when train scores are asked
+    # for).  A sharded search fills in the sums of ITS rows of every fold (scoring is row-sharded like the Gram build)
+    # and the tables are summed over the ranks; the metrics are formed from the complete sums afterwards.
+    resid = _residual_tables(n_cand, n_splits, want_train, stat_mask)
     fit_time = np.zeros(n_cand)
     score_time = np.zeros(n_cand)
-    info = dict(n_iter=np.zeros((n_cand, n_splits), dtype=int), status=np.zeros((n_cand, n_splits), dtype=int),
-                gap=np.zeros((n_cand, n_splits)), n_pass=np.zeros((n_cand, n_splits), dtype=int))
-    need_r2 = "r2" in metrics.values()
-    sst_test = np.array([float(((yv[t] - yv[t].mean()) ** 2).sum()) if need_r2 else 0.0 for t in test_folds])
-    need_d2 = "d2_absolute_error_score" in metrics.values()
-    stat_mask = _stat_mask(metrics)
-    if sharded and (stat_mask or need_d2):
-        raise ValueError("a sharded search scores the residual sums only: statistics and d2 need one rank's residuals")
-    # statistics per (candidate, fold) (rows 2-4 of slm_cv_score_stats); the training rows of fold f are scored as
-    # one row list [0, r0_f) + [r1_f, n) of the packed design, made once per call
-    EXT = np.zeros((3, n_cand, n_splits)) if stat_mask else None
-    TEXT = np.zeros((3, n_cand, n_splits)) if stat_mask and want_train else None
+    info = _SolveInfo(n_cand, n_splits)
+    # with a statistic, the training rows of fold f are scored as one row list [0, r0_f) + [r1_f, n) of the packed
+    # design, made once per call
     train_lists = {}
-    sad_test = [_abs_dev_median(yv[t]) if need_d2 else 0.0 for t in test_folds]
-    tot_sum, tot_sq = float(yv.sum()), float((yv * yv).sum())
-    n_unconverged = 0
-    newton_stats = {}
-    iters_run = 0
 
     fds = {} if fds is None else dict(fds)  # may arrive pre-populated (prepare started early)
     if n_cand and _fold_key(ests[0], specs[0]) not in fds:
         # enqueue the GPU side of the preparation (H2D, packing, Gram build) before the host-side grouping and
         # ordering of the candidates below: that Python work then runs while the GPU is busy
-        x_dev = isinstance(X, torch.Tensor) and X.is_cuda
-        score_folds = set() if (sharded and cache is None and not x_dev) else None
         fds[_fold_key(ests[0], specs[0])] = prepare_folds(engine, X, yv, test_folds, ests[0], specs[0], cache, cache_key,
-                                                         shard, sample_weight, score_folds)
+                                                         shard, sample_weight)
     warm = _WarmStarts()  # candidate -> device view [pe] of its solution on some training fold (refit start)
-    batches = {}
-    for ci, s in enumerate(specs):
-        batches.setdefault(s.key, []).append(ci)
-    for key, idxs in batches.items():
+    for idxs in candidate_batches(specs).values():
         s0, e0 = specs[idxs[0]], ests[idxs[0]]
         fkey = _fold_key(e0, s0)
-        # batch columns in order of increasing penalty strength (dense iterates first): the
-        # row-sparse apply shares one support list per chunk of adjacent columns
-        idxs = np.asarray(sorted(idxs, key=lambda ci: (specs[ci].strength, ci)))
         K = len(idxs)
         if sharded:
             from .parallel import assign_columns
@@ -477,136 +535,76 @@ def batched_cv(engine, X, y, test_folds, ests, specs, opts, scoring, return_trai
             owner = None
             mine = [np.arange(K)] * n_splits
         if fkey not in fds:
-            # a sharded rank only needs its own slice of every fold's rows on the device (Gram build
-            # and scoring are both row-sharded) when the design comes from the host; a design that is already
-            # device-resident, or the cached one of a LineSearchCV, is kept whole
-            x_dev = isinstance(X, torch.Tensor) and X.is_cuda
-            score_folds = set() if (sharded and cache is None and not x_dev) else None
-            fds[fkey] = prepare_folds(engine, X, yv, test_folds, e0, s0, cache, cache_key, shard, sample_weight,
-                                      score_folds)
+            fds[fkey] = prepare_folds(engine, X, yv, test_folds, e0, s0, cache, cache_key, shard, sample_weight)
         fd = fds[fkey]
         t0 = time.perf_counter()
         out = solve_specs(engine, fd, [[specs[idxs[k]] for k in mine[f]] for f in range(n_splits)], **opts)
         t1 = time.perf_counter()
         warm.add(out["B"], idxs, mine)
         wtd = bool(fd.extra.get("weighted"))
-        if not sharded or fd.extra.get("partial_folds") is None:
+        if not fd.extra.get("partial_folds"):
             # every row is resident: each rank scores the columns it solved on whole folds (a sharded grid then
             # needs no exchange of coefficients; the partial tables are summed with the info tables below).
             # All (fold, row range) problems go through one batched scoring launch.
             icpt = (lambda f: out["intercept"][f]) if fd.fit_intercept else (lambda f: None)
-            items, where, titems, tfolds = [], [], [], []
+            items, where, titems, twhere = [], [], [], []
             for f in range(n_splits):
                 kf = len(mine[f])
                 if kf == 0:
                     continue
+                ci = idxs[mine[f]]
                 items.append((fd.row_ptr[f], fd.row_ptr[f + 1], out["coef"][f], kf, icpt(f)))
-                where.append((0, f))
+                where.append((0, f, ci))
                 if want_train and stat_mask:
                     if f not in train_lists:
                         train_lists[f] = engine.to_device(np.concatenate(
                             [np.arange(0, fd.row_ptr[f]), np.arange(fd.row_ptr[f + 1], n)]).astype(np.int32))
                     titems.append((train_lists[f], out["coef"][f], kf, icpt(f)))
-                    tfolds.append(f)
+                    twhere.append((1, f, ci))
                 elif want_train:
                     for r0, r1 in ((0, fd.row_ptr[f]), (fd.row_ptr[f + 1], n)):
                         if r1 > r0:
                             items.append((r0, r1, out["coef"][f], kf, icpt(f)))
-                            where.append((1, f))
-            nst = 5 if stat_mask else 2
-            sc = np.zeros((n_splits, nst, K))
-            tsc = np.zeros((n_splits, nst, K)) if want_train else None
-            if items and stat_mask:
-                res = engine.cv_score_stats(fd.Xa, p, items, rows_scaled=wtd, stats=stat_mask).cpu().numpy()
-                if titems:
-                    tres = engine.cv_score_stats(fd.Xa, p, titems, rows_scaled=wtd, stats=stat_mask).cpu().numpy()
-                    for i, f in enumerate(tfolds):
-                        tsc[f] = tres[i][:, :K]
-                for i, (kind, f) in enumerate(where):
-                    sc[f] = res[i][:, :K]
+                            where.append((1, f, ci))
+            if stat_mask:
+                for it, wh in ((items, where), (titems, twhere)):
+                    if it:
+                        res = engine.cv_score_stats(fd.Xa, p, it, rows_scaled=wtd, stats=stat_mask).cpu().numpy()
+                        for i, (kind, f, ci) in enumerate(wh):
+                            resid[kind][:, ci, f] = res[i][:, :len(ci)]
             elif items:
                 res = engine.cv_score_many(fd.Xa, p, items, rows_scaled=wtd).cpu().numpy()  # one D2H
-                for i, (kind, f) in enumerate(where):
-                    tgt = sc if kind == 0 else tsc
-                    tgt[f][:, mine[f]] += res[i][:, :len(mine[f])]
+                for i, (kind, f, ci) in enumerate(where):
+                    resid[kind][:, ci, f] += res[i][:, :len(ci)]
         else:
-            sc, tsc = _sharded_residual_sums(engine, shard, fd, out, owner, mine, p, K, n_splits, wtd, want_train)
+            _sharded_residual_sums(engine, shard, fd, out, owner, mine, idxs, resid, wtd)
         t2 = time.perf_counter()
-        for f in range(n_splits):
-            SSE[idxs, f], SAE[idxs, f] = sc[f, 0], sc[f, 1]
-            if want_train:
-                TSSE[idxs, f], TSAE[idxs, f] = tsc[f, 0], tsc[f, 1]
-            if stat_mask:
-                EXT[:, idxs, f] = sc[f, 2:]
-                if want_train:
-                    TEXT[:, idxs, f] = tsc[f, 2:]
-            kf = len(mine[f])
-            ci = idxs[mine[f]]
-            info["n_iter"][ci, f] = out["n_iter"][f, :kf]
-            info["status"][ci, f] = out["status"][f, :kf]
-            info["gap"][ci, f] = out["gap"][f, :kf]
-            info["n_pass"][ci, f] = out["n_pass"][f, :kf]
+        info.record(out, range(n_splits), [idxs[m] for m in mine])
         fit_time[idxs] = (t1 - t0) / (K * n_splits)
         score_time[idxs] = (t2 - t1) / (K * n_splits)
-        n_unconverged += int(out["n_unconverged"])
-        iters_run += int(out["iters_run"])
-        for k, v in (out.get("newton") or {}).items():  # second-order phase of this rank's batches (engine._run_batch)
-            newton_stats[k] = newton_stats.get(k, 0) + v
     if sharded:
-        # the last exchange of the sharded grid: one sum of the residual-sum and info tables
-        tabs = [SSE, SAE] + ([TSSE, TSAE] if want_train else [])
-        keys = list(info)
-        tabs += [info[k].astype(np.float64) for k in keys] + [np.array([[float(n_unconverged)]])]
-        flat = shard.allreduce_sum_numpy(np.concatenate([t.ravel() for t in tabs]), engine.device)
-        parts, o = [], 0
-        for t in tabs:
-            parts.append(flat[o:o + t.size].reshape(t.shape))
-            o += t.size
-        SSE, SAE = parts.pop(0), parts.pop(0)
-        if want_train:
-            TSSE, TSAE = parts.pop(0), parts.pop(0)
-        for k in keys:
-            info[k] = parts.pop(0).astype(info[k].dtype)
-        n_unconverged = int(round(float(parts.pop(0)[0, 0])))
-    test_tabs = {m: np.empty((n_cand, n_splits)) for m in metrics}
-    train_tabs = {m: np.empty((n_cand, n_splits)) for m in metrics} if want_train else None
-    for f in range(n_splits):
-        nt = len(test_folds[f])
-        for m, scorer in metrics.items():
-            test_tabs[m][:, f] = _metric(scorer, SSE[:, f], SAE[:, f], nt, sst_test[f], _stats_of(EXT, f, sad_test[f]))
-        if want_train:
-            ntr = n - nt
-            s_tr = tot_sum - float(yv[test_folds[f]].sum())
-            q_tr = tot_sq - float((yv[test_folds[f]] ** 2).sum())
-            sad_tr = 0.0
-            if need_d2:
-                mask = np.ones(n, dtype=bool)
-                mask[test_folds[f]] = False
-                sad_tr = _abs_dev_median(yv[mask])
-            for m, scorer in metrics.items():
-                train_tabs[m][:, f] = _metric(scorer, TSSE[:, f], TSAE[:, f], ntr, q_tr - s_tr * s_tr / ntr,
-                                              _stats_of(TEXT, f, sad_tr))
-    test_scores = test_tabs if multi else test_tabs["score"]
-    train_scores = None
-    if want_train:
-        train_scores = train_tabs if multi else train_tabs["score"]
+        resid = info.allreduce(shard, engine.device, resid)
+    test_scores, train_scores = _scores(scoring, _metric, resid, *_partition_cells(yv, test_folds, metrics, want_train))
     return dict(test_scores=test_scores, train_scores=train_scores, fit_time=fit_time, score_time=score_time,
-                info=info, fds=fds, n_unconverged=n_unconverged, iters_run=iters_run, warm=warm, newton=newton_stats)
+                info=info.tables, fds=fds, n_unconverged=info.n_unconverged, iters_run=info.iters_run, warm=warm,
+                newton=info.newton)
 
 
-def _sharded_residual_sums(engine, shard, fd, out, owner, mine, p, K, n_splits, wtd, want_train):
+def _sharded_residual_sums(engine, shard, fd, out, owner, mine, idxs, resid, wtd):
     """Row-sharded scoring of a sharded grid (north_star: "NCCL all-gather of CV scores and
     coefficients").  Every rank publishes the coefficients (+ intercepts) of the columns it solved,
     ONE all-gather makes all K x n_splits solutions resident everywhere (C3: 10 MB per rank), and each
     rank forms the residual sums of ITS slice of every fold's rows -- the slice it uploaded for the
-    Gram build, so a host-resident design crosses the bus once, 1/world per rank.  Returns this
-    rank's partial sums [n_splits, 2, K] (test rows) and the same for the training rows (or None)."""
+    Gram build, so a host-resident design crosses the bus once, 1/world per rank.  Adds this rank's
+    partial sums of the batch's candidates `idxs` into the residual tables `resid` (test rows, and the
+    training rows when resid has them)."""
     import ctypes
 
     from .parallel import gather_layout, scoring_plan
 
     torch = engine.torch
     W = shard.world
+    p, n_splits = fd.p, len(mine)
     # send layout: [p + 1][ldg], the columns this rank solved, fold after fold (only what was solved travels: C3 on
     # 8 ranks, 2.6 MB per rank)
     kfr, pad, off, ldg = gather_layout(owner, W)
@@ -627,19 +625,15 @@ def _sharded_residual_sums(engine, shard, fd, out, owner, mine, p, K, n_splits, 
         shard.all_gather_(send, recv)
     # every (fold, solving rank) group against this rank's slice of the fold's rows -- and, for train scores,
     # against its slices of the other folds -- as ONE batched scoring launch
-    plan = scoring_plan(owner, shard.fold_row_ranges(fd.row_ptr), W, want_train)
+    plan = scoring_plan(owner, shard.fold_row_ranges(fd.row_ptr), W, len(resid) > 1)
     items = []
     for lo, hi, r, f, kind, cols in plan:
         o, kf = int(off[r, f]), len(cols)
         items.append((lo, hi, recv[r, :p, o:o + int(pad[r, f])], kf, recv[r, p, o:o + kf] if fd.fit_intercept else None))
-    part = np.zeros((n_splits, 2, K))
-    tpart = np.zeros((n_splits, 2, K)) if want_train else None
     if items:
         res = engine.cv_score_many(fd.Xa, p, items, rows_scaled=wtd).cpu().numpy()  # one D2H
         for i, (lo, hi, r, f, kind, cols) in enumerate(plan):
-            tgt = part if kind == 0 else tpart
-            tgt[f][:, cols] += res[i][:, :len(cols)]
-    return part, tpart
+            resid[kind][:, idxs[cols], f] += res[i][:, :len(cols)]
 
 
 def describe_candidates(est, candidates, X, y, on_first=None):
@@ -771,26 +765,19 @@ class GridSearchCV(_SkGridSearchCV):
         if any(not set(c) <= valid for c in candidates):
             return None
         pre_fds = {}
+        cache = getattr(self, "_fd_cache", None)
+        cache_key = _cache_key(cache, Xv, yv, sw)
 
         def start_prepare(e0, s0):
             # the design of the first candidate starts its way to the device (H2D, packing,
             # Gram build are only enqueued) while the host describes the other candidates
             opts0 = est._engine_options()
             engine = get_engine(opts0.pop("device", None))
-            cache = getattr(self, "_fd_cache", None)
-            cache_key = None if cache is None else (id(Xv), id(yv), None if sw is None else sw.tobytes())
             if route == "splits":
-                cache_key = _splits_cache_key(cache, Xv, yv, sw)
                 pre_fds[_fold_key(e0, s0)] = prepare_split_data(engine, Xv, yv, splits, e0, s0, cache, cache_key, sw)
-                return
-            score_folds = None
-            if shard is not None and shard.world > 1 and cache is None:
-                # host rows this rank needs: its slice of every fold (Gram build and scoring
-                # are both row-sharded)
-                score_folds = set()
-            pre_fds[_fold_key(e0, s0)] = prepare_folds(
-                engine, Xv, yv, [np.asarray(test) for _, test in splits], e0, s0, cache,
-                cache_key, shard, sw, score_folds)
+            else:
+                pre_fds[_fold_key(e0, s0)] = prepare_folds(engine, Xv, yv, [np.asarray(test) for _, test in splits],
+                                                           e0, s0, cache, cache_key, shard, sw)
 
         try:
             ests, specs = describe_candidates(est, candidates, Xv, yv, on_first=start_prepare)
@@ -799,7 +786,7 @@ class GridSearchCV(_SkGridSearchCV):
         except Exception:
             return None  # sklearn's loop applies error_score semantics per candidate
         return dict(X=Xv, y=yv, n=n, p=p, splits=splits, candidates=candidates, ests=ests, specs=specs,
-                    fds=pre_fds, sample_weight=sw, route=route)
+                    fds=pre_fds, sample_weight=sw, route=route, cache_key=cache_key)
 
     def _fit_batched(self, plan):
         Xv, yv, n, p = plan["X"], plan["y"], plan["n"], plan["p"]
@@ -811,12 +798,8 @@ class GridSearchCV(_SkGridSearchCV):
         scoring = _device_metrics(self.scoring)
         multi = not isinstance(scoring, str)
         test_folds = [np.asarray(test) for _, test in splits]
-        cache = getattr(self, "_fd_cache", None)
+        cache, cache_key = getattr(self, "_fd_cache", None), plan["cache_key"]
         sw = plan.get("sample_weight")
-        if plan["route"] == "splits":
-            cache_key = _splits_cache_key(cache, plan["X"], plan["y"], sw)
-        else:
-            cache_key = None if cache is None else (id(plan["X"]), id(plan["y"]), None if sw is None else sw.tobytes())
         if plan["route"] == "splits":
             res = batched_cv_splits(engine, Xv, yv, splits, ests, specs, opts, scoring,
                                     return_train_score=self.return_train_score, cache=cache, cache_key=cache_key,
@@ -828,8 +811,6 @@ class GridSearchCV(_SkGridSearchCV):
         test_scores, train_scores = res["test_scores"], res["train_scores"]
         fit_time, score_time, info, fds = res["fit_time"], res["score_time"], res["info"], res["fds"]
         if res["n_unconverged"]:
-            import warnings
-
             from sklearn.exceptions import ConvergenceWarning
 
             warnings.warn(f"{res['n_unconverged']} (candidate, fold) problems did not reach the gap tolerance",

@@ -21,9 +21,9 @@ from sklearn.model_selection import ParameterGrid
 from sklearn.utils import check_random_state
 from sklearn.utils.validation import check_is_fitted, check_X_y
 
-from .engine import get_engine, split_chunks
-from .model._base import EngineRegressor, solve_specs
-from .model_selection import _fold_key, describe_candidates, prepare_split_data
+from .engine import get_engine
+from .model._base import EngineRegressor
+from .model_selection import _SolveInfo, describe_candidates, split_batches
 
 __all__ = ["StabilitySelection", "batched_selection", "draw_subsamples", "selection_summary"]
 
@@ -84,43 +84,24 @@ def batched_selection(engine, X, y, subsamples, ests, specs, opts, selection_tol
     n_sub, n_cand = len(splits), len(specs)
     counts = np.zeros((p, n_cand), dtype=np.int64)
     union = np.zeros((n_sub, p), dtype=bool)
-    info = dict(n_iter=np.zeros((n_cand, n_sub), dtype=int), status=np.zeros((n_cand, n_sub), dtype=int),
-                gap=np.zeros((n_cand, n_sub)), n_pass=np.zeros((n_cand, n_sub), dtype=int))
-    n_unconverged = 0
-    batches = {}
-    for ci, s in enumerate(specs):
-        batches.setdefault(s.key, []).append(ci)
-    chunks = split_chunks(n_sub)
+    info = _SolveInfo(n_cand, n_sub)
     slot_split = np.empty(n_sub, dtype=np.int64)  # row r of a union table holds subsample slot_split[r]
-    sds, unions, perms = {}, {}, {}
-    buf = None  # training Grams of one chunk, reused by every chunk and batch
-    for key, idxs in batches.items():
-        s0, e0 = specs[idxs[0]], ests[idxs[0]]
-        fkey = _fold_key(e0, s0)
-        if fkey not in sds:
-            sds[fkey] = prepare_split_data(engine, X, yv, splits, e0, s0, sample_weight=sample_weight)
+    unions, perms = {}, {}
+    for fkey, _, idxs, chunks in split_batches(engine, X, yv, splits, ests, specs, opts, {},
+                                               sample_weight=sample_weight):
+        s0 = specs[idxs[0]]
+        if fkey not in unions:
             # per column order: the union of one subsample is OR-ed over the batches in Xa column order
             unions[fkey] = torch.zeros((n_sub, p), dtype=torch.uint8, device=engine.device)
             perms[fkey] = s0.col_perm
-        sd = sds[fkey]
-        if buf is None:
-            buf = torch.empty((chunks[0][1] - chunks[0][0], sd.pa, sd.pa), dtype=torch.float64, device=engine.device)
-        idxs = np.asarray(sorted(idxs, key=lambda ci: (specs[ci].strength, ci)))
         K = len(idxs)
-        bspecs = [specs[ci] for ci in idxs]
         cnt = torch.zeros((p, K), dtype=torch.int32, device=engine.device)
-        for c0, c1 in chunks:
-            order, fd = engine.split_chunk(sd, c0, c1, buf)
-            out = solve_specs(engine, fd, bspecs, **opts)
+        for c0, order, _, out, _ in chunks:
+            c1 = c0 + len(order)
             # the slot order of a chunk depends on the build modes only: the same for every batch
             slot_split[c0:c1] = order
             engine.support_counts(out["coef"], K, selection_tol, cnt, unions[fkey][c0:c1])
-            for f, s in enumerate(order):
-                info["n_iter"][idxs, s] = out["n_iter"][f, :K]
-                info["status"][idxs, s] = out["status"][f, :K]
-                info["gap"][idxs, s] = out["gap"][f, :K]
-                info["n_pass"][idxs, s] = out["n_pass"][f, :K]
-            n_unconverged += int(out["n_unconverged"])
+            info.record(out, order, [idxs] * len(order))
         c = cnt.cpu().numpy()  # one D2H per batch, in Xa column order
         if s0.col_perm is not None:
             c_orig = np.empty_like(c)
@@ -134,7 +115,7 @@ def batched_selection(engine, X, y, subsamples, ests, specs, opts, selection_tol
             u_orig[:, perms[fkey]] = u
             u = u_orig
         union[slot_split] |= u
-    return dict(counts=counts, union=union, info=info, n_unconverged=n_unconverged)
+    return dict(counts=counts, union=union, info=info.tables, n_unconverged=info.n_unconverged)
 
 
 class StabilitySelection(SelectorMixin, MetaEstimatorMixin, BaseEstimator):

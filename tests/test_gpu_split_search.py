@@ -162,16 +162,20 @@ def test_line_search_with_repeated_kfold_prepares_the_splits_once(monkeypatch):
     cv = RepeatedKFold(n_splits=4, n_repeats=2, random_state=3)
     grid = [("alpha", [0.01, 0.05, 0.2]), ("l1_ratio", [0.2, 0.8])]
     est = SparseGroupLasso(groups=groups, solver_options=OPTS)
-    calls = []
-    orig = Engine.prepare_splits
+    calls = {"prepare": 0, "prepare_splits": 0}
+    for name in calls:
+        def spy(self, *a, _name=name, _orig=getattr(Engine, name), **k):
+            calls[_name] += 1
+            return _orig(self, *a, **k)
 
-    def spy(self, *a, **k):
-        calls.append(1)
-        return orig(self, *a, **k)
-
-    monkeypatch.setattr(Engine, "prepare_splits", spy)
+        monkeypatch.setattr(Engine, name, spy)
+    # a KFold partition takes the fold path: its folds are prepared once too, whatever the identity of the y view
+    # check_X_y returns at every line
+    kf = LineSearchCV(est, grid, cv=KFold(4), n_iter=3).fit(X, y)
+    assert calls == {"prepare": 1, "prepare_splits": 0}
+    assert all(h.batched_ for h in kf.history_)
     ls = LineSearchCV(est, grid, cv=cv, n_iter=3).fit(X, y)
-    assert len(calls) == 1
+    assert calls["prepare_splits"] == 1
     assert all(h.batched_ for h in ls.history_)
     # the explicit loop of 1-D searches
     best = {"alpha": 0.01, "l1_ratio": 0.2}

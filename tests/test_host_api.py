@@ -277,3 +277,162 @@ def test_warm_start_views_are_lazy_and_first_fold_wins():
     assert w.get(7) is None
     with pytest.raises(KeyError):
         w[7]
+
+
+def _solve_out(rng, F, ldz):
+    """The info part of a solve_specs output with F slots of ldz columns."""
+    return dict(n_iter=rng.integers(1, 999, (F, ldz)).astype(np.int32),
+                status=rng.integers(0, 3, (F, ldz)).astype(np.int32), gap=rng.random((F, ldz)),
+                n_pass=rng.integers(1, 9, (F, ldz)).astype(np.int32), n_unconverged=int(rng.integers(1, 5)),
+                iters_run=int(rng.integers(1, 99)), newton={"steps": F})
+
+
+def test_candidate_batches_and_solve_info_of_sharded_folds_and_split_chunks():
+    from types import SimpleNamespace
+
+    from sparselm_b200.model_selection import _SolveInfo, candidate_batches
+    from sparselm_b200.parallel import assign_columns
+
+    specs = [SimpleNamespace(key=k, strength=s) for k, s in (("a", 0.3), ("a", 0.1), ("b", 0.2), ("a", 0.1))]
+    batches = candidate_batches(specs)
+    assert list(batches) == ["a", "b"] and batches["a"].tolist() == [1, 3, 0] and batches["b"].tolist() == [2]
+
+    rng = np.random.default_rng(0)
+    F, n_cand = 5, 9
+    idxs = np.array([4, 0, 7, 2, 8, 1, 3, 6, 5])  # batch column k -> candidate
+    full = _solve_out(rng, F, 16)  # one process solving every (fold, column)
+    ref = _SolveInfo(n_cand, F)
+    ref.record(full, range(F), [idxs] * F)
+    for k, t in ref.tables.items():
+        np.testing.assert_array_equal(t[idxs].T, full[k][:, :n_cand])
+    # a sharded grid: rank r solved the columns mine[f] of fold f, packed at the front of its slot
+    owner = assign_columns(F, n_cand, 2)
+    ranks = []
+    for r in range(2):
+        mine = [np.flatnonzero(owner[f] == r) for f in range(F)]
+        out = dict(full, iters_run=10 + r)
+        for k in ref.tables:
+            out[k] = np.zeros_like(full[k])
+            for f in range(F):
+                out[k][f, :len(mine[f])] = full[k][f, mine[f]]
+        ranks.append(_SolveInfo(n_cand, F))
+        ranks[-1].record(out, range(F), [idxs[m] for m in mine])
+
+    class _TwoRanks:
+        """All-reduce of two ranks: adds the other rank's buffer to this one's (and keeps this one's)."""
+        world = 2
+
+        def __init__(self, other=None):
+            self.other = other
+
+        def allreduce_sum_numpy(self, arr, device=None):
+            self.sent = arr.copy()
+            return arr if self.other is None else arr + self.other
+
+    resid = [rng.random((2, 2, n_cand, F)) for _ in range(2)]
+    first = _TwoRanks()
+    ranks[1].allreduce(first, None, resid[1])
+    got = ranks[0].allreduce(_TwoRanks(first.sent), None, resid[0])
+    np.testing.assert_array_equal(got, resid[0] + resid[1])
+    for k, t in ref.tables.items():
+        assert ranks[0].tables[k].dtype == t.dtype
+        np.testing.assert_array_equal(ranks[0].tables[k], t)
+    assert ranks[0].n_unconverged == 2 * full["n_unconverged"]
+    assert ranks[0].iters_run == 10 and ranks[0].newton == {"steps": F}  # not exchanged
+
+    # chunks of arbitrary splits: slot f holds split order[f] (direct builds first), every slot solves the batch
+    info = _SolveInfo(n_cand, 20)
+    outs = []
+    for c0, c1 in ((0, 16), (16, 20)):
+        order = c0 + rng.permutation(c1 - c0)
+        outs.append((order, _solve_out(rng, c1 - c0, 16)))
+        info.record(outs[-1][1], order, [idxs] * len(order))
+    for order, out in outs:
+        for k, t in info.tables.items():
+            np.testing.assert_array_equal(t[idxs][:, order].T, out[k][:, :n_cand])
+    assert info.n_unconverged == sum(o["n_unconverged"] for _, o in outs)
+    assert info.iters_run == sum(o["iters_run"] for _, o in outs) and info.newton == {"steps": 20}
+
+
+def _residual_rows(r, y):
+    """The [5][K] rows of slm_cv_score_stats for the residuals r [rows, K] of the targets y."""
+    a = np.abs(r)
+    return np.stack([(r * r).sum(0), a.sum(0), a.max(0), (a / np.maximum(np.abs(y), np.finfo(float).eps)[:, None]).sum(0),
+                     np.median(a, axis=0)])
+
+
+def test_score_assembly_on_a_partition_and_on_splits():
+    from sklearn.exceptions import UndefinedMetricWarning
+    from sklearn.metrics import (d2_absolute_error_score, mean_absolute_error, mean_absolute_percentage_error,
+                                 median_absolute_error, r2_score, root_mean_squared_error)
+
+    from sparselm_b200.model_selection import (_metric, _partition_cells, _residual_tables, _scores, _split_cells,
+                                               _split_metric, _stat_mask)
+
+    sk = {"r2": r2_score, "rmse": lambda a, b: -root_mean_squared_error(a, b),
+          "mae": lambda a, b: -mean_absolute_error(a, b), "med": lambda a, b: -median_absolute_error(a, b),
+          "mape": lambda a, b: -mean_absolute_percentage_error(a, b), "d2": d2_absolute_error_score}
+    scoring = {"r2": "r2", "rmse": "neg_root_mean_squared_error", "mae": "neg_mean_absolute_error",
+               "med": "neg_median_absolute_error", "mape": "neg_mean_absolute_percentage_error",
+               "d2": "d2_absolute_error_score"}
+    rng = np.random.default_rng(1)
+    n, K = 23, 3
+    y = rng.standard_normal(n)
+    allrows = np.arange(n)
+
+    def check(scores, cells, rows_of, preds):
+        for c, rows in enumerate(rows_of):
+            for m, fn in sk.items():
+                if len(rows) < 2 and m in ("r2", "d2"):
+                    continue
+                want = [fn(y[rows], preds[c][rows, k]) for k in range(K)]
+                np.testing.assert_allclose(scores[m][:, c], want, rtol=1e-10, err_msg=f"{m} cell {c}")
+
+    # a partition in row order with a one-row fold: train sums as the pieces [0, r0) + [r1, n)
+    folds = [np.arange(0, 1), np.arange(1, 12), np.arange(12, n)]
+    preds = [y[:, None] + rng.standard_normal((n, K)) for _ in folds]
+    resid = _residual_tables(K, len(folds), True, _stat_mask(scoring))
+    trains = [np.setdiff1d(allrows, te) for te in folds]
+    for f, (te, tr) in enumerate(zip(folds, trains)):
+        r = y[:, None] - preds[f]
+        resid[0][:, :, f] = _residual_rows(r[te], y[te])
+        for lo, hi in ((0, te[0]), (te[-1] + 1, n)):
+            if hi > lo:
+                resid[1][:2, :, f] += _residual_rows(r[lo:hi], y[lo:hi])[:2]
+        resid[1][2:, :, f] = _residual_rows(r[tr], y[tr])[2:]
+    cells = _partition_cells(y, folds, scoring, True)
+    for (n_tr, sst, _), te, tr in zip(cells[1], folds, trains):
+        # the training sst is downdated from the sums over all rows
+        s_tr, q_tr = float(y.sum()) - float(y[te].sum()), float((y * y).sum()) - float((y[te] ** 2).sum())
+        assert n_tr == len(tr) and sst == q_tr - s_tr * s_tr / n_tr
+        assert sst == pytest.approx(((y[tr] - y[tr].mean()) ** 2).sum(), rel=1e-12)
+    with pytest.warns(UndefinedMetricWarning):  # d2 of the one-row fold
+        test, train = _scores(scoring, _metric, resid, *cells)
+    assert set(test) == set(train) == set(scoring)
+    check(test, cells[0], folds, preds)
+    check(train, cells[1], trains, preds)
+    r0 = y[0] - preds[0][0]
+    np.testing.assert_array_equal(test["r2"][:, 0], np.where(r0 == 0.0, 1.0, 0.0))  # force-finite r2 on one row
+    assert np.isnan(test["d2"][:, 0]).all()
+    # one metric: its table itself; no train cells, no train scores
+    one, none = _scores("neg_mean_absolute_error", _metric, resid[:1, :2], cells[0])
+    np.testing.assert_array_equal(one, test["mae"])
+    assert none is None
+
+    # arbitrary splits: a one-row test set, rows in neither set; the downdated train sums are all rows - out rows
+    splits = [(np.arange(1, n), np.array([0])), (np.arange(0, 8), np.arange(15, n)), (np.arange(8, 20), np.arange(5))]
+    preds = [y[:, None] + rng.standard_normal((n, K)) for _ in splits]
+    resid = _residual_tables(K, len(splits), True, _stat_mask(scoring))
+    for s, (tr, te) in enumerate(splits):
+        r = y[:, None] - preds[s]
+        out = np.setdiff1d(allrows, tr)
+        resid[0][:, :, s] = _residual_rows(r[te], y[te])
+        resid[1][:2, :, s] += -1.0 * _residual_rows(r[out], y[out])[:2]
+        resid[1][:2, :, s] += _residual_rows(r, y)[:2]
+        resid[1][2:, :, s] = _residual_rows(r[tr], y[tr])[2:]
+    cells = _split_cells(y, splits, scoring, True)
+    with pytest.warns(UndefinedMetricWarning):  # r2 and d2 of the one-row test set
+        test, train = _scores(scoring, _split_metric, resid, *cells)
+    check(test, cells[0], [te for _, te in splits], preds)
+    check(train, cells[1], [tr for tr, _ in splits], preds)
+    assert np.isnan(test["r2"][:, 0]).all() and np.isnan(test["d2"][:, 0]).all()
