@@ -41,14 +41,12 @@ int slm_version(void);
 int slm_create(int device, slm_ctx** out);
 void slm_destroy(slm_ctx* ctx);
 /* engine switches (the SLM_* environment variables read at slm_create, settable later):
- * "coop" (cooperative few-column iterations), "small_fused" (fused small-design iterations),
- * "dense_apply" (solver uses the dense Gram apply), "chunk_w" (columns per support chunk),
+ * "coop" (cooperative few-column iterations),
  * "tma" (bit mask of the kernel families fed by TMA + mbarrier instead of cp.async: 1 Gram build,
  * 2 dense Gram apply, 4 row-sparse Gram apply, 8 / 16 wide padded-pitch bands instead of 128-byte
  * swizzled boxes for the gather / tiled kernels; default 15), "fused_prox" (default 1: one prox_fused_kernel per
  * iteration on the iterate buffers, the Gram applied to the iterate itself; 0: the two-kernel iteration on a
- * materialised extrapolated point), "prox2" (one-lane-per-column prox kernels of the two-kernel iteration,
- * default 0: measured slower than the 8-columns-per-row mapping), "force_apply_shape" / "force_sparse_shape" /
+ * materialised extrapolated point), "force_apply_shape" / "force_sparse_shape" /
  * "force_syrk_shape" (tile menu overrides of tools/gemm_probe.py, -1 = automatic). */
 int slm_set_option(slm_ctx* ctx, const char* name, int value);
 const char* slm_last_error(const slm_ctx* ctx);

@@ -76,20 +76,16 @@ struct slm_ctx {
     size_t colmax_cap = 0;
     double apply_exec_flops = 0.0;   // flops the row-sparse applies executed (useful, unpadded)
     double apply_dense_flops = 0.0;  // 2 p^2 K_active of the same applies
-    int chunk_w = 32;                // columns per support chunk (SLM_CHUNK_W)
-    bool dense_apply = false;        // SLM_DENSE_APPLY=1: solver uses the dense apply (A/B runs)
-    bool small_fused = true;         // SLM_SMALL_FUSED=0: never use the fused small-design iterations
     bool coop = true;                // SLM_COOP=0: never use the cooperative few-column iterations
     bool trace = false;              // SLM_TRACE=1: one stderr line per convergence check
     int coop_max_smem = 0;           // opt-in shared memory per block of the device
-    int max_cluster = 16;            // largest cluster size the cooperative cluster kernel may use
+    int max_cluster = 16;            // largest cluster of the cluster kernel (8 where non-portable sizes are refused)
     int force_sparse_shape = -1;     // SLM_FORCE_SPARSE_SHAPE
     int force_apply_shape = -1;  // tuning/testing hook (SLM_FORCE_APPLY_SHAPE)
     int force_syrk_shape = -1;   // tuning/testing hook (SLM_FORCE_SYRK_SHAPE)
     // TMA-fed GEMM kernels (gemm_f64_tma.cuh): bit 0 Gram build, bit 1 dense apply, bit 2 row-sparse
     // apply (SLM_TMA / slm_set_option "tma"); encode = cuTensorMapEncodeTiled resolved at run time
     bool fused_prox = true;          // SLM_FUSED_PROX=0: the two-kernel iteration (prox_main + prox_momentum on the extrapolated point)
-    bool prox2 = false;              // SLM_PROX2=1: one-lane-per-column prox kernels (measured slower: 3.34 vs 2.60 ms per C3 step)
     int tma_mask = 7 + 8;  // + bit 3: wide bands for the gather kernels, bit 4: for the tiled kernels
     void* encode = nullptr;
 };
@@ -1117,13 +1113,9 @@ int slm_create(int device, slm_ctx** out) {
     if (const char* e = getenv("SLM_FORCE_APPLY_SHAPE")) ctx->force_apply_shape = atoi(e);
     if (const char* e = getenv("SLM_FORCE_SYRK_SHAPE")) ctx->force_syrk_shape = atoi(e);
     if (const char* e = getenv("SLM_FORCE_SPARSE_SHAPE")) ctx->force_sparse_shape = atoi(e);
-    if (const char* e = getenv("SLM_CHUNK_W")) ctx->chunk_w = std::max(8, atoi(e) / 8 * 8);
-    if (const char* e = getenv("SLM_DENSE_APPLY")) ctx->dense_apply = atoi(e) != 0;
-    if (const char* e = getenv("SLM_SMALL_FUSED")) ctx->small_fused = atoi(e) != 0;
     if (const char* e = getenv("SLM_COOP")) ctx->coop = atoi(e) != 0;
     if (const char* e = getenv("SLM_TRACE")) ctx->trace = atoi(e) != 0;
     if (const char* e = getenv("SLM_TMA")) ctx->tma_mask = atoi(e);
-    if (const char* e = getenv("SLM_PROX2")) ctx->prox2 = atoi(e) != 0;
     if (const char* e = getenv("SLM_FUSED_PROX")) ctx->fused_prox = atoi(e) != 0;
     {
         void* fn = nullptr;
@@ -1136,15 +1128,12 @@ int slm_create(int device, slm_ctx** out) {
     }
     ctx->coop_max_smem = (int)prop.sharedMemPerBlockOptin;
     if (!prop.cooperativeLaunch) ctx->coop = false;
-    if (const char* e = getenv("SLM_MAX_CLUSTER")) ctx->max_cluster = std::max(1, std::min(16, atoi(e)));
-    if (ctx->max_cluster > 8) {
-        if (cudaFuncSetAttribute(fista_coop_kernel<true, true>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) !=
-                cudaSuccess ||
-            cudaFuncSetAttribute(fista_coop_kernel<false, true>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) !=
-                cudaSuccess) {
-            cudaGetLastError();
-            ctx->max_cluster = 8;
-        }
+    if (cudaFuncSetAttribute(fista_coop_kernel<true, true>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) !=
+            cudaSuccess ||
+        cudaFuncSetAttribute(fista_coop_kernel<false, true>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) !=
+            cudaSuccess) {
+        cudaGetLastError();
+        ctx->max_cluster = 8;
     }
     ctx->n_flags_cap = 1 << 20;
     if (cudaMalloc(&ctx->d_flags, sizeof(int) * (size_t)ctx->n_flags_cap) != cudaSuccess ||
@@ -1188,16 +1177,8 @@ int slm_set_option(slm_ctx* ctx, const char* name, int value) {
     const std::string nm(name);
     if (nm == "coop")
         ctx->coop = value != 0;
-    else if (nm == "small_fused")
-        ctx->small_fused = value != 0;
-    else if (nm == "dense_apply")
-        ctx->dense_apply = value != 0;
-    else if (nm == "chunk_w")
-        ctx->chunk_w = std::max(8, value / 8 * 8);
     else if (nm == "tma")
         ctx->tma_mask = value;
-    else if (nm == "prox2")
-        ctx->prox2 = value != 0;
     else if (nm == "fused_prox")
         ctx->fused_prox = value != 0;
     else if (nm == "force_apply_shape")
@@ -1597,282 +1578,288 @@ int slm_lipschitz_dev(slm_ctx* ctx, const double* G, int64_t g_stride, int64_t p
     return 0;
 }
 
-// support-chunk geometry of a solve: chunks of w columns, ncc chunk slots per fold
-static void chunk_geometry(const slm_ctx* ctx, int64_t ldz, int* w, int* ncc) {
-    int cw = ctx ? ctx->chunk_w : 32;
-    cw = std::max(8, cw / 8 * 8);
-    *w = cw;
-    *ncc = (int)((ldz + cw - 1) / cw);
+// ---- batched solve (slm_solve_batch) -------------------------------------------------------------
+constexpr int kChunkW = 32;  // columns per support chunk of the row-sparse apply (its narrow form)
+
+// byte offsets into the solve workspace: slm_solve_workspace sizes it, slm_solve_batch carves it up
+struct SolveLayout {
+    size_t Z, GZ, GB, T, Bw;         // [F][p][ldz] doubles each
+    size_t theta, tmom, rst, part;   // doubles: [2][F][ldz], [2][F][ldz], [F][ldz], [F][kMaxChunks][NQ][ldz]
+    size_t flag, colmap, src, newK;  // ints: [F][ldz] each, newK 64
+    size_t sidx, scount;             // support lists [F][ncc][p] and their lengths [F][ncc] (ncc chunks of kChunkW)
+    size_t zflag;                    // [F][p][ldz / 8] bytes
+    size_t bytes;
+};
+
+static SolveLayout solve_layout(int64_t p, int64_t ldz, int F) {
+    const size_t state = (size_t)F * p * ldz * sizeof(double), cols = (size_t)F * ldz;
+    const size_t nblk = (size_t)ldz / 8, ncc = (size_t)((ldz + kChunkW - 1) / kChunkW);
+    SolveLayout L;
+    L.Z = 0;
+    L.GZ = L.Z + state;
+    L.GB = L.GZ + state;
+    L.T = L.GB + state;
+    L.Bw = L.T + state;
+    L.theta = L.Bw + state;
+    L.tmom = L.theta + 2 * cols * sizeof(double);
+    L.rst = L.tmom + 2 * cols * sizeof(double);
+    L.part = L.rst + cols * sizeof(double);
+    L.flag = L.part + cols * kMaxChunks * NQ * sizeof(double);
+    L.colmap = L.flag + cols * sizeof(int);
+    L.src = L.colmap + cols * sizeof(int);
+    L.newK = L.src + cols * sizeof(int);
+    L.sidx = L.newK + 64 * sizeof(int);
+    L.scount = L.sidx + (size_t)F * ncc * p * sizeof(int);
+    L.zflag = L.sidx + (size_t)F * nblk * (p + 1) * sizeof(int);  // room for the lists of 8-column chunks
+    L.bytes = L.zflag + round_up((int64_t)((size_t)F * p * nblk), 16) + 64 + 256;  // + 320 bytes of slack
+    return L;
 }
 
-size_t slm_solve_workspace(int64_t p, int64_t ldz, int n_folds, int n_groups) {
-    (void)n_groups;
-    size_t state = (size_t)n_folds * (size_t)p * (size_t)ldz * sizeof(double);
-    size_t cols = (size_t)n_folds * (size_t)ldz;
-    size_t part = cols * (size_t)kMaxChunks * NQ * sizeof(double);
-    // row-sparse apply: support lists for the finest chunking (8 columns) + flag bytes
-    size_t nblk = (size_t)ldz / 8;
-    size_t lists = (size_t)n_folds * nblk * ((size_t)p + 1) * sizeof(int);
-    size_t zflag = round_up((int64_t)((size_t)n_folds * (size_t)p * nblk), 16);
-    return 5 * state + cols * (5 * sizeof(double) + 3 * sizeof(int)) + part + 64 * sizeof(int) + 256 + lists +
-           zflag + 64;
+size_t slm_solve_workspace(int64_t p, int64_t ldz, int n_folds, int /*n_groups*/) {
+    return solve_layout(p, ldz, n_folds).bytes;
 }
 
-int slm_solve_batch(slm_ctx* ctx, slm_batch* bt, void* stream) {
-    if (!ctx || !bt) return fail(ctx, 1, "slm_solve_batch: null argument");
-    if (bt->n_folds < 1 || bt->n_folds > SLM_MAX_FOLDS) return fail(ctx, 1, "slm_solve_batch: n_folds out of range");
-    if (bt->ldz % 8) return fail(ctx, 1, "slm_solve_batch: ldz must be a multiple of 8");
-    if (!bt->G_dev || !bt->B_dev || !bt->work_dev) return fail(ctx, 1, "slm_solve_batch: null device pointer");
+// One slm_solve_batch call.  An iteration is a stretch (small, coop and cluster modes: every iteration up to the
+// next check in one launch) or apply, check (when scheduled), prox, compact (after a check that retired columns)
+// and the hand-over to the cluster kernels.  finish scatters the coefficients and certifies them.
+struct BatchSolve {
+    slm_ctx* const ctx;
+    slm_batch* const bt;
+    const cudaStream_t s;
     const int F = bt->n_folds;
     const int64_t p = bt->p, ldz = bt->ldz;
-    if (bt->work_bytes < slm_solve_workspace(p, ldz, F, bt->n_groups))
-        return fail(ctx, 1, "slm_solve_batch: workspace too small");
-    const int Gn = bt->gptr_dev ? bt->n_groups : (int)p;
-    cudaStream_t s = (cudaStream_t)stream;
-
-    const size_t state = (size_t)F * p * ldz;
-    const size_t cols = (size_t)F * ldz;
-    double* Z = (double*)bt->work_dev;
-    double* GZ = Z + state;
-    double* GB = GZ + state;
-    double* T = GB + state;
-    double* Bw = T + state;
-    double* theta = Bw + state;       // [2][cols]
-    double* tmom = theta + 2 * cols;  // [2][cols]
-    double* rst = tmom + 2 * cols;    // [cols]
-    double* part = rst + cols;        // [F][n_chunks][NQ][ldz]
-    int* flag = (int*)(part + cols * (size_t)kMaxChunks * NQ);
-    int* colmap = flag + cols;
-    int* src = colmap + cols;
-    int* newK = src + cols;  // [F] (64 ints reserved)
-    int cw, ncc;
-    chunk_geometry(ctx, ldz, &cw, &ncc);
-    int* sidx = newK + 64;                  // [F][ncc][p]
-    int* scount = sidx + (size_t)F * ncc * p;  // [F][ncc]
-    unsigned char* zflag = (unsigned char*)(newK + 64 + (size_t)F * (ldz / 8) * (p + 1));
-    // small designs: the iterations between two convergence checks run inside one kernel
-    // (fista_small_kernel, Gram in shared memory); the checks use the regular dense path
-    const bool small = ctx->small_fused && p <= kSmallPMax;
-    const bool sparse = !ctx->dense_apply && !small;
-    // few columns on a large design: the whole GPU iterates on them inside one cooperative
-    // launch between two convergence checks (coop_kernels.cuh)
-    bool coop = false;
-    CoopArgs ca;
-    memset(&ca, 0, sizeof(ca));
-    int coop_nb = 0;
-    size_t coop_sm = 0;
-
-    SolveDev sp;
-    memset(&sp, 0, sizeof(sp));
-    sp.F = F;
-    sp.p = (int)p;
-    sp.Gn = Gn;
-    sp.ldz = ldz;
-    sp.pa = bt->pa;
-    sp.g_stride = bt->g_stride;
-    sp.G = bt->G_dev;
-    sp.gptr = bt->gptr_dev;
-    sp.lam1 = bt->lam1_dev;
-    sp.W1 = bt->W1_dev;
-    sp.W2 = bt->W2_dev;
-    sp.D2 = bt->D2_dev;
-    sp.B = Bw;
-    sp.Bout = bt->B_dev;
-    sp.colmap = colmap;
-    sp.skip = bt->skip_dev;
-    sp.Z = Z;
-    sp.GZ = GZ;
-    sp.GB = GB;
-    sp.T = T;
-    sp.theta[0] = theta;
-    sp.theta[1] = theta + cols;
-    sp.tmom[0] = tmom;
-    sp.tmom[1] = tmom + cols;
-    sp.part = part;
-    sp.rst = rst;
-    sp.flag = flag;
+    const size_t state = (size_t)F * p * ldz;  // elements of one [F][p][ldz] array
     const bool grouped = bt->gptr_dev != nullptr;
-    const int gpb = grouped ? GPB : SG;  // groups per block iteration
-    sp.gpt = std::max(1, (Gn + gpb * kMaxChunks - 1) / (gpb * kMaxChunks));
-    sp.n_chunks = (Gn + gpb * sp.gpt - 1) / (gpb * sp.gpt);
-    sp.gap = bt->gap_dev;
-    sp.primal = bt->primal_dev;
-    sp.n_iter = bt->n_iter_dev;
-    sp.status = bt->status_dev;
-    sp.counter = ctx->d_counter;
-    sp.ratio = ctx->d_ratio;
-    sp.zflag = sparse ? zflag : nullptr;
-    sp.nblk = (int)(ldz / SC);
-    sp.tol = bt->tol;
-    sp.floor_rel = bt->floor_rel;
-    sp.lips_dev = bt->lipschitz_dev;
-    int Kcur[SLM_MAX_FOLDS];
-    int Kmax0 = 0;
-    long long Ktot = 0;
-    for (int f = 0; f < F; ++f) {
-        if (bt->K[f] < 0 || bt->K[f] > ldz) return fail(ctx, 1, "slm_solve_batch: K[f] out of range");
-        if (bt->K[f] > 0 && ((!bt->lipschitz_dev && !(bt->lipschitz[f] > 0.0)) || !(bt->n_obs[f] > 0.0)))
-            return fail(ctx, 1, "slm_solve_batch: lipschitz and n_obs must be positive");
-        sp.K[f] = Kcur[f] = bt->K[f];
-        sp.n_obs[f] = bt->n_obs[f] > 0.0 ? bt->n_obs[f] : 1.0;
-        sp.step[f] = bt->lipschitz[f] > 0.0 ? 1.0 / bt->lipschitz[f] : 0.0;
-        Kmax0 = std::max(Kmax0, bt->K[f]);
-        Ktot += bt->K[f];
-    }
-    bt->iters_run = 0;
-    bt->n_unconverged = 0;
-    if (Kmax0 == 0) return 0;
-    if (!small && ctx->coop && Ktot <= kCoopMaxProb) {
-        const int nprob = (int)Ktot;
-        const int maxg = bt->gptr_dev ? bt->max_group : 1;  // 0: the caller did not say
-        coop_nb = (int)std::min<int64_t>(ctx->sm_count / nprob, std::max<int64_t>(1, p / 16));
-        coop_sm = coop_smem((int)p);
-        if (maxg > 0 && coop_nb >= 1 && (p + coop_nb - 1) / coop_nb + maxg <= CO_ROWS &&
-            coop_sm <= (size_t)ctx->coop_max_smem) {
-            coop = true;
-            ca.nprob = nprob;
-            ca.seg = coop_seg((int)p);
-            ca.buf[0] = T;
-            ca.buf[1] = T + (size_t)nprob * p;
-            ca.buf[2] = GZ;
-            ca.dpart = part;
-            int q = 0;
-            for (int f = 0; f < F; ++f)
-                for (int k = 0; k < bt->K[f]; ++k, ++q) {
-                    ca.pf[q] = f;
-                    ca.pk[q] = k;
-                }
-            CUDA_OK(cudaFuncSetAttribute(fista_coop_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)coop_sm));
-            CUDA_OK(cudaFuncSetAttribute(fista_coop_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)coop_sm));
-        }
-    }
-
-    // cluster mode: when few columns are left (or given), one thread-block cluster per column
-    // iterates on it between two checks; columns are independent, so any number of clusters
-    bool clus = false;
-    int clus_cs_min = 0, clus_thr = 0;
-    if (!small && !coop && ctx->coop && p <= 16 * CO_ROWS) {
-        const int maxg = bt->gptr_dev ? bt->max_group : 1;
-        const size_t sm = coop_smem((int)p);
-        if (maxg > 0 && sm <= (size_t)ctx->coop_max_smem) {
-            for (int cs = 1; cs <= ctx->max_cluster; cs *= 2)
-                if ((p + cs - 1) / cs + maxg <= CO_ROWS) {
-                    clus_cs_min = cs;
-                    break;
-                }
-            if (clus_cs_min > 0) {
-                // three rounds of co-resident clusters at most, and the three beta buffers of
-                // every column must fit in the T / GZ scratch arrays
-                clus_thr = (int)std::min<long long>(3LL * (ctx->sm_count / clus_cs_min), (long long)F * ldz / 2);
-                coop_sm = sm;
-                ca.seg = coop_seg((int)p);
-                CUDA_OK(cudaFuncSetAttribute(fista_coop_kernel<true, true>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coop_sm));
-                CUDA_OK(cudaFuncSetAttribute(fista_coop_kernel<false, true>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coop_sm));
-            }
-        }
-    }
-
-    init_cols_kernel<<<(unsigned)((cols + 255) / 256), 256, 0, s>>>(theta, tmom, flag, colmap, sp.status, sp.n_iter,
-                                                                    bt->skip_dev, (long long)cols, (int)ldz);
-    LAUNCH_OK("init_cols_kernel");
-    CUDA_OK(cudaMemcpyAsync(Bw, bt->B_dev, state * sizeof(double), cudaMemcpyDeviceToDevice, s));
-    CUDA_OK(cudaMemcpyAsync(Z, bt->B_dev, state * sizeof(double), cudaMemcpyDeviceToDevice, s));
-    CUDA_OK(cudaMemsetAsync(GB, 0, state * sizeof(double), s));
-    // fused iteration (solver_kernels.cuh, prox_fused_kernel): the iterates W_t / W_{t-1} alternate between Bw and
-    // T, their Gram products between GZ and GB; Z is scratch.  One-way switch to the two-kernel state when the
-    // cluster kernels take over the tail.
-    bool fused = ctx->fused_prox && !small && !coop;
-    double* Bc[2] = {Bw, T};
-    double* GBc[2] = {GZ, GB};
-    int use_rst = 0;
-    if (fused) CUDA_OK(cudaMemcpyAsync(T, bt->B_dev, state * sizeof(double), cudaMemcpyDeviceToDevice, s));
-    const dim3 zgrid((unsigned)(((long long)p * sp.nblk + 255) / 256), (unsigned)F);
-    if (sparse) {
-        CUDA_OK(cudaMemsetAsync(ctx->d_stat, 0, sizeof(unsigned long long), s));
-        zflags_kernel<<<zgrid, 256, 0, s>>>(sp, Z);
-        LAUNCH_OK("zflags_kernel");
-    }
-
-    auto grids = [&](int Kmax, dim3& cgrid, dim3& mgrid, dim3& fgrid) {
-        cgrid = dim3((unsigned)((Kmax + SC - 1) / SC), (unsigned)sp.n_chunks, (unsigned)F);
-        mgrid = dim3((unsigned)((Kmax + SC - 1) / SC), (unsigned)((p + MOM_ROWS - 1) / MOM_ROWS), (unsigned)F);
-        fgrid = dim3((unsigned)((Kmax + 127) / 128), (unsigned)F);
-    };
-    dim3 cgrid, mgrid, fgrid;
-    int Kmax = Kmax0;
-    grids(Kmax, cgrid, mgrid, fgrid);
+    // small designs: the iterations between two convergence checks run inside one kernel (fista_small_kernel,
+    // Gram in shared memory) and the checks use the dense apply; larger designs use the row-sparse apply
+    const bool small = p <= kSmallPMax, sparse = !small;
+    const int ncc = (int)((ldz + kChunkW - 1) / kChunkW);  // support chunks of kChunkW columns per fold
     const int check_every = std::max(1, bt->check_every);
-    long long n_active = Ktot;
+    const int cw_wide = (int)std::min<int64_t>(ldz, 128);  // columns per chunk of the wide row-sparse apply
+    int *colmap = nullptr, *src = nullptr, *newK = nullptr, *sidx = nullptr, *scount = nullptr;
+    SolveDev sp = {};  // the arrays Z, GZ, GB, T, B (Bw), part of the workspace; K: current column counts
     int n_active_f[SLM_MAX_FOLDS] = {0};
-    bool do_compact = false;
-    // chunk width of the row-sparse apply: narrow chunks (cw) pay when the supports of the
-    // column chunks differ, one wide chunk per fold when they are all (nearly) dense -- the
-    // narrow form then re-reads G once per chunk.  Decided at every convergence check from
-    // the list lengths of that iteration (which always runs narrow).
-    const int cw_wide = (int)std::min<int64_t>(ldz, 128);
-    const bool can_adapt = sparse && cw < cw_wide && F * ncc <= kMaxScount;
-    bool wide = false;
+    int Kmax0 = 0, Kmax = 0;
+    long long Ktot = 0, n_active = 0;
+    dim3 cgrid, mgrid, fgrid, zgrid;
+    // coop: few columns on a large design, the whole GPU iterates on them inside one cooperative launch between
+    // two checks.  clus: when few columns are left (or given), one thread-block cluster per column; columns are
+    // independent, so any number of clusters (coop_kernels.cuh)
+    bool coop = false, clus = false;
+    CoopArgs ca = {};
+    int coop_nb = 0, clus_cs_min = 0, clus_thr = 0;
+    size_t coop_sm = 0;
+    int p32 = 0, nsplit = 0;  // fista_small_kernel geometry
+    size_t small_smem = 0;
+    // fused iteration (solver_kernels.cuh, prox_fused_kernel): the iterates W_t / W_{t-1} alternate between Bw
+    // and T, their Gram products between GZ and GB; Z is scratch.  One-way switch to the two-kernel state when
+    // the cluster kernels take over the tail
+    bool fused = false;
+    double *Bc[2] = {}, *GBc[2] = {};
+    int use_rst = 0;
     int it = 0;
-    // chunk-width decision from the support-list lengths of a narrow iteration (host copy in
-    // ctx->h_scount): time of the narrow form (per-chunk supports, G re-read per chunk) against
-    // one wide chunk per fold contracting over the largest support
-    auto decide_width = [&]() {
-        double fw = 0.0, fn = 0.0, bw = 0.0, bn = 0.0;  // flops / G bytes, wide and narrow
-        for (int f = 0; f < F; ++f) {
-            const int Kp = (int)std::min<int64_t>(round_up(Kcur[f], 8), ldz);
-            int smax = 0;
-            for (int cc = 0; cc * cw < Kp; ++cc) {
-                const int sc = ctx->h_scount[f * ncc + cc];
-                smax = std::max(smax, sc);
-                fn += 2.0 * (double)p * sc * std::min(cw, Kp - cc * cw);
-                bn += 8.0 * (double)p * sc;
-            }
-            fw += 2.0 * (double)p * smax * std::min(Kp, cw_wide) * ((Kp + cw_wide - 1) / cw_wide);
-            bw += 8.0 * (double)p * smax * ((Kp + cw_wide - 1) / cw_wide);
-        }
-        const double tn = std::max(fn / (0.84 * 35e12), bn / 6.0e12);
-        const double tw = std::max(fw / (0.776 * 35e12), bw / 6.0e12);
-        wide = (fn == 0.0) || (tw < tn);
-    };
-    int next_check = 0, interval = check_every;  // small mode: checks get rarer while nothing converges
+    // stretching modes: checks get rarer while nothing converges
+    int next_check = 0, prev_check = 0, interval = check_every;
     double prev_ratio = 0.0;
-    int prev_check = 0;
     int next_regular = 0;  // next check of the per-iteration kernels: every check_every iterations, twice
                            // as often once an eighth of the columns is left (the tail iterates at the
                            // latency floor of the launch set, a check costs about one iteration)
-    const int p32 = (int)round_up(p, 32);
-    const int nsplit = std::max(1, std::min(8, 256 / p32));
-    const size_t small_smem = fista_small_smem((int)p, p32, nsplit);
-    if (small) {
-        CUDA_OK(cudaFuncSetAttribute(fista_small_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)small_smem));
-        CUDA_OK(cudaFuncSetAttribute(fista_small_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)small_smem));
+    bool do_compact = false;
+    // chunk width of the row-sparse apply: narrow chunks (kChunkW) pay when the supports of the column chunks
+    // differ, one wide chunk per fold when they are all (nearly) dense -- the narrow form then re-reads G once
+    // per chunk.  Decided at every convergence check from the list lengths of that iteration (which always runs
+    // narrow)
+    const bool can_adapt = sparse && kChunkW < cw_wide && F * ncc <= kMaxScount;
+    bool wide = false;
+
+    BatchSolve(slm_ctx* c, slm_batch* b, cudaStream_t st) : ctx(c), bt(b), s(st) {}
+
+    bool stretches() const { return small || coop || clus; }
+
+    void set_grids(int K) {
+        cgrid = dim3((unsigned)((K + SC - 1) / SC), (unsigned)sp.n_chunks, (unsigned)F);
+        mgrid = dim3((unsigned)((K + SC - 1) / SC), (unsigned)((p + MOM_ROWS - 1) / MOM_ROWS), (unsigned)F);
+        fgrid = dim3((unsigned)((K + 127) / 128), (unsigned)F);
     }
-    for (it = 0; it < bt->max_iter; ++it) {
+
+    // row-sparse apply: the row support flags of z from scratch
+    int zflags(const SolveDev& d, const double* z) {
+        if (!sparse) return 0;
+        zflags_kernel<<<zgrid, 256, 0, s>>>(d, z);
+        LAUNCH_OK("zflags_kernel");
+        return 0;
+    }
+
+    // duality gaps and convergence flags of every column (final_mode: the certificate only)
+    void gap_kernels(const SolveDev& d, int par, int final_mode) {
+        (grouped ? gap_partial_kernel<true> : gap_partial_kernel<false>)<<<cgrid, ST, 0, s>>>(d, par, final_mode);
+        gap_final_kernel<<<fgrid, 128, 0, s>>>(d, it, final_mode);
+    }
+
+    // the cooperative kernels' three beta buffers of nprob columns, in the T / GZ scratch arrays
+    void coop_buffers(int nprob) {
+        ca.nprob = nprob;
+        ca.buf[0] = sp.T;
+        ca.buf[1] = sp.T + (size_t)nprob * p;
+        ca.buf[2] = sp.GZ;
+        ca.dpart = sp.part;
+    }
+
+    int coop_smem_attr(bool cluster) {
+        CUDA_OK(cudaFuncSetAttribute(cluster ? fista_coop_kernel<true, true> : fista_coop_kernel<true, false>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coop_sm));
+        CUDA_OK(cudaFuncSetAttribute(cluster ? fista_coop_kernel<false, true> : fista_coop_kernel<false, false>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coop_sm));
+        return 0;
+    }
+
+    // workspace pointers, the kernels' view of the solve, the column counts
+    int init() {
+        const size_t cols = (size_t)F * ldz;
+        const SolveLayout L = solve_layout(p, ldz, F);
+        char* w = (char*)bt->work_dev;
+        colmap = (int*)(w + L.colmap);
+        src = (int*)(w + L.src);
+        newK = (int*)(w + L.newK);
+        sidx = (int*)(w + L.sidx);
+        scount = (int*)(w + L.scount);
+        const int Gn = grouped ? bt->n_groups : (int)p;
+        sp.F = F;
+        sp.p = (int)p;
+        sp.Gn = Gn;
+        sp.ldz = ldz;
+        sp.pa = bt->pa;
+        sp.g_stride = bt->g_stride;
+        sp.G = bt->G_dev;
+        sp.gptr = bt->gptr_dev;
+        sp.lam1 = bt->lam1_dev;
+        sp.W1 = bt->W1_dev;
+        sp.W2 = bt->W2_dev;
+        sp.D2 = bt->D2_dev;
+        sp.B = Bc[0] = (double*)(w + L.Bw);
+        sp.Bout = bt->B_dev;
+        sp.colmap = colmap;
+        sp.skip = bt->skip_dev;
+        sp.Z = (double*)(w + L.Z);
+        sp.GZ = GBc[0] = (double*)(w + L.GZ);
+        sp.GB = GBc[1] = (double*)(w + L.GB);
+        sp.T = Bc[1] = (double*)(w + L.T);
+        sp.theta[0] = (double*)(w + L.theta);
+        sp.theta[1] = sp.theta[0] + cols;
+        sp.tmom[0] = (double*)(w + L.tmom);
+        sp.tmom[1] = sp.tmom[0] + cols;
+        sp.part = (double*)(w + L.part);
+        sp.rst = (double*)(w + L.rst);
+        sp.flag = (int*)(w + L.flag);
+        const int gpb = grouped ? GPB : SG;  // groups per block iteration
+        sp.gpt = std::max(1, (Gn + gpb * kMaxChunks - 1) / (gpb * kMaxChunks));
+        sp.n_chunks = (Gn + gpb * sp.gpt - 1) / (gpb * sp.gpt);
+        sp.gap = bt->gap_dev;
+        sp.primal = bt->primal_dev;
+        sp.n_iter = bt->n_iter_dev;
+        sp.status = bt->status_dev;
+        sp.counter = ctx->d_counter;
+        sp.ratio = ctx->d_ratio;
+        sp.zflag = sparse ? (unsigned char*)(w + L.zflag) : nullptr;
+        sp.nblk = (int)(ldz / SC);
+        sp.tol = bt->tol;
+        sp.floor_rel = bt->floor_rel;
+        sp.lips_dev = bt->lipschitz_dev;
+        for (int f = 0; f < F; ++f) {
+            if (bt->K[f] < 0 || bt->K[f] > ldz) return fail(ctx, 1, "slm_solve_batch: K[f] out of range");
+            if (bt->K[f] > 0 && ((!bt->lipschitz_dev && !(bt->lipschitz[f] > 0.0)) || !(bt->n_obs[f] > 0.0)))
+                return fail(ctx, 1, "slm_solve_batch: lipschitz and n_obs must be positive");
+            sp.K[f] = bt->K[f];
+            sp.n_obs[f] = bt->n_obs[f] > 0.0 ? bt->n_obs[f] : 1.0;
+            sp.step[f] = bt->lipschitz[f] > 0.0 ? 1.0 / bt->lipschitz[f] : 0.0;
+            Kmax0 = std::max(Kmax0, bt->K[f]);
+            Ktot += bt->K[f];
+        }
+        bt->iters_run = 0;
+        bt->n_unconverged = 0;
+        Kmax = Kmax0;
+        n_active = Ktot;
+        set_grids(Kmax);
+        zgrid = dim3((unsigned)(((long long)p * sp.nblk + 255) / 256), (unsigned)F);
+        return 0;
+    }
+
+    // mode choice (small, coop, cluster eligibility) and the kernel attributes the chosen mode needs
+    int plan() {
+        if (small) {
+            p32 = (int)round_up(p, 32);
+            nsplit = std::max(1, std::min(8, 256 / p32));
+            small_smem = fista_small_smem((int)p, p32, nsplit);
+            CUDA_OK(cudaFuncSetAttribute(fista_small_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)small_smem));
+            CUDA_OK(cudaFuncSetAttribute(fista_small_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)small_smem));
+            return 0;
+        }
+        if (!ctx->coop) return 0;
+        const int maxg = grouped ? bt->max_group : 1;  // 0: the caller did not say
+        coop_sm = coop_smem((int)p);
+        if (maxg <= 0 || coop_sm > (size_t)ctx->coop_max_smem) return 0;
+        ca.seg = coop_seg((int)p);
+        if (Ktot <= kCoopMaxProb) {
+            const int nprob = (int)Ktot;
+            coop_nb = (int)std::min<int64_t>(ctx->sm_count / nprob, std::max<int64_t>(1, p / 16));
+            if (coop_nb >= 1 && (p + coop_nb - 1) / coop_nb + maxg <= CO_ROWS) {
+                coop = true;
+                coop_buffers(nprob);
+                int q = 0;
+                for (int f = 0; f < F; ++f)
+                    for (int k = 0; k < bt->K[f]; ++k, ++q) {
+                        ca.pf[q] = f;
+                        ca.pk[q] = k;
+                    }
+                return coop_smem_attr(false);
+            }
+        }
+        if (p > 16 * CO_ROWS) return 0;
+        for (int cs = 1; cs <= ctx->max_cluster; cs *= 2)
+            if ((p + cs - 1) / cs + maxg <= CO_ROWS) {
+                clus_cs_min = cs;
+                break;
+            }
+        if (clus_cs_min == 0) return 0;
+        // three rounds of co-resident clusters at most, and the three beta buffers of every column must fit in
+        // the T / GZ scratch arrays
+        clus_thr = (int)std::min<long long>(3LL * (ctx->sm_count / clus_cs_min), (long long)F * ldz / 2);
+        return coop_smem_attr(true);
+    }
+
+    // initial state of every column and of the iterate buffers, the support flags
+    int start() {
+        const size_t cols = (size_t)F * ldz;
+        init_cols_kernel<<<(unsigned)((cols + 255) / 256), 256, 0, s>>>(sp.theta[0], sp.tmom[0], sp.flag, colmap,
+                                                                        sp.status, sp.n_iter, bt->skip_dev,
+                                                                        (long long)cols, (int)ldz);
+        LAUNCH_OK("init_cols_kernel");
+        CUDA_OK(cudaMemcpyAsync(sp.B, bt->B_dev, state * sizeof(double), cudaMemcpyDeviceToDevice, s));
+        CUDA_OK(cudaMemcpyAsync(sp.Z, bt->B_dev, state * sizeof(double), cudaMemcpyDeviceToDevice, s));
+        CUDA_OK(cudaMemsetAsync(sp.GB, 0, state * sizeof(double), s));
+        fused = ctx->fused_prox && !small && !coop;
+        if (fused) CUDA_OK(cudaMemcpyAsync(sp.T, bt->B_dev, state * sizeof(double), cudaMemcpyDeviceToDevice, s));
+        if (sparse) CUDA_OK(cudaMemsetAsync(ctx->d_stat, 0, sizeof(unsigned long long), s));
+        return zflags(sp, sp.Z);
+    }
+
+    // small, coop and cluster modes: every iteration up to the next check (or max_iter) in one launch
+    int stretch() {
         const int par = it & 1;
-        const bool check = (small || coop || clus) ? (it == next_check) : (it == next_regular);
-        if (clus && !check) {
-            int n_inner = std::min(next_check, (int)bt->max_iter) - it;
-            int parv = par;
+        int n_inner = std::min(next_check, (int)bt->max_iter) - it;
+        if (clus) {
             const int nprob = (int)n_active;
             int cs = clus_cs_min;
             while (cs * 2 <= ctx->max_cluster && nprob * cs * 2 <= ctx->sm_count) cs *= 2;
-            if (ctx->trace) fprintf(stderr, "[slm] cluster launch it=%d n_inner=%d nprob=%d cs=%d\n", it, n_inner, nprob, cs);
+            if (ctx->trace)
+                fprintf(stderr, "[slm] cluster launch it=%d n_inner=%d nprob=%d cs=%d\n", it, n_inner, nprob, cs);
             coop_list_kernel<<<1, 32, 0, s>>>(sp, src);
             LAUNCH_OK("coop_list_kernel");
-            ca.nprob = nprob;
+            coop_buffers(nprob);
             ca.plist = src;
-            ca.buf[0] = T;
-            ca.buf[1] = T + (size_t)nprob * p;
-            ca.buf[2] = GZ;
-            ca.dpart = part;
-            cudaLaunchConfig_t cfg;
-            memset(&cfg, 0, sizeof(cfg));
+            cudaLaunchConfig_t cfg = {};
             cfg.gridDim = dim3((unsigned)(nprob * cs));
             cfg.blockDim = dim3(CO_T);
             cfg.dynamicSmemBytes = coop_sm;
@@ -1885,57 +1872,68 @@ int slm_solve_batch(slm_ctx* ctx, slm_batch* bt, void* stream) {
             cfg.attrs = at;
             cfg.numAttrs = 1;
             FamTimer tm(ctx, FAM_PROX, s, 0.0);
-            if (grouped)
-                CUDA_OK(cudaLaunchKernelEx(&cfg, fista_coop_kernel<true, true>, sp, ca, parv, n_inner));
-            else
-                CUDA_OK(cudaLaunchKernelEx(&cfg, fista_coop_kernel<false, true>, sp, ca, parv, n_inner));
+            CUDA_OK(cudaLaunchKernelEx(&cfg, grouped ? fista_coop_kernel<true, true> : fista_coop_kernel<false, true>,
+                                       sp, ca, par, n_inner));
             ctx->launches++;
-            it += n_inner - 1;
-            continue;
-        }
-        if (coop && !check) {
-            // every iteration up to the next check in one cooperative launch: the SMs share the
-            // column(s), one grid barrier per iteration
-            int n_inner = std::min(next_check, (int)bt->max_iter) - it;
-            int parv = par;
+        } else if (coop) {
+            // the SMs share the column(s), one grid barrier per iteration
             FamTimer tm(ctx, FAM_PROX, s, 0.0);
+            int parv = par;
             void* args[] = {(void*)&sp, (void*)&ca, (void*)&parv, (void*)&n_inner};
-            const dim3 cgrid2((unsigned)coop_nb, (unsigned)ca.nprob);
             CUDA_OK(cudaLaunchCooperativeKernel(grouped ? (const void*)fista_coop_kernel<true, false>
                                                         : (const void*)fista_coop_kernel<false, false>,
-                                                cgrid2, dim3(CO_T), args, coop_sm, s));
+                                                dim3((unsigned)coop_nb, (unsigned)ca.nprob), dim3(CO_T), args,
+                                                coop_sm, s));
             ctx->launches++;
-            it += n_inner - 1;
-            continue;
-        }
-        if (small && !check) {
-            // every iteration up to the next check (or max_iter) in one launch
-            const int n_inner = std::min(next_check, (int)bt->max_iter) - it;
+        } else {
             FamTimer tm(ctx, FAM_PROX, s, 0.0);
-            const dim3 sgrid((unsigned)Kmax, (unsigned)F);
-            if (grouped)
-                fista_small_kernel<true><<<sgrid, p32 * nsplit, small_smem, s>>>(sp, par, n_inner, p32, nsplit);
-            else
-                fista_small_kernel<false><<<sgrid, p32 * nsplit, small_smem, s>>>(sp, par, n_inner, p32, nsplit);
+            (grouped ? fista_small_kernel<true> : fista_small_kernel<false>)<<<dim3((unsigned)Kmax, (unsigned)F),
+                                                                             p32 * nsplit, small_smem, s>>>(
+                sp, par, n_inner, p32, nsplit);
             LAUNCH_OK("fista_small_kernel");
-            it += n_inner - 1;
-            continue;
         }
-        double algo = 2.0 * (double)p * (double)p * (double)n_active;
-        // the supports change fastest in the first iterations (a cold start is all-zero, then
-        // every weakly penalised column fills up): re-decide the width there without waiting
-        // for the next convergence check
-        if ((coop || clus) && sparse && it > 0) {  // the cooperative iterations do not maintain the row flags
-            zflags_kernel<<<zgrid, 256, 0, s>>>(sp, Z);
-            LAUNCH_OK("zflags_kernel");
+        it += n_inner - 1;
+        return 0;
+    }
+
+    // chunk-width decision from the support-list lengths of a narrow iteration (host copy in ctx->h_scount):
+    // time of the narrow form (per-chunk supports, G re-read per chunk) against one wide chunk per fold
+    // contracting over the largest support
+    void decide_width() {
+        double fw = 0.0, fn = 0.0, bw = 0.0, bn = 0.0;  // flops / G bytes, wide and narrow
+        for (int f = 0; f < F; ++f) {
+            const int Kp = (int)std::min<int64_t>(round_up(sp.K[f], 8), ldz);
+            int smax = 0;
+            for (int cc = 0; cc * kChunkW < Kp; ++cc) {
+                const int sc = ctx->h_scount[f * ncc + cc];
+                smax = std::max(smax, sc);
+                fn += 2.0 * (double)p * sc * std::min(kChunkW, Kp - cc * kChunkW);
+                bn += 8.0 * (double)p * sc;
+            }
+            fw += 2.0 * (double)p * smax * std::min(Kp, cw_wide) * ((Kp + cw_wide - 1) / cw_wide);
+            bw += 8.0 * (double)p * smax * ((Kp + cw_wide - 1) / cw_wide);
         }
+        const double tn = std::max(fn / (0.84 * 35e12), bn / 6.0e12);
+        const double tw = std::max(fw / (0.776 * 35e12), bw / 6.0e12);
+        wide = (fn == 0.0) || (tw < tn);
+    }
+
+    // the Gram apply of one iteration (G Z, or G W_t in the fused iteration): support-flag refresh, width probe,
+    // then the row-sparse or the dense apply
+    int apply(bool check) {
+        const int par = it & 1;
+        const double algo = 2.0 * (double)p * (double)p * (double)n_active;
+        int rc;
+        // the cooperative iterations do not maintain the row flags
+        if ((coop || clus) && it > 0 && (rc = zflags(sp, sp.Z))) return rc;
+        // the supports change fastest in the first iterations (a cold start is all-zero, then every weakly
+        // penalised column fills up): re-decide the width there without waiting for the next convergence check
         const bool probe = can_adapt && !check && !coop && !clus && (it == 1 || it == 3 || it == 6);
-        const int cw_now = (wide && !check && !probe) ? cw_wide : cw;
-        const double* ap_in = fused ? Bc[par] : Z;  // fused: the Gram acts on the iterate itself
-        double* ap_out = fused ? GBc[par] : GZ;
-        int rc = sparse ? apply_rowsparse(ctx, sp, Kcur, ap_in, ap_out, cw_now, (int)((ldz + cw_now - 1) / cw_now), sidx,
-                                          scount, s, algo)
-                        : apply_batched(ctx, bt->G_dev, bt->g_stride, bt->pa, p, F, Kcur, ap_in, ldz, ap_out, s, algo);
+        const int cw = (wide && !check && !probe) ? cw_wide : kChunkW;
+        const double* in = fused ? Bc[par] : sp.Z;  // fused: the Gram acts on the iterate itself
+        double* out = fused ? GBc[par] : sp.GZ;
+        rc = sparse ? apply_rowsparse(ctx, sp, sp.K, in, out, cw, (int)((ldz + cw - 1) / cw), sidx, scount, s, algo)
+                    : apply_batched(ctx, bt->G_dev, bt->g_stride, bt->pa, p, F, sp.K, in, ldz, out, s, algo);
         if (rc) return rc;
         if ((check || probe) && (can_adapt || (clus_thr > 0 && sparse && F * ncc <= kMaxScount)))
             CUDA_OK(cudaMemcpyAsync(ctx->h_scount, scount, sizeof(int) * (size_t)F * ncc, cudaMemcpyDeviceToHost, s));
@@ -1943,94 +1941,101 @@ int slm_solve_batch(slm_ctx* ctx, slm_batch* bt, void* stream) {
             CUDA_OK(cudaStreamSynchronize(s));
             decide_width();
         }
-        if (check) {
-            CUDA_OK(cudaMemsetAsync(ctx->d_counter, 0, sizeof(int) * SLM_MAX_FOLDS, s));
-            CUDA_OK(cudaMemsetAsync(ctx->d_ratio, 0, sizeof(unsigned long long), s));
-            {
-                FamTimer tm(ctx, FAM_GAP, s, 0.0);
-                SolveDev spg = sp;
-                if (fused) {  // B = W_t, GZ = G W_t itself
-                    spg.B = Bc[par];
-                    spg.GZ = GBc[par];
-                    spg.direct = 1;
-                }
-                if (grouped)
-                    gap_partial_kernel<true><<<cgrid, ST, 0, s>>>(spg, par, 0);
-                else
-                    gap_partial_kernel<false><<<cgrid, ST, 0, s>>>(spg, par, 0);
-                gap_final_kernel<<<fgrid, 128, 0, s>>>(spg, it, 0);
-                if (fused) settle_done_kernel<<<mgrid, ST, 0, s>>>(sp, Bc[par], Bc[par ^ 1]);
+        return 0;
+    }
+
+    // few columns left: one cluster per column pays when the columns are sparse (every cluster reads its own
+    // support rows of the Gram: |S| p 8 bytes per column and iteration, nothing shared between columns) --
+    // otherwise the GEMM path, which shares the Gram between the columns of a chunk, stays
+    bool cluster_pays() const {
+        if (n_active > clus_thr || !sparse || F * ncc > kMaxScount) return false;
+        double bytes = 0.0, flops = 0.0;
+        for (int f = 0; f < F; ++f) {
+            const int Kp = (int)std::min<int64_t>(round_up(n_active_f[f], 8), ldz);
+            for (int cc = 0; cc * kChunkW < Kp; ++cc) {
+                const double sc = (double)std::min<long long>(ctx->h_scount[f * ncc + cc], p);
+                const double ncol = (double)std::min(kChunkW, Kp - cc * kChunkW);
+                bytes += ncol * (double)p * sc * 8.0;
+                flops += 2.0 * ncol * (double)p * sc;
             }
-            LAUNCH_OK("gap kernels");
-            ctx->launches++;
-            CUDA_OK(cudaMemcpyAsync(ctx->h_counter, ctx->d_counter, sizeof(int) * SLM_MAX_FOLDS,
-                                    cudaMemcpyDeviceToHost, s));
-            CUDA_OK(cudaMemcpyAsync(ctx->h_ratio, ctx->d_ratio, sizeof(unsigned long long),
-                                    cudaMemcpyDeviceToHost, s));
-            CUDA_OK(cudaStreamSynchronize(s));
-            n_active = 0;
-            bool shrink = false;
-            for (int f = 0; f < F; ++f) {
-                n_active_f[f] = ctx->h_counter[f];
-                n_active += n_active_f[f];
-                if (round_up(n_active_f[f], 8) < round_up(Kcur[f], 8)) shrink = true;
-            }
-            next_regular = it + ((n_active * 8 <= Ktot && Ktot >= 16) ? std::max(2, check_every / 2) : check_every);
-            if (ctx->trace)
-                fprintf(stderr, "[slm] it=%d active=%lld Kmax=%d%s\n", it, n_active, Kmax,
-                        coop ? " coop" : (small ? " small" : (clus ? " cluster" : "")));
-            if (n_active == 0) break;
-            if (clus_thr > 0) {
-                // few columns left: one cluster per column pays when the columns are sparse (every
-                // cluster reads its own support rows of the Gram: |S| p 8 bytes per column and
-                // iteration, nothing shared between columns) -- otherwise the GEMM path, which
-                // shares the Gram between the columns of a chunk, stays
-                bool pays = false;
-                if (n_active <= clus_thr && sparse && F * ncc <= kMaxScount) {
-                    double bytes = 0.0, flops = 0.0;
-                    for (int f = 0; f < F; ++f) {
-                        const int Kp = (int)std::min<int64_t>(round_up(n_active_f[f], 8), ldz);
-                        for (int cc = 0; cc * cw < Kp; ++cc) {
-                            const double sc = (double)std::min<long long>(ctx->h_scount[f * ncc + cc], p);
-                            const double ncol = (double)std::min(cw, Kp - cc * cw);
-                            bytes += ncol * (double)p * sc * 8.0;
-                            flops += 2.0 * ncol * (double)p * sc;
-                        }
-                    }
-                    const int conc = std::max(1, std::min(ctx->sm_count / clus_cs_min, 8 * (16 / clus_cs_min)));
-                    const double rounds = (double)((n_active + conc - 1) / conc);
-                    const double t_cl = std::max(rounds * 12e-6, bytes / 3.0e12);
-                    const double t_ge = 90e-6 + flops / 20e12;
-                    pays = t_cl < 0.5 * t_ge;
-                }
-                if (pays && !clus) {
-                    clus = true;
-                    interval = check_every;
-                    prev_ratio = 0.0;
-                } else if (!pays && clus) {
-                    clus = false;  // the supports filled up: back to the shared-Gram GEMM iterations
-                }
-            }
-            do_compact = shrink && !small && !coop;  // idle CTAs of the fused kernels cost nothing: no compaction
-            if (small || coop || clus) {
-                // checks at 0, c, 3c, 7c, ... (c = check_every), at most 2048 apart -- sooner when
-                // the worst gap/tolerance ratio of the last two checks says the tolerance is
-                // nearer than that (linear-rate extrapolation + 15 %)
-                int step_to = interval;
-                double ratio;
-                memcpy(&ratio, ctx->h_ratio, sizeof(double));
-                if (prev_ratio > 0.0 && ratio > 1.0 && ratio < prev_ratio && it > prev_check) {
-                    const double rate = log(prev_ratio / ratio) / (double)(it - prev_check);
-                    const double need = 1.15 * log(ratio) / rate + 1.0;
-                    if (need < (double)step_to) step_to = std::max(std::max(2, check_every / 2), (int)ceil(need));
-                }
-                prev_ratio = ratio;
-                prev_check = it;
-                next_check = it + step_to;
-                interval = std::min(interval * 2, 2048);
-            }
-            if (can_adapt) decide_width();
         }
+        const int conc = std::max(1, std::min(ctx->sm_count / clus_cs_min, 8 * (16 / clus_cs_min)));
+        const double rounds = (double)((n_active + conc - 1) / conc);
+        const double t_cl = std::max(rounds * 12e-6, bytes / 3.0e12);
+        const double t_ge = 90e-6 + flops / 20e12;
+        return t_cl < 0.5 * t_ge;
+    }
+
+    // convergence check after this iteration's apply: gaps and flags, active counts on the host, the cluster
+    // switch, the next check, the chunk width
+    int check() {
+        const int par = it & 1;
+        CUDA_OK(cudaMemsetAsync(ctx->d_counter, 0, sizeof(int) * SLM_MAX_FOLDS, s));
+        CUDA_OK(cudaMemsetAsync(ctx->d_ratio, 0, sizeof(unsigned long long), s));
+        {
+            FamTimer tm(ctx, FAM_GAP, s, 0.0);
+            SolveDev spg = sp;
+            if (fused) {  // B = W_t, GZ = G W_t itself
+                spg.B = Bc[par];
+                spg.GZ = GBc[par];
+                spg.direct = 1;
+            }
+            gap_kernels(spg, par, 0);
+            if (fused) settle_done_kernel<<<mgrid, ST, 0, s>>>(sp, Bc[par], Bc[par ^ 1]);
+        }
+        LAUNCH_OK("gap kernels");
+        ctx->launches++;
+        CUDA_OK(cudaMemcpyAsync(ctx->h_counter, ctx->d_counter, sizeof(int) * SLM_MAX_FOLDS, cudaMemcpyDeviceToHost,
+                                s));
+        CUDA_OK(cudaMemcpyAsync(ctx->h_ratio, ctx->d_ratio, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+        CUDA_OK(cudaStreamSynchronize(s));
+        n_active = 0;
+        bool shrink = false;
+        for (int f = 0; f < F; ++f) {
+            n_active_f[f] = ctx->h_counter[f];
+            n_active += n_active_f[f];
+            if (round_up(n_active_f[f], 8) < round_up(sp.K[f], 8)) shrink = true;
+        }
+        next_regular = it + ((n_active * 8 <= Ktot && Ktot >= 16) ? std::max(2, check_every / 2) : check_every);
+        if (ctx->trace)
+            fprintf(stderr, "[slm] it=%d active=%lld Kmax=%d%s\n", it, n_active, Kmax,
+                    coop ? " coop" : (small ? " small" : (clus ? " cluster" : "")));
+        if (n_active == 0) return 0;  // every column converged: the solve stops
+        if (clus_thr > 0) {
+            const bool pays = cluster_pays();
+            if (pays && !clus) {
+                clus = true;
+                interval = check_every;
+                prev_ratio = 0.0;
+            } else if (!pays && clus) {
+                clus = false;  // the supports filled up: back to the shared-Gram GEMM iterations
+            }
+        }
+        do_compact = shrink && !small && !coop;  // idle CTAs of the fused kernels cost nothing: no compaction
+        if (stretches()) {
+            // checks at 0, c, 3c, 7c, ... (c = check_every), at most 2048 apart -- sooner when the worst
+            // gap/tolerance ratio of the last two checks says the tolerance is nearer than that (linear-rate
+            // extrapolation + 15 %)
+            int step_to = interval;
+            double ratio;
+            memcpy(&ratio, ctx->h_ratio, sizeof(double));
+            if (prev_ratio > 0.0 && ratio > 1.0 && ratio < prev_ratio && it > prev_check) {
+                const double rate = log(prev_ratio / ratio) / (double)(it - prev_check);
+                const double need = 1.15 * log(ratio) / rate + 1.0;
+                if (need < (double)step_to) step_to = std::max(std::max(2, check_every / 2), (int)ceil(need));
+            }
+            prev_ratio = ratio;
+            prev_check = it;
+            next_check = it + step_to;
+            interval = std::min(interval * 2, 2048);
+        }
+        if (can_adapt) decide_width();
+        return 0;
+    }
+
+    // proximal step, momentum and restart of one iteration: fused or two-kernel
+    int prox() {
+        const int par = it & 1;
         {
             FamTimer tm(ctx, FAM_PROX, s, 0.0);
             if (fused) {
@@ -2039,7 +2044,7 @@ int slm_solve_batch(slm_ctx* ctx, slm_batch* bt, void* stream) {
                 fa.Bnew = Bc[par ^ 1];
                 fa.GBcur = GBc[par];
                 fa.GBold = GBc[par ^ 1];
-                fa.stash = Z;
+                fa.stash = sp.Z;
                 fa.it = it;
                 fa.use_rst = use_rst;
                 use_rst = 0;
@@ -2056,119 +2061,118 @@ int slm_solve_batch(slm_ctx* ctx, slm_batch* bt, void* stream) {
                     prox_fused_kernel<true, 5><<<cgrid, ST, 0, s>>>(sp, fa, par);
                 else
                     prox_fused_kernel<true, 8><<<cgrid, ST, 0, s>>>(sp, fa, par);
-            } else if (ctx->prox2) {
-                // one lane per column, 32 columns per block (solver_kernels.cuh, second mapping)
-                SolveDev s2 = sp;
-                s2.gpt = std::max(1, (Gn + PX_W * kMaxChunks - 1) / (PX_W * kMaxChunks));
-                s2.n_chunks = (Gn + PX_W * s2.gpt - 1) / (PX_W * s2.gpt);
-                const dim3 cgrid2((unsigned)((Kmax + PX_C - 1) / PX_C), (unsigned)s2.n_chunks, (unsigned)F);
-                const dim3 mgrid2((unsigned)((Kmax + PX_C - 1) / PX_C), (unsigned)((p + MOM_ROWS - 1) / MOM_ROWS),
-                                  (unsigned)F);
-                if (grouped)
-                    prox_main2_kernel<true><<<cgrid2, PX_W * PX_C, 0, s>>>(s2, par);
-                else
-                    prox_main2_kernel<false><<<cgrid2, PX_W * PX_C, 0, s>>>(s2, par);
-                prox_momentum2_kernel<<<mgrid2, PX_W * PX_C, 0, s>>>(s2, par);
             } else {
-                if (grouped)
-                    prox_main_kernel<true><<<cgrid, ST, 0, s>>>(sp, par);
-                else
-                    prox_main_kernel<false><<<cgrid, ST, 0, s>>>(sp, par);
+                (grouped ? prox_main_kernel<true> : prox_main_kernel<false>)<<<cgrid, ST, 0, s>>>(sp, par);
                 prox_momentum_kernel<<<mgrid, ST, 0, s>>>(sp, par);
             }
         }
         LAUNCH_OK("prox kernels");
         ctx->launches++;
-        if (do_compact) {
-            // converged columns leave the batch (after this iteration's epilogue, so that GZ of
-            // the old layout is no longer needed): scatter their coefficients to the caller's
-            // array, move the active columns of Z, B, GB to the front
-            SolveDev spc = sp;
-            if (fused) {
-                // live state after this iteration's prox: W_{t+1} (other buffer), W_t, G W_t; the restart dot of the
-                // iteration is reduced per column before the columns are renumbered
-                spc.Z = Bc[par ^ 1];
-                spc.B = Bc[par];
-                spc.GB = GBc[par];
-                restart_reduce_kernel<<<fgrid, 128, 0, s>>>(sp, par);
-                use_rst = 1;
-            }
-            compact_plan_kernel<<<F, 32, 0, s>>>(sp, src, newK);
-            scatter_done_kernel<<<mgrid, ST, 0, s>>>(spc, 0);
-            compact_move_kernel<<<dim3((unsigned)((p + 127) / 128), 3, (unsigned)F), 128, 0, s>>>(spc, src, newK);
-            compact_cols_kernel<<<F, 32, 0, s>>>(sp, src, newK, colmap);
-            LAUNCH_OK("compaction kernels");
-            ctx->launches += 3;
-            Kmax = 0;
-            for (int f = 0; f < F; ++f) {
-                sp.K[f] = Kcur[f] = n_active_f[f];
-                Kmax = std::max(Kmax, Kcur[f]);
-            }
-            grids(Kmax, cgrid, mgrid, fgrid);
-            do_compact = false;
-            if (sparse) {  // the column blocks moved: support flags from scratch
-                zflags_kernel<<<zgrid, 256, 0, s>>>(sp, fused ? Bc[par ^ 1] : Z);
-                LAUNCH_OK("zflags_kernel");
-            }
-        }
-        if (fused && clus) {
-            // the cluster kernels take over from the next iteration: hand them the two-kernel state
-            const int pn = par ^ 1;
-            fused_to_classic_kernel<<<mgrid, ST, 0, s>>>(sp, Bc[pn], Bc[par], GBc[par], it + 1, pn, use_rst);
-            LAUNCH_OK("fused_to_classic_kernel");
-            use_rst = 0;
-            fused = false;
-            if (sparse) {
-                zflags_kernel<<<zgrid, 256, 0, s>>>(sp, Z);
-                LAUNCH_OK("zflags_kernel");
-            }
-        }
+        return 0;
     }
-    bt->iters_run = it;
-    // coefficients still in the working array go back to the caller's layout
-    {
+
+    // converged columns leave the batch (after this iteration's epilogue, so that GZ of the old layout is no
+    // longer needed): scatter their coefficients to the caller's array, move the active columns of Z, B, GB to
+    // the front
+    int compact() {
+        const int par = it & 1;
+        SolveDev spc = sp;
+        if (fused) {
+            // live state after this iteration's prox: W_{t+1} (other buffer), W_t, G W_t; the restart dot of the
+            // iteration is reduced per column before the columns are renumbered
+            spc.Z = Bc[par ^ 1];
+            spc.B = Bc[par];
+            spc.GB = GBc[par];
+            restart_reduce_kernel<<<fgrid, 128, 0, s>>>(sp, par);
+            use_rst = 1;
+        }
+        compact_plan_kernel<<<F, 32, 0, s>>>(sp, src, newK);
+        scatter_done_kernel<<<mgrid, ST, 0, s>>>(spc, 0);
+        compact_move_kernel<<<dim3((unsigned)((p + 127) / 128), 3, (unsigned)F), 128, 0, s>>>(spc, src, newK);
+        compact_cols_kernel<<<F, 32, 0, s>>>(sp, src, newK, colmap);
+        LAUNCH_OK("compaction kernels");
+        ctx->launches += 3;
+        Kmax = 0;
+        for (int f = 0; f < F; ++f) {
+            sp.K[f] = n_active_f[f];
+            Kmax = std::max(Kmax, sp.K[f]);
+        }
+        set_grids(Kmax);
+        do_compact = false;
+        return zflags(sp, fused ? Bc[par ^ 1] : sp.Z);  // the column blocks moved: support flags from scratch
+    }
+
+    // the cluster kernels take over from the next iteration: hand them the two-kernel state
+    int hand_over() {
+        const int par = it & 1, pn = par ^ 1;
+        fused_to_classic_kernel<<<mgrid, ST, 0, s>>>(sp, Bc[pn], Bc[par], GBc[par], it + 1, pn, use_rst);
+        LAUNCH_OK("fused_to_classic_kernel");
+        use_rst = 0;
+        fused = false;
+        return zflags(sp, sp.Z);
+    }
+
+    // coefficients still in the working array go back to the caller's layout; then the final certificate from an
+    // exact G*B, in the original column order
+    int finish() {
+        bt->iters_run = it;
         SolveDev spe = sp;
         if (fused) spe.B = Bc[it & 1];
         scatter_done_kernel<<<mgrid, ST, 0, s>>>(spe, 1);
+        LAUNCH_OK("scatter_done_kernel");
+        SolveDev fin = sp;
+        fin.B = bt->B_dev;
+        fin.colmap = nullptr;
+        for (int f = 0; f < F; ++f) fin.K[f] = bt->K[f];
+        set_grids(Kmax0);
+        CUDA_OK(cudaMemcpyAsync(sp.Z, bt->B_dev, state * sizeof(double), cudaMemcpyDeviceToDevice, s));
+        int rc = zflags(fin, sp.Z);
+        if (rc) return rc;
+        if (sparse) {
+            if ((rc = apply_rowsparse(ctx, fin, bt->K, sp.Z, sp.GZ, kChunkW, ncc, sidx, scount, s, 0.0))) return rc;
+            CUDA_OK(cudaMemcpyAsync(ctx->h_stat, ctx->d_stat, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+        } else if ((rc = apply_batched(ctx, bt->G_dev, bt->g_stride, bt->pa, p, F, bt->K, sp.Z, ldz, sp.GZ, s, 0.0)))
+            return rc;
+        CUDA_OK(cudaMemsetAsync(ctx->d_counter, 0, sizeof(int) * SLM_MAX_FOLDS, s));
+        {
+            FamTimer tm(ctx, FAM_GAP, s, 0.0);
+            gap_kernels(fin, 0, 1);
+        }
+        LAUNCH_OK("gap kernels(final)");
+        ctx->launches++;
+        CUDA_OK(cudaMemcpyAsync(ctx->h_counter, ctx->d_counter, sizeof(int) * SLM_MAX_FOLDS, cudaMemcpyDeviceToHost, s));
+        CUDA_OK(cudaStreamSynchronize(s));
+        bt->n_unconverged = 0;
+        for (int f = 0; f < F; ++f) bt->n_unconverged += ctx->h_counter[f];
+        if (sparse) ctx->apply_exec_flops += 2.0 * (double)p * (double)(*ctx->h_stat);
+        return 0;
     }
-    LAUNCH_OK("scatter_done_kernel");
+};
 
-    // final certificate from an exact G*B, in the original column order
-    SolveDev fin = sp;
-    fin.B = bt->B_dev;
-    fin.colmap = nullptr;
-    for (int f = 0; f < F; ++f) fin.K[f] = bt->K[f];
-    grids(Kmax0, cgrid, mgrid, fgrid);
-    CUDA_OK(cudaMemcpyAsync(Z, bt->B_dev, state * sizeof(double), cudaMemcpyDeviceToDevice, s));
-    if (sparse) {
-        zflags_kernel<<<zgrid, 256, 0, s>>>(fin, Z);
-        LAUNCH_OK("zflags_kernel");
-        int rc = apply_rowsparse(ctx, fin, bt->K, Z, GZ, cw, ncc, sidx, scount, s, 0.0);
-        if (rc) return rc;
-        CUDA_OK(cudaMemcpyAsync(ctx->h_stat, ctx->d_stat, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
-    } else {
-        int rc = apply_batched(ctx, bt->G_dev, bt->g_stride, bt->pa, p, F, bt->K, Z, ldz, GZ, s, 0.0);
-        if (rc) return rc;
+int slm_solve_batch(slm_ctx* ctx, slm_batch* bt, void* stream) {
+    if (!ctx || !bt) return fail(ctx, 1, "slm_solve_batch: null argument");
+    if (bt->n_folds < 1 || bt->n_folds > SLM_MAX_FOLDS) return fail(ctx, 1, "slm_solve_batch: n_folds out of range");
+    if (bt->ldz % 8) return fail(ctx, 1, "slm_solve_batch: ldz must be a multiple of 8");
+    if (!bt->G_dev || !bt->B_dev || !bt->work_dev) return fail(ctx, 1, "slm_solve_batch: null device pointer");
+    if (bt->work_bytes < slm_solve_workspace(bt->p, bt->ldz, bt->n_folds, bt->n_groups))
+        return fail(ctx, 1, "slm_solve_batch: workspace too small");
+    BatchSolve b(ctx, bt, (cudaStream_t)stream);
+    int rc = b.init();
+    if (rc || b.Kmax0 == 0) return rc;
+    if ((rc = b.plan()) || (rc = b.start())) return rc;
+    for (b.it = 0; b.it < bt->max_iter; ++b.it) {
+        const bool check = b.it == (b.stretches() ? b.next_check : b.next_regular);
+        if (b.stretches() && !check) {
+            if ((rc = b.stretch())) return rc;
+            continue;
+        }
+        if ((rc = b.apply(check)) || (check && (rc = b.check()))) return rc;
+        if (b.n_active == 0) break;
+        if ((rc = b.prox()) || (b.do_compact && (rc = b.compact())) || (b.fused && b.clus && (rc = b.hand_over())))
+            return rc;
     }
-    CUDA_OK(cudaMemsetAsync(ctx->d_counter, 0, sizeof(int) * SLM_MAX_FOLDS, s));
-    {
-        FamTimer tm(ctx, FAM_GAP, s, 0.0);
-        if (grouped)
-            gap_partial_kernel<true><<<cgrid, ST, 0, s>>>(fin, 0, 1);
-        else
-            gap_partial_kernel<false><<<cgrid, ST, 0, s>>>(fin, 0, 1);
-        gap_final_kernel<<<fgrid, 128, 0, s>>>(fin, it, 1);
-    }
-    LAUNCH_OK("gap kernels(final)");
-    ctx->launches++;
-    CUDA_OK(cudaMemcpyAsync(ctx->h_counter, ctx->d_counter, sizeof(int) * SLM_MAX_FOLDS, cudaMemcpyDeviceToHost, s));
-    CUDA_OK(cudaStreamSynchronize(s));
-    bt->n_unconverged = 0;
-    for (int f = 0; f < F; ++f) bt->n_unconverged += ctx->h_counter[f];
-    if (sparse) ctx->apply_exec_flops += 2.0 * (double)p * (double)(*ctx->h_stat);
-    return 0;
+    return b.finish();
 }
-
 
 // ---- second-order phase: one lock-step Newton step of k columns (newton_kernels.cuh) ------------
 static inline int64_t nw_ldh(int64_t p) { return round_up(p, 8); }

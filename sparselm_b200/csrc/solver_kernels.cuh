@@ -20,12 +20,8 @@
 
 namespace slm {
 
-#ifndef SLM_PROX_UR
-#define SLM_PROX_UR 1    // rows of a group in flight together in prox_main_kernel
-#endif
-#ifndef SLM_PROX_MINB
-#define SLM_PROX_MINB 4  // resident blocks per SM prox_main_kernel is compiled for
-#endif
+constexpr int PROX_UR = 1;         // rows of a group in flight together in prox_main_kernel
+constexpr int PROX_MINB = 4;       // resident blocks per SM prox_main_kernel is compiled for
 constexpr int SC = 8;              // grid columns per block
 constexpr int SG = 32;             // group lanes per block
 constexpr int ST = SC * SG;        // threads per block
@@ -128,7 +124,7 @@ __device__ __forceinline__ bool sub_any(unsigned qmask, bool v) {
 // ---- K6a: GB recurrence, gradient step, soft-threshold, group shrink, ridge -----
 // writes T = beta_{k+1} and the per-chunk restart dot  sum (z - b+)(b+ - b)
 template <bool GROUPED>
-__global__ void __launch_bounds__(ST, SLM_PROX_MINB) prox_main_kernel(const __grid_constant__ SolveDev sp, int par) {
+__global__ void __launch_bounds__(ST, PROX_MINB) prox_main_kernel(const __grid_constant__ SolveDev sp, int par) {
     const int f = blockIdx.z, chunk = blockIdx.y;
     const int Kf = sp.K[f];
     const int k0 = blockIdx.x * SC;
@@ -160,7 +156,7 @@ __global__ void __launch_bounds__(ST, SLM_PROX_MINB) prox_main_kernel(const __gr
     const int rstep = GROUPED ? SUB : 1;
     const unsigned qmask = 0x01010101u << c;
 
-    constexpr int UR = GROUPED ? SLM_PROX_UR : 1;  // rows of a group whose loads are in flight together
+    constexpr int UR = GROUPED ? PROX_UR : 1;  // rows of a group whose loads are in flight together
     double dot = 0.0;
     for (int i = 0; i < sp.gpt; ++i) {
         const int g = (chunk * sp.gpt + i) * gstep + gsl;
@@ -343,7 +339,7 @@ __device__ __forceinline__ double fused_theta(int it, double tm, double dsum, do
 // FZ_RC: rows per lane kept in registers across the group-norm reduction (the host picks the smallest
 // instantiation that covers the largest group: unused row slots still cost issue slots)
 template <bool GROUPED, int FZ_RC>
-__global__ void __launch_bounds__(ST, GROUPED ? (FZ_RC <= 5 ? 3 : 2) : SLM_PROX_MINB)
+__global__ void __launch_bounds__(ST, GROUPED ? (FZ_RC <= 5 ? 3 : 2) : PROX_MINB)
     prox_fused_kernel(const __grid_constant__ SolveDev sp, const __grid_constant__ FusedArgs fa, int par) {
     const int f = blockIdx.z, chunk = blockIdx.y;
     const int Kf = sp.K[f];
@@ -583,195 +579,6 @@ __global__ void __launch_bounds__(ST) fused_to_classic_kernel(const __grid_const
     if (active && blockIdx.y == 0 && r == 0) {
         sp.theta[par][colbase] = th;
         sp.tmom[par][colbase] = tn;
-    }
-}
-
-// ---- K6 (second mapping): one lane per grid column --------------------------------------------
-// prox_main_kernel / prox_momentum_kernel above give a row of the state arrays to 8 threads (a
-// 64-byte segment) and a group to 4 sub-lanes; ncu shows them latency-bound (long_scoreboard 22-24
-// stalls per issue, DRAM 19-23 %).  Here a warp covers 32 ADJACENT COLUMNS of one row (one 256-byte
-// request per array and row), a lane walks the rows of its groups alone (group norms are
-// thread-local: no shuffles) and issues the loads of PX_UR rows before it uses the first.
-// Same arithmetic, same per-chunk partial sums of the restart dot (chunk order fixed).
-constexpr int PX_W = 8;    // warps per block = groups handled side by side
-constexpr int PX_C = 32;   // columns per block
-constexpr int PX_UR = 4;   // rows of a group in flight together
-
-template <bool GROUPED>
-__global__ void __launch_bounds__(PX_W * PX_C) prox_main2_kernel(const __grid_constant__ SolveDev sp, int par) {
-    const int f = blockIdx.z, chunk = blockIdx.y;
-    const int Kf = sp.K[f];
-    const int k0 = blockIdx.x * PX_C;
-    if (k0 >= Kf) return;
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int k = k0 + lane;
-    __shared__ double red[PX_W][PX_C];
-    const long long ldz = sp.ldz;
-    const long long colbase = (long long)f * ldz + k;
-    const bool active = (k < Kf) && sp.flag[colbase] == 0;
-    if (__syncthreads_and(!active)) return;
-
-    const double theta = active ? sp.theta[par][colbase] : 0.0;
-    const double inv1pt = 1.0 / (1.0 + theta);
-    const double* __restrict__ cvec = sp.G + (long long)f * sp.g_stride + (long long)sp.p * sp.pa;
-    const double n = sp.n_obs[f], step = sp.lips_dev ? 1.0 / sp.lips_dev[f] : sp.step[f];
-    const double son = step / n;
-    const int ko = (active && sp.colmap) ? sp.colmap[colbase] : k;
-    const int kk = active ? k : 0;  // inactive lanes shadow column 0 of their fold (reads only)
-    const long long sbase = (long long)f * sp.p * ldz + kk;
-    const long long wbase = (long long)f * sp.p * ldz + (active ? ko : 0);
-    const long long gbase = (long long)f * sp.Gn * ldz + (active ? ko : 0);
-    const double lam1 = (active && sp.lam1) ? sp.lam1[(long long)f * ldz + ko] : 0.0;
-
-    double dot = 0.0;
-    for (int i = 0; i < sp.gpt; ++i) {
-        const int g = (chunk * sp.gpt + i) * PX_W + w;
-        if (g >= sp.Gn) break;  // uniform over the warp
-        const int ja = (GROUPED && sp.gptr) ? sp.gptr[g] : g;
-        const int jb = (GROUPED && sp.gptr) ? sp.gptr[g + 1] : g + 1;
-        double ss = 0.0;
-        for (int j0 = ja; j0 < jb; j0 += PX_UR) {
-            double gz[PX_UR], gbo[PX_UR], z[PX_UR], cj[PX_UR], w1[PX_UR];
-#pragma unroll
-            for (int r = 0; r < PX_UR; ++r) {
-                const int j = j0 + r;
-                if (j < jb) {
-                    const long long e = sbase + (long long)j * ldz;
-                    gz[r] = sp.GZ[e];
-                    gbo[r] = sp.GB[e];
-                    z[r] = sp.Z[e];
-                    cj[r] = cvec[j];
-                    w1[r] = sp.W1 ? sp.W1[wbase + (long long)j * ldz] : lam1;
-                }
-            }
-#pragma unroll
-            for (int r = 0; r < PX_UR; ++r) {
-                const int j = j0 + r;
-                if (j < jb) {
-                    const long long e = sbase + (long long)j * ldz;
-                    const double gb = (gz[r] + theta * gbo[r]) * inv1pt;
-                    const double v = z[r] - son * (gz[r] - cj[r]);
-                    const double u = softt(v, step * w1[r]);
-                    if (active) {
-                        sp.GB[e] = gb;
-                        sp.T[e] = u;  // stash; scaled below
-                    }
-                    ss += u * u;
-                }
-            }
-        }
-        const double nrm = sqrt(ss);
-        const double w2 = sp.W2 ? sp.W2[gbase + (long long)g * ldz] : 0.0;
-        const double d2 = sp.D2 ? sp.D2[gbase + (long long)g * ldz] : 0.0;
-        double scale = nrm > 0.0 ? fmax(0.0, 1.0 - step * w2 / nrm) : 0.0;
-        scale = scale / (1.0 + step * d2);
-        if (active) {
-            for (int j0 = ja; j0 < jb; j0 += PX_UR) {
-                double t[PX_UR], z[PX_UR], bo[PX_UR];
-#pragma unroll
-                for (int r = 0; r < PX_UR; ++r) {
-                    const int j = j0 + r;
-                    if (j < jb) {
-                        const long long e = sbase + (long long)j * ldz;
-                        t[r] = sp.T[e];
-                        z[r] = sp.Z[e];
-                        bo[r] = sp.B[e];
-                    }
-                }
-#pragma unroll
-                for (int r = 0; r < PX_UR; ++r) {
-                    const int j = j0 + r;
-                    if (j < jb) {
-                        const double bn = scale * t[r];
-                        sp.T[sbase + (long long)j * ldz] = bn;
-                        dot += (z[r] - bn) * (bn - bo[r]);
-                    }
-                }
-            }
-        }
-    }
-    red[w][lane] = active ? dot : 0.0;
-    __syncthreads();
-    if (w == 0 && active) {
-        double d = 0.0;
-#pragma unroll
-        for (int q = 0; q < PX_W; ++q) d += red[q][lane];
-        sp.part[(((long long)f * sp.n_chunks + chunk) * NQ + 0) * ldz + k] = d;
-    }
-}
-
-// restart test, momentum, state rotation; row support flags per 8-column block for the row-sparse apply
-__global__ void __launch_bounds__(PX_W * PX_C) prox_momentum2_kernel(const __grid_constant__ SolveDev sp, int par) {
-    const int f = blockIdx.z;
-    const int Kf = sp.K[f];
-    const int k0 = blockIdx.x * PX_C;
-    if (k0 >= Kf) return;
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int k = k0 + lane;
-    const long long ldz = sp.ldz;
-    const long long colbase = (long long)f * ldz + k;
-    const bool active = (k < Kf) && sp.flag[colbase] == 0;
-    const int j0 = blockIdx.y * MOM_ROWS;
-    const int j1 = min(j0 + MOM_ROWS, sp.p);
-    const int cb0 = blockIdx.x * (PX_C / SC);  // first 8-column flag block of this thread block
-    if (__syncthreads_and(!active)) {
-        if (sp.zflag)
-            for (int e = threadIdx.x; e < (j1 - j0) * (PX_C / SC); e += PX_W * PX_C) {
-                const int j = j0 + e / (PX_C / SC), cb = cb0 + e % (PX_C / SC);
-                if (cb < sp.nblk) sp.zflag[((long long)f * sp.p + j) * sp.nblk + cb] = 0;
-            }
-        return;
-    }
-    // restart decision of this column: every warp sums the chunk partials itself (fixed order)
-    double dsum = 0.0;
-    if (active)
-        for (int ch = 0; ch < sp.n_chunks; ++ch) dsum += sp.part[(((long long)f * sp.n_chunks + ch) * NQ + 0) * ldz + k];
-    const double tm = active ? sp.tmom[par][colbase] : 1.0;
-    double tn = 0.5 * (1.0 + sqrt(1.0 + 4.0 * tm * tm));
-    double th = (tm - 1.0) / tn;
-    if (dsum > 0.0) {  // gradient-scheme adaptive restart (O'Donoghue & Candes)
-        th = 0.0;
-        tn = 1.0;
-    }
-    const long long sbase = (long long)f * sp.p * ldz + k;
-#pragma unroll 1
-    for (int jj = w; jj < MOM_ROWS; jj += 4 * PX_W) {  // uniform trip count: the ballots need whole warps
-        double bn[4], b[4];
-        bool inb[4];
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const int j = j0 + jj + r * PX_W;
-            inb[r] = j < j1;
-            if (inb[r] && active) {
-                const long long e = sbase + (long long)j * ldz;
-                bn[r] = sp.T[e];
-                b[r] = sp.B[e];
-            }
-        }
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const int j = j0 + jj + r * PX_W;
-            bool nz = false;
-            if (inb[r] && active) {
-                const long long e = sbase + (long long)j * ldz;
-                const double z = bn[r] + th * (bn[r] - b[r]);
-                sp.Z[e] = z;
-                sp.B[e] = bn[r];
-                nz = z != 0.0;
-            }
-            if (sp.zflag) {
-                const unsigned bal = __ballot_sync(0xffffffffu, nz);
-                if ((lane & 7) == 0 && inb[r]) {
-                    const int cb = cb0 + (lane >> 3);
-                    if (cb < sp.nblk)
-                        sp.zflag[((long long)f * sp.p + j) * sp.nblk + cb] = (unsigned char)(((bal >> lane) & 0xffu) != 0u);
-                }
-            }
-        }
-    }
-    if (active && blockIdx.y == 0 && w == 0) {
-        sp.theta[par ^ 1][colbase] = th;
-        sp.tmom[par ^ 1][colbase] = tn;
     }
 }
 

@@ -274,8 +274,8 @@ class Engine:
     # second-order phase (_run_batch): iterations before the first Newton phase / between two phases
     # (measured on BASELINE configs[3], profiles/r02o_newton_tuning.txt: 500/200 469 ms, 300/200 430 ms, 300/100 422 ms,
     # 200/100 457 ms per search)
-    NEWTON_FIRST = int(os.environ.get("SLM_NEWTON_FIRST", 300))
-    NEWTON_LATER = int(os.environ.get("SLM_NEWTON_LATER", 100))
+    NEWTON_FIRST = 300
+    NEWTON_LATER = 100
     # an l1 phase that removed coordinates from a column's support counts as progress, not as one of the three failed
     # phases after which the column stays first-order: a truncated step drops about one coordinate, so a support with
     # many spurious coordinates needs several phases (profiles/r03_newton_l1_probe.jsonl: with / without this rule)
@@ -342,7 +342,8 @@ class Engine:
         return t.contiguous()
 
     def set_option(self, name, value):
-        """Engine switch by name ("coop", "small_fused", "dense_apply", "chunk_w", "tma")."""
+        """Engine switch by name ("coop", "tma", "fused_prox", "force_apply_shape", "force_sparse_shape",
+        "force_syrk_shape")."""
         self._ck(self.lib.slm_set_option(self.h, name.encode(), int(value)), "slm_set_option")
 
     def launch_count(self):

@@ -11,7 +11,7 @@ pytestmark = pytest.mark.gpu
 @pytest.fixture()
 def tma_switch(engine):
     yield engine
-    engine.set_option("tma", 7)
+    engine.set_option("tma", 15)  # the engine default: later tests run on the wide-band gather kernels
 
 
 def _expected_image(A, col0, rows):
