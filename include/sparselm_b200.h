@@ -47,7 +47,10 @@ void slm_destroy(slm_ctx* ctx);
  * swizzled boxes for the gather / tiled kernels; default 15), "fused_prox" (default 1: one prox_fused_kernel per
  * iteration on the iterate buffers, the Gram applied to the iterate itself; 0: the two-kernel iteration on a
  * materialised extrapolated point), "force_apply_shape" / "force_sparse_shape" /
- * "force_syrk_shape" (tile menu overrides of tools/gemm_probe.py, -1 = automatic). */
+ * "force_syrk_shape" / "force_score_shape" (tile menu overrides of tools/gemm_probe.py and
+ * tests/test_gpu_gemm_shapes.py: -1 = automatic, else an id of the dense apply (17 shapes), row-sparse apply
+ * (14), Gram build (4) or scoring menu (5, shared by slm_cv_score, slm_cv_score_many, slm_cv_score_rows and
+ * slm_cv_score_stats); an id outside [-1, menu size) is an error). */
 int slm_set_option(slm_ctx* ctx, const char* name, int value);
 const char* slm_last_error(const slm_ctx* ctx);
 int slm_sm_count(const slm_ctx* ctx);

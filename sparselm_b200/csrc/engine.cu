@@ -83,6 +83,7 @@ struct slm_ctx {
     int force_sparse_shape = -1;     // SLM_FORCE_SPARSE_SHAPE
     int force_apply_shape = -1;  // tuning/testing hook (SLM_FORCE_APPLY_SHAPE)
     int force_syrk_shape = -1;   // tuning/testing hook (SLM_FORCE_SYRK_SHAPE)
+    int force_score_shape = -1;  // testing hook: scoring tile of the range and gathered-row scoring GEMMs
     // TMA-fed GEMM kernels (gemm_f64_tma.cuh): bit 0 Gram build, bit 1 dense apply, bit 2 row-sparse
     // apply (SLM_TMA / slm_set_option "tma"); encode = cuTensorMapEncodeTiled resolved at run time
     bool fused_prox = true;          // SLM_FUSED_PROX=0: the two-kernel iteration (prox_main + prox_momentum on the extrapolated point)
@@ -541,7 +542,7 @@ static int apply_rowsparse(slm_ctx* ctx, const SolveDev& sp, const int32_t* K, c
             b.rowsQ = (int64_t)F * p;
         }
         int sid = pick_shape(kSparseShapes, kNumSparseShapes, pd, np, ctx->sm_count);
-        if (ctx->force_sparse_shape >= 0 && ctx->force_sparse_shape < 14) sid = ctx->force_sparse_shape;
+        if (ctx->force_sparse_shape >= 0 && ctx->force_sparse_shape < kNumSparseShapes) sid = ctx->force_sparse_shape;
         FamTimer tm(ctx, FAM_APPLY, s, first ? std::max(algo_flops, 0.0) : 0.0);
         first = false;
         cudaError_t e = launch_sparse_shape(ctx, sid, b, s);
@@ -1181,13 +1182,23 @@ int slm_set_option(slm_ctx* ctx, const char* name, int value) {
         ctx->tma_mask = value;
     else if (nm == "fused_prox")
         ctx->fused_prox = value != 0;
-    else if (nm == "force_apply_shape")
-        ctx->force_apply_shape = value;
-    else if (nm == "force_sparse_shape")
-        ctx->force_sparse_shape = value;
-    else if (nm == "force_syrk_shape")
-        ctx->force_syrk_shape = value;
-    else
+    else if (nm == "force_apply_shape" || nm == "force_sparse_shape" || nm == "force_syrk_shape" ||
+             nm == "force_score_shape") {
+        // tile menu overrides: -1 = the cost model's choice, else an id of the menu (an id past the menu is an
+        // error rather than a silent "automatic", so a caller knows which tile ran)
+        const int n_menu = nm == "force_apply_shape"    ? kNumApplyShapes
+                           : nm == "force_sparse_shape" ? kNumSparseShapes
+                           : nm == "force_syrk_shape"   ? kNumSyrkShapes
+                                                        : kNumScoreShapes;
+        if (value < -1 || value >= n_menu)
+            return fail(ctx, 1, "slm_set_option: " + nm + " must be -1 (automatic) or in [0, " + std::to_string(n_menu) +
+                                    ")");
+        int& slot = nm == "force_apply_shape"    ? ctx->force_apply_shape
+                    : nm == "force_sparse_shape" ? ctx->force_sparse_shape
+                    : nm == "force_syrk_shape"   ? ctx->force_syrk_shape
+                                                 : ctx->force_score_shape;
+        slot = value;
+    } else
         return fail(ctx, 1, "slm_set_option: unknown option " + nm);
     return 0;
 }
@@ -2414,6 +2425,7 @@ int slm_cv_score(slm_ctx* ctx, const double* Xa, int64_t lda, int64_t p, int64_t
     pr.Kd = (int)p;
     ProblemDims pd = {pr.M, pr.N};
     int sid = pick_shape(kScoreShapes, kNumScoreShapes, &pd, 1, ctx->sm_count);
+    if (ctx->force_score_shape >= 0) sid = ctx->force_score_shape;
     {
         FamTimer tm(ctx, FAM_SCORE, s, 2.0 * (double)m * (double)p * (double)K);
         cudaError_t e = launch_score_shape(ctx, sid, b, s);
@@ -2470,7 +2482,7 @@ static int cv_score_impl(slm_ctx* ctx, const char* fn, const double* Xa, int64_t
             pr.ldc = ldy[i];
             pr.M = (int)m;
             pr.N = (int)std::min<int64_t>(round_up(K[i], 8), ldy[i]);
-            pr.qlim = pr.N;
+            pr.qlim = (int)std::min<int64_t>(pr.N, ldb[i]);  // an odd K may leave ldb < N: no read past a B row
             pr.Kd = (int)p;
             pd[np] = {pr.M, pr.N};
             flops += 2.0 * (double)m * (double)p * (double)K[i];
@@ -2478,7 +2490,8 @@ static int cv_score_impl(slm_ctx* ctx, const char* fn, const double* Xa, int64_t
         }
         if (np == 0) continue;
         b.n_problems = np;
-        const int sid = pick_shape(kScoreShapes, kNumScoreShapes, pd, np, ctx->sm_count);
+        const int sid =
+            ctx->force_score_shape >= 0 ? ctx->force_score_shape : pick_shape(kScoreShapes, kNumScoreShapes, pd, np, ctx->sm_count);
         {
             FamTimer tm(ctx, FAM_SCORE, s, flops);
             cudaError_t e = rows ? launch_score_rows_shape(ctx, sid, b, s) : launch_score_shape(ctx, sid, b, s);

@@ -343,7 +343,8 @@ class Engine:
 
     def set_option(self, name, value):
         """Engine switch by name ("coop", "tma", "fused_prox", "force_apply_shape", "force_sparse_shape",
-        "force_syrk_shape")."""
+        "force_syrk_shape", "force_score_shape").  The force_* options pin a tile of the GEMM menus:
+        -1 = automatic, an id past the menu raises EngineError."""
         self._ck(self.lib.slm_set_option(self.h, name.encode(), int(value)), "slm_set_option")
 
     def launch_count(self):

@@ -34,7 +34,11 @@ def _lists(n, lens, rng):
     return lists, ptr, np.concatenate(lists).astype(np.int32)
 
 
-@pytest.mark.parametrize("tma", [True, False], ids=["tma", "cp_async"])
+# "tma" option masks of the gathered Gram: 15 wide gather bands, 7 128-byte swizzled gather boxes, 0 cp.async copies
+TMA_MASKS = pytest.mark.parametrize("tma", [15, 7, 0], ids=["tma", "tma_boxes", "cp_async"])
+
+
+@TMA_MASKS
 @pytest.mark.parametrize("p", [126, 127, 254])
 def test_gram_rows_update_matches_numpy(eng, p, tma):
     n = 300
@@ -48,13 +52,13 @@ def test_gram_rows_update_matches_numpy(eng, p, tma):
     S = len(lists)
     G0 = rng.standard_normal((S, pa, pa))
     G0 = G0 + G0.transpose(0, 2, 1)
-    eng.set_option("tma", 15 if tma else 0)
+    eng.set_option("tma", tma)
     try:
         for mode in ("plain", "accumulate", "negate"):
             G = torch.from_numpy(G0).to(eng.device)
             tma0 = eng.tma_launch_count()
             eng.gram_rows_update(Xa, ptr, rows_dev, G, accumulate=mode != "plain", negate=mode == "negate")
-            assert (eng.tma_launch_count() > tma0) == tma
+            assert (eng.tma_launch_count() > tma0) == (tma != 0)
             got = G.cpu().numpy()
             for s, idx in enumerate(lists):
                 A = Xh[idx]
@@ -79,7 +83,7 @@ def test_gram_rows_update_matches_numpy(eng, p, tma):
         eng.set_option("tma", 15)
 
 
-@pytest.mark.parametrize("tma", [True, False], ids=["tma", "cp_async"])
+@TMA_MASKS
 def test_downdate_equals_direct_build(eng, tma):
     n, p = 3000, 127
     _, _, Xa, Xh = _design(eng, n, p, 5)
@@ -87,7 +91,7 @@ def test_downdate_equals_direct_build(eng, tma):
     rng = np.random.default_rng(6)
     train = np.sort(rng.choice(n, 2200, replace=False))
     out = np.setdiff1d(np.arange(n), train)
-    eng.set_option("tma", 15 if tma else 0)
+    eng.set_option("tma", tma)
     try:
         G_full = eng.gram_blocks(Xa, np.array([0, n]))[0]
         direct = torch.empty((1, pa, pa), dtype=torch.float64, device=eng.device)
