@@ -301,6 +301,29 @@ int slm_cv_score_stats(slm_ctx* ctx, const double* Xa_dev, int64_t lda, int64_t 
 int slm_support_counts(slm_ctx* ctx, const double* coef_dev, int F, int64_t p, int64_t ldz, int K, double rel_tol,
                        int32_t* counts_dev, uint8_t* union_dev, void* stream);
 
+/* K11b: the same counts per group, for group structures that partition the features.  gptr_dev (device int32
+ * [n_groups+1], ascending, gptr[0] = 0, gptr[n_groups] <= p) holds group g's features gptr[g] .. gptr[g+1]-1 in the
+ * row order of coef_dev; groups of any length from 1 to p.  Group g is selected in fit (f, k) iff some feature of g
+ * is selected by the rule of slm_support_counts (the same column maxima: the OR of its per-feature predicates).
+ *   counts_dev[g][k] += number of fits f of the call that select g for candidate k   (int32 [n_groups][K])
+ *   union_dev[f][g]   = 1 if some candidate k < K of fit f selects g, else left as is  (uint8 [F][n_groups])
+ * Both accumulate over calls; no atomics on the counts; a NaN is never selected; columns k >= K are never read.
+ * Only enqueues work. */
+int slm_group_support_counts(slm_ctx* ctx, const double* coef_dev, int F, int64_t p, int64_t ldz, int K,
+                             double rel_tol, const int32_t* gptr_dev, int32_t n_groups, int32_t* counts_dev,
+                             uint8_t* union_dev, void* stream);
+
+/* K11c: random column weights of randomized stability selection on S <= SLM_MAX_FOLDS training Grams, in place:
+ *   G[s][i][j] = G[s][i][j] * (d_i * d_j),  d_i = w_dev[slot[s]][i] for i < p, 1 for i >= p (y row, ones row,
+ *                                              padding),
+ * G_dev [S][pa][pa] with stride g_stride; w_dev the device table [n_rows][p] in the column order of the Grams;
+ * slot a HOST int64 array [S] of rows of that table (0 <= slot[s] < n_rows).  d_i * d_j is rounded once and then
+ * multiplies G (bitwise G * outer(d, d)); the result stays exactly symmetric and the block i, j >= p is not
+ * touched.  With a centred Gram this is the centred Gram of the design whose column j is multiplied by d_j.
+ * One read and one write of S * pa^2 doubles.  Only enqueues work. */
+int slm_gram_scale(slm_ctx* ctx, double* G_dev, int64_t g_stride, int64_t pa, int64_t p, int S, const double* w_dev,
+                   int64_t n_rows, const int64_t* slot, void* stream);
+
 /* intercept[k] = ybar - mu^T B[:,k] from the (uncentred) training Gram's ones row
  * (LinearModel._set_intercept, _base.py:202). */
 int slm_intercepts(slm_ctx* ctx, const double* G_dev, int64_t pa, int64_t p,

@@ -101,6 +101,10 @@ SYMBOLS = {
     "slm_cv_score_stats": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32,
                                           c_i32, c_vp, c_vp, c_vp, c_vp]),
     "slm_support_counts": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, c_i64, c_i64, ctypes.c_int, c_dbl, c_vp, c_vp, c_vp]),
+    "slm_group_support_counts": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, c_i64, c_i64, ctypes.c_int, c_dbl, c_vp, c_i32,
+                                                c_vp, c_vp, c_vp]),
+    "slm_gram_scale": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, ctypes.c_int, c_vp, c_i64, ctypes.POINTER(c_i64),
+                                      c_vp]),
     "slm_intercepts": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp]),
     "slm_gram_apply": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, ctypes.c_int, ctypes.POINTER(c_i32), c_vp, c_i64, c_vp, c_vp]),
     "slm_newton_workspace": (c_sz, [c_i64, c_i32, c_i32, ctypes.c_int]),

@@ -13,6 +13,8 @@
 //   K10 scoring         gemm_f64_kernel<A_MMAJOR> + score_kernel
 //   K10b statistics     stat_residual/final/median_kernel (max, percentage sum, median of |r|)
 //   K11 selection       support_colmax_kernel + support_count_kernel (stability selection counts)
+//   K11b group counts   support_colmax_kernel + group_support_count_kernel (the same counts per group)
+//   K11c weakness       gram_scale_kernel (random column weights of randomized stability selection)
 #include <cuda_runtime.h>
 #include <float.h>
 #include <math.h>
@@ -2374,14 +2376,8 @@ int slm_fold_back(slm_ctx* ctx, const double* Be, const int32_t* inv_ptr, const 
     return 0;
 }
 
-int slm_support_counts(slm_ctx* ctx, const double* coef, int F, int64_t p, int64_t ldz, int K, double rel_tol,
-                       int32_t* counts, uint8_t* uni, void* stream) {
-    if (!ctx || !coef || !counts || !uni) return fail(ctx, 1, "slm_support_counts: null argument");
-    if (F < 0 || F > SLM_MAX_FOLDS || K < 0 || (int64_t)K > ldz || p < 0)
-        return fail(ctx, 1, "slm_support_counts: bad shape (need 0 <= F <= SLM_MAX_FOLDS, 0 <= K <= ldz)");
-    if (!(rel_tol >= 0.0 && rel_tol <= DBL_MAX)) return fail(ctx, 1, "slm_support_counts: rel_tol must be finite and >= 0");
-    if (F == 0 || K == 0 || p == 0) return 0;
-    cudaStream_t s = (cudaStream_t)stream;
+// Stage 1 of both selection counts: ctx->d_colmax[f][k] = max_j |coef[f][j][k]| (grown on demand, zeroed here).
+static int support_colmax(slm_ctx* ctx, const double* coef, int F, int64_t p, int64_t ldz, int K, cudaStream_t s) {
     const size_t need = (size_t)F * (size_t)ldz;
     if (need > ctx->colmax_cap) {
         // growing synchronises the device (cudaFree): it happens once per larger shape
@@ -2396,9 +2392,55 @@ int slm_support_counts(slm_ctx* ctx, const double* coef, int F, int64_t p, int64
     dim3 g1((unsigned)((K + 31) / 32), (unsigned)F, (unsigned)((p + rows_per_block - 1) / rows_per_block));
     support_colmax_kernel<<<g1, dim3(32, SEL_ROWS), 0, s>>>(coef, p, ldz, K, ctx->d_colmax);
     LAUNCH_OK("support_colmax_kernel");
+    return 0;
+}
+
+int slm_support_counts(slm_ctx* ctx, const double* coef, int F, int64_t p, int64_t ldz, int K, double rel_tol,
+                       int32_t* counts, uint8_t* uni, void* stream) {
+    if (!ctx || !coef || !counts || !uni) return fail(ctx, 1, "slm_support_counts: null argument");
+    if (F < 0 || F > SLM_MAX_FOLDS || K < 0 || (int64_t)K > ldz || p < 0)
+        return fail(ctx, 1, "slm_support_counts: bad shape (need 0 <= F <= SLM_MAX_FOLDS, 0 <= K <= ldz)");
+    if (!(rel_tol >= 0.0 && rel_tol <= DBL_MAX)) return fail(ctx, 1, "slm_support_counts: rel_tol must be finite and >= 0");
+    if (F == 0 || K == 0 || p == 0) return 0;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (int rc = support_colmax(ctx, coef, F, p, ldz, K, s)) return rc;
     support_count_kernel<<<(unsigned)((p + SEL_ROWS - 1) / SEL_ROWS), dim3(32, SEL_ROWS), 0, s>>>(
         coef, F, p, ldz, K, rel_tol, ctx->d_colmax, counts, uni);
     LAUNCH_OK("support_count_kernel");
+    return 0;
+}
+
+int slm_group_support_counts(slm_ctx* ctx, const double* coef, int F, int64_t p, int64_t ldz, int K, double rel_tol,
+                             const int32_t* gptr, int32_t n_groups, int32_t* counts, uint8_t* uni, void* stream) {
+    if (!ctx || !coef || !gptr || !counts || !uni) return fail(ctx, 1, "slm_group_support_counts: null argument");
+    if (F < 0 || F > SLM_MAX_FOLDS || K < 0 || (int64_t)K > ldz || p < 0 || n_groups < 0)
+        return fail(ctx, 1, "slm_group_support_counts: bad shape (need 0 <= F <= SLM_MAX_FOLDS, 0 <= K <= ldz)");
+    if (!(rel_tol >= 0.0 && rel_tol <= DBL_MAX))
+        return fail(ctx, 1, "slm_group_support_counts: rel_tol must be finite and >= 0");
+    if (F == 0 || K == 0 || p == 0 || n_groups == 0) return 0;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (int rc = support_colmax(ctx, coef, F, p, ldz, K, s)) return rc;
+    group_support_count_kernel<<<(unsigned)n_groups, dim3(32, SEL_ROWS), 0, s>>>(
+        coef, F, p, ldz, K, rel_tol, ctx->d_colmax, gptr, n_groups, counts, uni);
+    LAUNCH_OK("group_support_count_kernel");
+    return 0;
+}
+
+int slm_gram_scale(slm_ctx* ctx, double* G, int64_t g_stride, int64_t pa, int64_t p, int S, const double* w,
+                   int64_t n_rows, const int64_t* slot, void* stream) {
+    if (!ctx || !G || !w || !slot) return fail(ctx, 1, "slm_gram_scale: null argument");
+    if (S < 0 || S > SLM_MAX_FOLDS || p < 0 || pa < p || g_stride < pa * pa)
+        return fail(ctx, 1, "slm_gram_scale: bad shape (need 0 <= S <= SLM_MAX_FOLDS, p <= pa, g_stride >= pa^2)");
+    GramScaleSlots sl;
+    static_assert(sizeof(sl.slot) / sizeof(sl.slot[0]) == SLM_MAX_FOLDS, "one slot per Gram of a chunk");
+    for (int s = 0; s < SLM_MAX_FOLDS; ++s) sl.slot[s] = 0;
+    for (int s = 0; s < S; ++s) {
+        if (slot[s] < 0 || slot[s] >= n_rows) return fail(ctx, 1, "slm_gram_scale: slot outside the weights table");
+        sl.slot[s] = (int32_t)slot[s];
+    }
+    if (S == 0 || p == 0) return 0;
+    gram_scale_kernel<<<dim3((unsigned)pa, (unsigned)S), 256, 0, (cudaStream_t)stream>>>(G, g_stride, pa, p, w, sl);
+    LAUNCH_OK("gram_scale_kernel");
     return 0;
 }
 

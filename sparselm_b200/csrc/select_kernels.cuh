@@ -1,9 +1,11 @@
-// Stability selection: selection counts of the coefficient tables of one chunk of subsample fits
-// (slm_support_counts, DESIGN section 2 item 17).
+// Stability selection: selection counts of the coefficient tables of one chunk of subsample fits per feature
+// (slm_support_counts) and per group (slm_group_support_counts), and the random column weights of randomized
+// stability selection applied to the chunk's training Grams (slm_gram_scale); DESIGN section 2 item 17.
 //
 // coef is [F][p][ldz] as the solve returns it (fit f, feature j, candidate column k).  Coefficient j of
 // fit (f, k) is selected iff |coef| > rel_tol * max_j' |coef[f][j'][k]|; an all-zero fit selects nothing
-// and a NaN coefficient is never selected.  Columns k >= K (batch padding) are never read.
+// and a NaN coefficient is never selected.  Columns k >= K (batch padding) are never read.  A group is
+// selected in a fit iff one of its features is.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -68,6 +70,69 @@ __global__ void __launch_bounds__(32 * SEL_ROWS) support_count_kernel(const doub
         if (k < K) counts[j * K + k] += cnt;
     }
     if (lane < F && ((any >> lane) & 1u)) uni[(int64_t)lane * p + j] = 1;
+}
+
+// Stage 2 of the group counts: one block per group g (features gptr[g] .. gptr[g+1]), lane = candidate column k
+// (32 at a time).  The block's warps stride over the group's features, so a group of any length from 1 to p is
+// read by all SEL_ROWS warps; each thread keeps bit f of "some feature of g in its rows selected for (f, k)" and
+// the warps' masks are OR-ed in shared memory.  Thread (warp 0, lane) then adds the popcount of the merged mask
+// to counts[g][k] (one writer per entry: no atomics), and an OR over the lanes gives bit f of "g selected by some
+// candidate of fit f", OR-ed into union[f][g].  The predicate of one feature is the one of support_count_kernel.
+__global__ void __launch_bounds__(32 * SEL_ROWS) group_support_count_kernel(
+    const double* __restrict__ coef, int F, int64_t p, int64_t ldz, int K, double rel_tol,
+    const unsigned long long* __restrict__ colmax, const int32_t* __restrict__ gptr, int n_groups,
+    int32_t* __restrict__ counts, uint8_t* __restrict__ uni) {
+    __shared__ unsigned part[SEL_ROWS][32];
+    const int g = blockIdx.x;
+    const int lane = threadIdx.x;
+    const int64_t j0 = __ldg(gptr + g), j1 = __ldg(gptr + g + 1);
+    unsigned any = 0;  // warp 0: bit f, g selected by some candidate of fit f
+    for (int k0 = 0; k0 < K; k0 += 32) {
+        const int k = k0 + lane;
+        unsigned m = 0;
+        if (k < K) {
+            for (int f = 0; f < F; ++f) {
+                const double thr = rel_tol * __longlong_as_double((long long)__ldg(colmax + (int64_t)f * ldz + k));
+                const double* c = coef + (int64_t)f * p * ldz + k;
+                bool sel = false;
+                for (int64_t j = j0 + threadIdx.y; j < j1; j += SEL_ROWS)
+                    sel |= fabs(__ldg(c + j * ldz)) > thr;  // false for NaN
+                m |= (unsigned)sel << f;
+            }
+        }
+        part[threadIdx.y][lane] = m;
+        __syncthreads();
+        if (threadIdx.y == 0) {
+#pragma unroll
+            for (int r = 1; r < SEL_ROWS; ++r) m |= part[r][lane];
+            if (k < K) counts[(int64_t)g * K + k] += __popc(m);
+            any |= __reduce_or_sync(0xffffffffu, m);
+        }
+        __syncthreads();  // part is rewritten by the next column chunk
+    }
+    if (threadIdx.y == 0 && lane < F && ((any >> lane) & 1u)) uni[(int64_t)lane * n_groups + g] = 1;
+}
+
+// Randomized stability selection (slm_gram_scale): G[s][i][j] *= d_i * d_j in place, d_i = w[slot[s]][i] for
+// i < p and 1 for the y row, the ones row and the padding.  One block per (row i, Gram s); the product d_i * d_j
+// is rounded once and then multiplies G, which is bitwise numpy's G * np.outer(d, d) and keeps G exactly
+// symmetric.  Rows i >= p only scale their first p columns; nothing in the trailing block is touched.
+struct GramScaleSlots {
+    int32_t slot[16];  // SLM_MAX_FOLDS: row of the weights table of Gram s
+};
+
+__global__ void __launch_bounds__(256) gram_scale_kernel(double* __restrict__ G, int64_t g_stride, int64_t pa,
+                                                         int64_t p, const double* __restrict__ w, GramScaleSlots sl) {
+    const int64_t i = blockIdx.x;
+    const int s = blockIdx.y;
+    const double* ws = w + (int64_t)sl.slot[s] * p;
+    const double di = i < p ? __ldg(ws + i) : 1.0;
+    double* row = G + (int64_t)s * g_stride + i * pa;
+    const int64_t jend = i < p ? pa : p;
+    for (int64_t j = threadIdx.x; j < jend; j += blockDim.x) {
+        const double dj = j < p ? __ldg(ws + j) : 1.0;
+        row[j] = row[j] * __dmul_rn(di, dj);
+    }
 }
 
 }  // namespace slm

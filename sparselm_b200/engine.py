@@ -1273,6 +1273,36 @@ class Engine:
         self._ck(self.lib.slm_support_counts(self.h, self._ptr(coef), F, p, ldz, int(K), float(rel_tol),
                                              self._ptr(counts), self._ptr(union), self.stream), "slm_support_counts")
 
+    def group_support_counts(self, coef, K, rel_tol, gptr_dev, counts, union):
+        """support_counts per group (slm_group_support_counts): group g holds rows gptr_dev[g] .. gptr_dev[g+1]-1 of
+        `coef` (device int32 [G+1]) and is selected in a fit iff one of its features is.  counts [G, K] int32 +=
+        fits that select (g, k); union [F, G] uint8 |= some candidate of fit f selects g."""
+        torch = self.torch
+        F, p, ldz = coef.shape
+        G = gptr_dev.shape[0] - 1
+        assert coef.dtype == torch.float64 and coef.is_contiguous()
+        assert gptr_dev.dtype == torch.int32 and gptr_dev.is_contiguous() and gptr_dev.is_cuda
+        assert counts.dtype == torch.int32 and counts.is_contiguous() and tuple(counts.shape) == (G, K)
+        assert union.dtype == torch.uint8 and union.is_contiguous() and tuple(union.shape) == (F, G)
+        self._ck(self.lib.slm_group_support_counts(self.h, self._ptr(coef), F, p, ldz, int(K), float(rel_tol),
+                                                   self._ptr(gptr_dev), G, self._ptr(counts), self._ptr(union),
+                                                   self.stream), "slm_group_support_counts")
+
+    def gram_scale(self, G, p, weights, slots):
+        """G[s] *= outer(d, d) in place (slm_gram_scale) for the Grams G [S, pa, pa]: d = weights[slots[s]] (device
+        float64 [n_rows, p], the Grams' column order) on the p feature rows and columns, 1 elsewhere."""
+        torch = self.torch
+        pa = G.shape[-1]
+        Gs = G.reshape(-1, pa, pa)
+        S = Gs.shape[0]
+        slots = np.ascontiguousarray(slots, dtype=np.int64)
+        assert Gs.dtype == torch.float64 and Gs.is_contiguous() and len(slots) == S
+        assert weights.dtype == torch.float64 and weights.is_contiguous() and weights.shape[1] == p
+        self._ck(self.lib.slm_gram_scale(self.h, self._ptr(Gs), pa * pa, pa, int(p), S, self._ptr(weights),
+                                         weights.shape[0], slots.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)),
+                                         self.stream), "slm_gram_scale")
+        return G
+
     def intercepts(self, G, p, B, K):
         torch = self.torch
         ldz = B.shape[-1]

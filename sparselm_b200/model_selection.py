@@ -380,13 +380,16 @@ def _scores(scoring, metric, resid, test_cells, train_cells=None):
     return out
 
 
-def split_batches(engine, X, yv, splits, ests, specs, opts, sds, cache=None, cache_key=None, sample_weight=None):
+def split_batches(engine, X, yv, splits, ests, specs, opts, sds, cache=None, cache_key=None, sample_weight=None,
+                  on_chunk=None):
     """The (batch, chunk) loop of a search over arbitrary splits.  Per structure key yields (fkey, sd, idxs, chunks):
     the SplitData of the batch's (fit_intercept, column order), prepared on first use into `sds`; the batch's
     candidates (candidate_batches); and a generator that yields per chunk of at most 16 splits (c0, order, fd, out, t):
     the chunk's training Grams (Engine.split_chunk: slot j holds split order[j], c0 the chunk's first split), every
     candidate of the batch solved on them (solve_specs) and the host time the two took.  One [16, pa, pa] buffer
-    serves every chunk and batch: a batch's chunks are walked before the next batch is asked for."""
+    serves every chunk and batch: a batch's chunks are walked before the next batch is asked for.
+    on_chunk(spec, order, fd), when given, runs on every chunk's training Grams (built and centred) before the solve,
+    with spec the batch's first ProblemSpec: whatever it does to fd.G_train is what the candidates are solved on."""
     chunks = split_chunks(len(splits))
     buf = None
     for idxs in candidate_batches(specs).values():
@@ -398,13 +401,15 @@ def split_batches(engine, X, yv, splits, ests, specs, opts, sds, cache=None, cac
         if buf is None:
             buf = engine.torch.empty((chunks[0][1] - chunks[0][0], sd.pa, sd.pa), dtype=engine.torch.float64,
                                      device=engine.device)
-        yield fkey, sd, idxs, _solved_chunks(engine, sd, [specs[ci] for ci in idxs], chunks, buf, opts)
+        yield fkey, sd, idxs, _solved_chunks(engine, sd, [specs[ci] for ci in idxs], chunks, buf, opts, on_chunk)
 
 
-def _solved_chunks(engine, sd, bspecs, chunks, buf, opts):
+def _solved_chunks(engine, sd, bspecs, chunks, buf, opts, on_chunk=None):
     for c0, c1 in chunks:
         t0 = time.perf_counter()
         order, fd = engine.split_chunk(sd, c0, c1, buf)
+        if on_chunk is not None:
+            on_chunk(bspecs[0], order, fd)
         out = solve_specs(engine, fd, bspecs, **opts)
         yield c0, order, fd, out, time.perf_counter() - t0
 

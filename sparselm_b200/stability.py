@@ -4,8 +4,13 @@ engine.
 How often does feature j enter the model when the fit is repeated on random halves of the rows, along a grid of
 penalties?  Every (candidate, subsample) cell is a fit of one structure on its own row subset: the subsample Grams
 are built 16 at a time (Engine.split_chunk), all candidates are solved on them as one batch (solve_specs), and the
-coefficient tables are reduced to selection counts on the device (slm_support_counts).  Coefficients never leave the
-device; per chunk only the solver's convergence info comes back.
+coefficient tables are reduced to selection counts on the device (slm_support_counts, and slm_group_support_counts
+per group for the group estimators).  Coefficients never leave the device; per chunk only the solver's convergence
+info comes back.
+
+Randomized stability selection (Meinshausen & Buehlmann 2010, section 3.1; sklearn's former RandomizedLasso) also
+multiplies every column of a subsample's design by a random weight, `weakness` or 1 with probability 1/2 each: the
+chunk's Grams are rescaled on the device (slm_gram_scale) between their build and the solve.
 """
 
 from __future__ import annotations
@@ -23,9 +28,10 @@ from sklearn.utils.validation import check_is_fitted, check_X_y
 
 from .engine import get_engine
 from .model._base import EngineRegressor
+from .model._lasso import GroupLasso, OverlapGroupLasso
 from .model_selection import _SolveInfo, describe_candidates, split_batches
 
-__all__ = ["StabilitySelection", "batched_selection", "draw_subsamples", "selection_summary"]
+__all__ = ["StabilitySelection", "batched_selection", "draw_subsamples", "draw_weights", "selection_summary"]
 
 
 def draw_subsamples(n, n_subsamples, sample_fraction, complementary_pairs, random_state=None):
@@ -53,12 +59,25 @@ def draw_subsamples(n, n_subsamples, sample_fraction, complementary_pairs, rando
     return out
 
 
+def draw_weights(n_subsamples, p, weakness, random_state=None):
+    """Column weights of randomized stability selection: float64 [n_subsamples, p], entry (s, j) `weakness` or 1
+    with probability 1/2 each, independently (sklearn's former RandomizedLasso with scaling = 1 - weakness), drawn
+    from check_random_state(random_state).  weakness == 1 draws nothing and returns all ones."""
+    if not (isinstance(weakness, numbers.Real) and 0.0 < weakness <= 1.0):
+        raise ValueError(f"weakness must be finite and lie in (0, 1], got {weakness!r}")
+    if weakness == 1.0:
+        return np.ones((n_subsamples, p))
+    bits = check_random_state(random_state).randint(0, 2, size=(n_subsamples, p))
+    return np.where(bits == 1, float(weakness), 1.0)
+
+
 def selection_summary(counts, union, threshold):
     """Stability statistics of n_sub subsample fits: counts [p, n_cand] (fits selecting feature j for candidate c),
     union [n_sub, p] (feature selected by some candidate on that subsample).  Returns (stability_scores [p, n_cand],
     scores [p], q, bound): q is the mean size of the union of the selected sets over the candidates, and bound the
     Meinshausen-Buehlmann bound on the expected number of falsely selected features, q^2 / ((2 threshold - 1) p),
-    inf for threshold <= 0.5."""
+    inf for threshold <= 0.5.  The same statistics of groups take counts [G, n_cand] and union [n_sub, G]: p is then
+    the number of groups."""
     union = np.asarray(union, dtype=bool)
     n_sub, p = union.shape
     stability = np.asarray(counts, dtype=np.float64) / float(n_sub)
@@ -67,15 +86,19 @@ def selection_summary(counts, union, threshold):
     return stability, stability.max(axis=1), q, bound
 
 
-def batched_selection(engine, X, y, subsamples, ests, specs, opts, selection_tol=1e-6, sample_weight=None):
+def batched_selection(engine, X, y, subsamples, ests, specs, opts, selection_tol=1e-6, sample_weight=None,
+                      weights=None, n_groups=None):
     """Fit every (candidate, subsample) cell and count selections on the device.
 
     X: (n, p) float64 design; y: (n,); subsamples: row index arrays (distinct rows each); ests/specs: per candidate
     its fit_intercept and ProblemSpec (describe_candidates); opts: solver options; sample_weight: optional strictly
-    positive (n,) fit weights.  Candidates of different structure keys run as separate batches.
+    positive (n,) fit weights; weights: optional [n_sub, p] column weights (original feature order): subsample s is
+    fitted on X[rows_s] * weights[s]; n_groups: count the selections of the G groups of a partition too (every
+    spec's gptr, in Xa column order, holds them).  Candidates of different structure keys run as separate batches.
     Returns counts [p, n_cand] (int64, original feature order: fits that select feature j for candidate c),
-    union [n_sub, p] (bool: feature selected by some candidate on that subsample), info {n_iter, status, gap,
-    n_pass: [n_cand, n_sub]} and n_unconverged."""
+    union [n_sub, p] (bool: feature selected by some candidate on that subsample), group_counts [G, n_cand] and
+    group_union [n_sub, G] (None without n_groups), info {n_iter, status, gap, n_pass: [n_cand, n_sub]} and
+    n_unconverged."""
     torch = engine.torch
     yv = np.asarray(y, dtype=np.float64)
     p = X.shape[1]
@@ -84,23 +107,46 @@ def batched_selection(engine, X, y, subsamples, ests, specs, opts, selection_tol
     n_sub, n_cand = len(splits), len(specs)
     counts = np.zeros((p, n_cand), dtype=np.int64)
     union = np.zeros((n_sub, p), dtype=bool)
+    G = n_groups
+    group_counts = None if G is None else np.zeros((G, n_cand), dtype=np.int64)
+    group_union = None if G is None else np.zeros((n_sub, G), dtype=bool)
     info = _SolveInfo(n_cand, n_sub)
     slot_split = np.empty(n_sub, dtype=np.int64)  # row r of a union table holds subsample slot_split[r]
-    unions, perms = {}, {}
+    unions, gunions, perms = {}, {}, {}
+    scale = None
+    if weights is not None:
+        w = np.ascontiguousarray(weights, dtype=np.float64)
+        assert w.shape == (n_sub, p)
+        tables = {}  # the weights in the Xa column order of each batch, uploaded once per column order
+
+        def scale(spec, order, fd):
+            key = None if spec.col_perm is None else spec.col_perm.tobytes()
+            if key not in tables:
+                tables[key] = engine.to_device(w if spec.col_perm is None else w[:, spec.col_perm])
+            engine.gram_scale(fd.G_train, p, tables[key], order)
+
     for fkey, _, idxs, chunks in split_batches(engine, X, yv, splits, ests, specs, opts, {},
-                                               sample_weight=sample_weight):
+                                               sample_weight=sample_weight, on_chunk=scale):
         s0 = specs[idxs[0]]
         if fkey not in unions:
             # per column order: the union of one subsample is OR-ed over the batches in Xa column order
             unions[fkey] = torch.zeros((n_sub, p), dtype=torch.uint8, device=engine.device)
             perms[fkey] = s0.col_perm
+            if G is not None:
+                gunions[fkey] = torch.zeros((n_sub, G), dtype=torch.uint8, device=engine.device)
         K = len(idxs)
         cnt = torch.zeros((p, K), dtype=torch.int32, device=engine.device)
+        if G is not None:
+            assert s0.gptr is not None and len(s0.gptr) == G + 1 and s0.ext_idx is None
+            gptr_dev = engine.to_device(np.asarray(s0.gptr, dtype=np.int32))
+            gcnt = torch.zeros((G, K), dtype=torch.int32, device=engine.device)
         for c0, order, _, out, _ in chunks:
             c1 = c0 + len(order)
             # the slot order of a chunk depends on the build modes only: the same for every batch
             slot_split[c0:c1] = order
             engine.support_counts(out["coef"], K, selection_tol, cnt, unions[fkey][c0:c1])
+            if G is not None:
+                engine.group_support_counts(out["coef"], K, selection_tol, gptr_dev, gcnt, gunions[fkey][c0:c1])
             info.record(out, order, [idxs] * len(order))
         c = cnt.cpu().numpy()  # one D2H per batch, in Xa column order
         if s0.col_perm is not None:
@@ -108,6 +154,9 @@ def batched_selection(engine, X, y, subsamples, ests, specs, opts, selection_tol
             c_orig[s0.col_perm] = c
             c = c_orig
         counts[:, idxs] = c
+        if G is not None:
+            # groups are numbered in sorted-label order whatever the column order: no permutation
+            group_counts[:, idxs] = gcnt.cpu().numpy()
     for fkey, u in unions.items():
         u = u.cpu().numpy().astype(bool)
         if perms[fkey] is not None:
@@ -115,7 +164,10 @@ def batched_selection(engine, X, y, subsamples, ests, specs, opts, selection_tol
             u_orig[:, perms[fkey]] = u
             u = u_orig
         union[slot_split] |= u
-    return dict(counts=counts, union=union, info=info.tables, n_unconverged=info.n_unconverged)
+        if G is not None:
+            group_union[slot_split] |= gunions[fkey].cpu().numpy().astype(bool)
+    return dict(counts=counts, union=union, group_counts=group_counts, group_union=group_union, info=info.tables,
+                n_unconverged=info.n_unconverged)
 
 
 class StabilitySelection(SelectorMixin, MetaEstimatorMixin, BaseEstimator):
@@ -125,6 +177,20 @@ class StabilitySelection(SelectorMixin, MetaEstimatorMixin, BaseEstimator):
     fit iff ``|b_j| > selection_tol * max_k |b_k|`` (an all-zero fit selects nothing).  A feature's stability
     score is its largest selection frequency over the candidates; ``get_support`` / ``transform`` keep the
     features whose score reaches `threshold`.
+
+    Randomized stability selection (``weakness < 1``): subsample s also draws a weight w[s, j] per feature,
+    `weakness` or 1 with probability 1/2 each, and fit (s, c) is exactly
+    ``clone(estimator).set_params(**c).fit(X[rows_s] * w[s], y[rows_s], sample_weight=sw[rows_s])``; features are
+    selected from that fit's coefficients.  For the Lasso this is Meinshausen & Buehlmann's randomized Lasso (the
+    l1 weight of feature j divided by w[s, j]), sklearn's former ``RandomizedLasso(scaling=1 - weakness)``; it
+    recovers variables the plain Lasso misses when the irrepresentable condition fails.  Defining it through the
+    rescaled design makes it apply to every engine estimator.  A ``standardize=True`` group norm ``||X_g b_g||``
+    does not change when columns are rescaled: the weakness randomizes only the l1 term of the standardized
+    sparse-group estimators and has no effect on standardized pure group penalties.
+
+    For the estimators whose groups partition the features (GroupLasso, SparseGroupLasso, RidgedGroupLasso and
+    their adaptive variants, with `groups` not set by the grid) group g is selected in a fit iff one of its
+    features is, and the same statistics are kept per group.
 
     Args:
         estimator: an engine estimator with a penalty (Lasso, the group Lassos, their adaptive variants).
@@ -136,7 +202,9 @@ class StabilitySelection(SelectorMixin, MetaEstimatorMixin, BaseEstimator):
             sample_fraction 0.5 and an even n_subsamples; with an odd n the complement has ceil(n / 2) rows).
         threshold (float): selection frequency in (0, 1] a feature needs to be selected.
         selection_tol (float): relative size below which a coefficient counts as zero.
-        random_state: seed of the subsample draws.
+        weakness (float): in (0, 1]; 1 (the default) is plain stability selection and draws no weights.
+        random_state: seed of the subsample draws and then of the weights (the subsamples of a seed do not depend
+            on `weakness`).
 
     Attributes:
         subsamples_ (list[ndarray]): the row indices of every subsample.
@@ -146,12 +214,20 @@ class StabilitySelection(SelectorMixin, MetaEstimatorMixin, BaseEstimator):
         selected_size_ (float): mean over the subsamples of the size of the union of the selected sets over the
             candidates (q_Lambda).
         expected_false_positives_ (float): q_Lambda^2 / ((2 threshold - 1) p), inf for threshold <= 0.5.
+        weights_ (ndarray [n_subsamples, p]): the column weights of every subsample (all ones at weakness 1).
+        group_labels_ (ndarray [G]): the group labels in sorted order (the group order of the group estimators).
+        group_stability_scores_ (ndarray [G, n_candidates]): selection frequency per group and candidate.
+        group_scores_ (ndarray [G]): group_stability_scores_.max(axis=1).
+        group_selected_size_ (float): selected_size_ counted in groups.
+        group_expected_false_positives_ (float): expected_false_positives_ with G in place of p.
+            The group attributes are None for estimators without a partition of the features into groups (Lasso,
+            AdaptiveLasso, the overlap group Lassos) and for grids that set `groups`.
         solver_info_ (dict): n_iter, status, gap, n_pass per (candidate, subsample).
         n_features_in_ (int).
     """
 
     def __init__(self, estimator, param_grid, *, n_subsamples=100, sample_fraction=0.5, complementary_pairs=True,
-                 threshold=0.6, selection_tol=1e-6, random_state=None):
+                 threshold=0.6, selection_tol=1e-6, weakness=1.0, random_state=None):
         self.estimator = estimator
         self.param_grid = param_grid
         self.n_subsamples = n_subsamples
@@ -159,6 +235,7 @@ class StabilitySelection(SelectorMixin, MetaEstimatorMixin, BaseEstimator):
         self.complementary_pairs = complementary_pairs
         self.threshold = threshold
         self.selection_tol = selection_tol
+        self.weakness = weakness
         self.random_state = random_state
 
     def _check_params(self):
@@ -170,6 +247,18 @@ class StabilitySelection(SelectorMixin, MetaEstimatorMixin, BaseEstimator):
             raise ValueError(f"threshold must lie in (0, 1], got {self.threshold!r}")
         if not (0.0 <= self.selection_tol < math.inf):
             raise ValueError(f"selection_tol must be finite and >= 0, got {self.selection_tol!r}")
+        w = self.weakness
+        if not (isinstance(w, numbers.Real) and 0.0 < w <= 1.0):
+            raise ValueError(f"weakness must be finite and lie in (0, 1], got {w!r}")
+
+    def _group_labels(self, candidates, p):
+        """Group label of every feature when the estimator's groups partition the features, else None."""
+        est = self.estimator
+        if not isinstance(est, GroupLasso) or isinstance(est, OverlapGroupLasso):
+            return None
+        if any("groups" in c for c in candidates):
+            return None
+        return np.arange(p) if est.groups is None else np.asarray(est.groups).reshape(-1)
 
     def fit(self, X, y, sample_weight=None):
         """Draw the subsamples, fit every (candidate, subsample) cell on the GPU and count the selections."""
@@ -182,17 +271,23 @@ class StabilitySelection(SelectorMixin, MetaEstimatorMixin, BaseEstimator):
             sw = np.asarray(sample_weight, dtype=np.float64).reshape(-1)
             if sw.shape[0] != n or not np.all(np.isfinite(sw)) or not np.all(sw > 0):
                 raise ValueError("sample_weight must hold one finite, strictly positive weight per row")
-        subsamples = draw_subsamples(n, self.n_subsamples, self.sample_fraction, self.complementary_pairs,
-                                     self.random_state)
+        # one generator: the weights are drawn after the subsamples, which therefore do not depend on the weakness
+        rng = check_random_state(self.random_state)
+        subsamples = draw_subsamples(n, self.n_subsamples, self.sample_fraction, self.complementary_pairs, rng)
+        weights = draw_weights(len(subsamples), p, self.weakness, rng)
         candidates = list(ParameterGrid(self.param_grid))
         valid = set(self.estimator.get_params(deep=False))
         for c in candidates:
             if not set(c) <= valid:
                 raise ValueError(f"invalid parameters {sorted(set(c) - valid)} for {type(self.estimator).__name__}")
+        labels = self._group_labels(candidates, p)
+        group_labels = None if labels is None else np.unique(labels)
         ests, specs = describe_candidates(self.estimator, candidates, Xv, yv)
         opts = self.estimator._engine_options()
         engine = get_engine(opts.pop("device", None))
-        res = batched_selection(engine, Xv, yv, subsamples, ests, specs, opts, self.selection_tol, sw)
+        res = batched_selection(engine, Xv, yv, subsamples, ests, specs, opts, self.selection_tol, sw,
+                                weights=None if self.weakness == 1.0 else weights,
+                                n_groups=None if group_labels is None else len(group_labels))
         if res["n_unconverged"]:
             from sklearn.exceptions import ConvergenceWarning
 
@@ -200,8 +295,17 @@ class StabilitySelection(SelectorMixin, MetaEstimatorMixin, BaseEstimator):
                           ConvergenceWarning)
         self.subsamples_ = subsamples
         self.candidates_ = candidates
+        self.weights_ = weights
         self.stability_scores_, self.scores_, self.selected_size_, self.expected_false_positives_ = \
             selection_summary(res["counts"], res["union"], self.threshold)
+        self.group_labels_ = group_labels
+        if group_labels is None:
+            self.group_stability_scores_ = self.group_scores_ = None
+            self.group_selected_size_ = self.group_expected_false_positives_ = None
+        else:
+            (self.group_stability_scores_, self.group_scores_, self.group_selected_size_,
+             self.group_expected_false_positives_) = selection_summary(res["group_counts"], res["group_union"],
+                                                                       self.threshold)
         self.solver_info_ = res["info"]
         self.n_features_in_ = p
         return self
