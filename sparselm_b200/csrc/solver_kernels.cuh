@@ -26,8 +26,9 @@ constexpr int SC = 8;              // grid columns per block
 constexpr int SG = 32;             // group lanes per block
 constexpr int ST = SC * SG;        // threads per block
 constexpr int kMaxChunks = 64;     // group chunks per column (partials per column)
-constexpr int NQ = 7;              // partial quantities per (chunk, column): 0-4 gap pieces / restart dot of the
-                                   // two-kernel iteration, 5-6 restart dots of the fused iteration (by parity)
+constexpr int NQ = 9;              // partial quantities per (chunk, column): 0-4 gap pieces / restart dot of the
+                                   // two-kernel iteration, 5-6 restart dots of the fused iteration (by parity),
+                                   // 7-8 stationarity test of the smooth rows (gap kernels)
 constexpr int MOM_ROWS = 256;      // rows per block in the momentum kernel
 
 struct SolveDev {
@@ -699,6 +700,20 @@ __device__ __forceinline__ double group_dual_newton(unsigned qmask, int ja, int 
     return hi;
 }
 
+// Smooth rows: w1_j = 0 in a group with w2_g = 0 (a group left unpenalised, or an unpenalised coordinate of a
+// pure-l1 group; the ridge D2 may be anything).  Their dual constraint is g_j = 0, which a scaled residual meets
+// only to rounding: taken into omega, such a row makes the dual norm +inf (dual 0, gap = primal) at the optimum.
+// So they stay out of omega, and a column is converged only if in addition every smooth row is stationary to
+// the rounding bound of (c - G b)_j (Cauchy-Schwarz: |G_jk| <= sqrt(G_jj G_kk)):
+//     |g_j| <= tau_j = kSmoothKappa * eps * (|c_j| + sqrt(G_jj) * S) / n,   S = sum_k sqrt(G_kk) |b_k|.
+// gap_partial_kernel keeps per chunk its share of S (slot 7) and the largest S a smooth row needs to pass,
+// (n |g_j| / (kSmoothKappa eps) - |c_j|) / sqrt(G_jj) (slot 8); gap_final_kernel compares the two.  The bound is
+// loose: converged fits leave |g_j| at most 0.19 tau_j(kappa = 1) (B200, test_zero_weight_group_fits_converge;
+// 0.02-0.08 in the float64 model), so kappa = 64 leaves room for the GB recurrence of the small-design and
+// two-kernel checks and still asks for stationarity to within ~1e-14 relative.
+constexpr double kSmoothKappa = 64.0;
+constexpr double kSmoothTau = kSmoothKappa * 2.220446049250313e-16;  // kappa * eps
+
 // ---- K7a: per-chunk pieces of the duality gap of B_k ------------------------------
 // G B_k comes from the momentum recurrence (GZ, GB_{k-1}, theta) or, in final mode
 // (Z == B), from GZ directly.
@@ -768,7 +783,7 @@ __global__ void __launch_bounds__(ST) gap_partial_kernel(const __grid_constant__
             if (gj > 0.0) {
                 if (w1 > 0.0)
                     ratio = fmax(ratio, gj / w1);
-                else
+                else if (w2 > 0.0)  // w2 = 0: a smooth row, tested below
                     anyinf = true;
             }
         }
@@ -796,10 +811,24 @@ __global__ void __launch_bounds__(ST) gap_partial_kernel(const __grid_constant__
             lb = gn / (w2 + sqrt(ww2));
         lbmax = fmax(lbmax, lb);
     }
+    cb = lanes_sum(active ? cb : 0.0, red, gl, c);
+    bgb = lanes_sum(active ? bgb : 0.0, red, gl, c);
+    pen = lanes_sum(active ? pen : 0.0, red, gl, c);
+    ridge = lanes_sum(active ? ridge : 0.0, red, gl, c);
+    double* dst = sp.part + (((long long)f * sp.n_chunks + chunk) * NQ) * ldz + k;
+    if (active && gl == 0) {
+        dst[0 * ldz] = cb;
+        dst[1 * ldz] = bgb;
+        dst[2 * ldz] = pen;
+        dst[3 * ldz] = ridge;
+    }
     if (!active) lbmax = 0.0;
     // block-wide threshold: only groups whose upper bound exceeds it can hold the max
     const double thr = lanes_max(lbmax, red, gl, c);
     double omega = lbmax;
+    // second pass: Newton refinement of the groups that can hold the max, the smooth-row test
+    const double* __restrict__ gdiag = sp.G + (long long)f * sp.g_stride;  // G_jj at gdiag[j * (pa + 1)]
+    double sroot = 0.0, sneed = 0.0;
     for (int i = 0; i < sp.gpt; ++i) {
         const int g = (chunk * sp.gpt + i) * gstep + gsl;
         if (g >= sp.Gn) break;
@@ -816,13 +845,18 @@ __global__ void __launch_bounds__(ST) gap_partial_kernel(const __grid_constant__
         bool anyinf = false;
         for (int j = ja + sub; j < jb; j += rstep) {
             const double gj = gfun(j), w1 = wfun(j);
+            const double dj = sqrt(gdiag[(long long)j * (sp.pa + 1)]);
+            sroot += dj * fabs(sp.B[sbase + (long long)j * ldz]);
             gg2 += gj * gj;
             ww2 += w1 * w1;
             if (gj > 0.0) {
-                if (w1 > 0.0)
+                if (w1 > 0.0) {
                     ratio = fmax(ratio, gj / w1);
-                else
+                } else {
                     anyinf = true;
+                    if (w2 <= 0.0)  // smooth row (fmax drops the NaN of 0 / 0 for an all-zero column)
+                        sneed = fmax(sneed, (gj / (inv_n * kSmoothTau) - fabs(cvec[j])) / dj);
+                }
             }
         }
         if (GROUPED) {
@@ -841,18 +875,13 @@ __global__ void __launch_bounds__(ST) gap_partial_kernel(const __grid_constant__
             omega = fmax(omega, group_dual_newton<GROUPED>(qmask, ja, jb, sub, rstep, w2, lo, hi, gfun, wfun));
         }
     }
-    cb = lanes_sum(active ? cb : 0.0, red, gl, c);
-    bgb = lanes_sum(active ? bgb : 0.0, red, gl, c);
-    pen = lanes_sum(active ? pen : 0.0, red, gl, c);
-    ridge = lanes_sum(active ? ridge : 0.0, red, gl, c);
     omega = lanes_max(active ? omega : 0.0, red, gl, c);
+    sroot = lanes_sum(active ? sroot : 0.0, red, gl, c);
+    sneed = lanes_max(active ? sneed : 0.0, red, gl, c);
     if (active && gl == 0) {
-        double* dst = sp.part + (((long long)f * sp.n_chunks + chunk) * NQ) * ldz + k;
-        dst[0 * ldz] = cb;
-        dst[1 * ldz] = bgb;
-        dst[2 * ldz] = pen;
-        dst[3 * ldz] = ridge;
         dst[4 * ldz] = omega;
+        dst[7 * ldz] = sroot;
+        dst[8 * ldz] = sneed;
     }
 }
 
@@ -868,7 +897,7 @@ __global__ void gap_final_kernel(const __grid_constant__ SolveDev sp, int it, in
     if (!active) return;
     const int ko = sp.colmap ? sp.colmap[colbase] : k;
     const long long obase = (long long)f * ldz + ko;
-    double cb = 0.0, bgb = 0.0, pen = 0.0, ridge = 0.0, omega = 0.0;
+    double cb = 0.0, bgb = 0.0, pen = 0.0, ridge = 0.0, omega = 0.0, sroot = 0.0, sneed = 0.0;
     for (int ch = 0; ch < sp.n_chunks; ++ch) {
         const double* src = sp.part + (((long long)f * sp.n_chunks + ch) * NQ) * ldz + k;
         cb += src[0 * ldz];
@@ -876,7 +905,10 @@ __global__ void gap_final_kernel(const __grid_constant__ SolveDev sp, int it, in
         pen += src[2 * ldz];
         ridge += src[3 * ldz];
         omega = fmax(omega, src[4 * ldz]);
+        sroot += src[7 * ldz];
+        sneed = fmax(sneed, src[8 * ldz]);
     }
+    const bool smooth_ok = sneed <= sroot;  // every smooth row stationary to rounding (none: 0 <= S)
     const double* Gf = sp.G + (long long)f * sp.g_stride;
     const double n = sp.n_obs[f];
     const double yty = Gf[(long long)sp.p * sp.pa + sp.p];
@@ -895,7 +927,7 @@ __global__ void gap_final_kernel(const __grid_constant__ SolveDev sp, int it, in
     // noise-free data with a vanishing penalty stall between 1e-15 and 4e-15 yty/2n).
     const double scale = fmax(fabs(P), fmax(sp.floor_rel, 4e-15 / sp.tol) * yty / (2.0 * n));
     const bool finite = isfinite(P) && isfinite(gap);
-    const bool conv = finite && gap <= sp.tol * scale;
+    const bool conv = finite && gap <= sp.tol * scale && smooth_ok;
     if (sp.gap) sp.gap[obase] = gap;
     if (sp.primal) sp.primal[obase] = P;
     if (!final_mode) {
@@ -915,7 +947,7 @@ __global__ void gap_final_kernel(const __grid_constant__ SolveDev sp, int it, in
         // (the two differ by the rounding of the recurrence); beyond that the recurrence has
         // drifted and the column is reported as not converged.  Columns the loop never flagged
         // are judged at tol.
-        const bool ok = undecided ? conv : (finite && gap <= 4.0 * sp.tol * scale);
+        const bool ok = undecided ? conv : (finite && gap <= 4.0 * sp.tol * scale && smooth_ok);
         if (sp.status && (undecided || !ok)) sp.status[obase] = !finite ? 2 : (ok ? 0 : 1);
         if (!ok) atomicAdd(sp.counter + f, 1);
     }

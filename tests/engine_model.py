@@ -49,8 +49,33 @@ class BatchProblem:
         self.gid = np.repeat(np.arange(len(self.gptr) - 1), np.diff(self.gptr))
 
 
+SMOOTH_KAPPA = 64.0  # kSmoothKappa of csrc/solver_kernels.cuh
+
+
+def smooth_rows(pb: BatchProblem):
+    """(p, K) mask of the rows without any penalty: w1_j = 0 in a group with w2_g = 0."""
+    return (pb.W1 == 0) & (pb.W2[pb.gid] == 0)
+
+
+def smooth_ok(pb: BatchProblem, B, GB, kappa=SMOOTH_KAPPA):
+    """Per column: every smooth row is stationary to the rounding bound of (c - G b)_j,
+    |g_j| <= kappa * eps * (|c_j| + sqrt(G_jj) * sum_k sqrt(G_kk) |b_k|) / n (gap kernels)."""
+    return smooth_excess(pb, B, GB) <= kappa
+
+
+def smooth_excess(pb: BatchProblem, B, GB):
+    """Per column: max over the smooth rows of |g_j| / tau_j at kappa = 1 (0 without smooth rows)."""
+    g = np.abs((pb.c[:, None] - GB) / pb.n - pb.D2[pb.gid] * B)
+    d = np.sqrt(np.diag(pb.G))
+    tau = np.finfo(float).eps * (np.abs(pb.c)[:, None] + d[:, None] * (d[:, None] * np.abs(B)).sum(0)) / pb.n
+    with np.errstate(divide="ignore", invalid="ignore"):
+        r = np.where(smooth_rows(pb) & (g > 0), g / tau, 0.0)
+    return r.max(0)
+
+
 def gap_terms(pb: BatchProblem, B, GB):
-    """Primal, dual, gap per column from Gram quantities (gap kernel)."""
+    """Primal, dual, gap per column from Gram quantities (gap kernel).  Smooth rows stay out of
+    the dual norm: their dual constraint g_j = 0 is tested separately (smooth_ok)."""
     n = pb.n
     cb = pb.c @ B
     bgb = (B * GB).sum(0)
@@ -58,6 +83,7 @@ def gap_terms(pb: BatchProblem, B, GB):
     pen = (pb.W1 * np.abs(B)).sum(0) + (pb.W2 * np.sqrt(ss)).sum(0)
     ridge = (pb.D2 * ss).sum(0)
     g = (pb.c[:, None] - GB) / n - pb.D2[pb.gid] * B
+    g = np.where(smooth_rows(pb), 0.0, g)
     omega = np.zeros(pb.K)
     for gi in range(len(pb.gptr) - 1):
         a, b = pb.gptr[gi], pb.gptr[gi + 1]
@@ -117,7 +143,7 @@ def solve(pb: BatchProblem, tol=1e-10, floor_rel=1e-14, max_iter=20000, check_ev
         if it % check_every == 0:
             GBk = np.where(done, GB, (GZ + theta * GB) / (1 + theta))
             P, D, g = gap_terms(pb, B, GBk)
-            newly = (~done) & (g <= tol * np.maximum(np.abs(P), floor))
+            newly = (~done) & (g <= tol * np.maximum(np.abs(P), floor)) & smooth_ok(pb, B, GBk)
             gap = np.where(done, gap, g)
             iters[newly] = it
             if newly.any():
@@ -158,7 +184,7 @@ def solve_fused(pb: BatchProblem, tol=1e-10, floor_rel=1e-14, max_iter=20000, ch
         GW = pb.G @ W               # exact product of the iterate (the kernel contracts over its support rows)
         if it % check_every == 0:
             P, D, g = gap_terms(pb, W, GW)
-            newly = (~done) & (g <= tol * np.maximum(np.abs(P), floor))
+            newly = (~done) & (g <= tol * np.maximum(np.abs(P), floor)) & smooth_ok(pb, W, GW)
             iters[newly] = it
             done |= newly
             if done.all():
