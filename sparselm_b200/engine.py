@@ -96,8 +96,9 @@ class FoldData:
         return float(self.extra.get("n_obs_train", self.n_train)[which])
 
     def lipschitz(self, engine, which):
-        """L >= lambda_max(G)/n for the training Gram of fold `which` (or "full"), computed on
-        first use (a sharded rank only pays for the Grams it iterates on)."""
+        """L = LIPSCHITZ_MARGIN x (power-iteration lower bound of lambda_max(G)) / n for the training Gram of fold
+        `which` (or "full"), computed on first use (a sharded rank only pays for the Grams it iterates on).  The
+        margin covers lambda_max on most spectra, not all (DESIGN section 2 item 3)."""
         keys = list(which) if isinstance(which, (list, tuple, np.ndarray)) else [which]
         missing = [k for k in keys if k not in self._lam]
         if missing:
@@ -132,7 +133,7 @@ class FoldData:
         return out if isinstance(which, (list, tuple, np.ndarray)) else float(out[0])
 
     def lipschitz_dev(self, engine, keys, used):
-        """Device tensor [len(keys)] of L >= lambda_max(G_k)/n_k for the Grams `keys`
+        """Device tensor [len(keys)] of L (as `lipschitz`) for the Grams `keys`
         (training folds or "full"); entries of keys not listed in `used` are 1.  Nothing
         here synchronises the host: the power iterations are only enqueued and their
         results stay on the device (cached per Gram for later searches on the same data)."""
